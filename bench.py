@@ -2,6 +2,7 @@
 """Headline benchmark: ViT-B/16 224px bf16 training images/sec (BASELINE.json `metric`).
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--config 1..5 | --model NAME --batch B] [--impl ours|reference]
+                  [--dump-outputs DIR]
 
 --config selects one of BASELINE.json's configs as written (default 3 = the headline: vit_base_patch16_224, batch 256/GPU):
   1 vit_tiny_patch16_224 batch 8            2 vit_small_patch16_224 batch 256        3 vit_base_patch16_224 batch 256
@@ -177,6 +178,44 @@ def synth_batch(batch, img, gen):
     return x, soft_targets(labels), labels
 
 
+#: --dump-outputs writes an array of more elements than this as a seeded sample of that many: at most five arrays (loss,
+#: up to three outputs, parameters) of 8 MB of float32 each keep a dump well under 64 MB
+DUMP_MAX_ELEMS = 1 << 21
+
+
+def _dump_array(t):
+    """``t`` as float32, or, if it has more than DUMP_MAX_ELEMS elements, the flat sample at fixed seeded positions."""
+    t = t.detach().float()
+    if t.numel() <= DUMP_MAX_ELEMS:
+        return t
+    idx = torch.randint(0, t.numel(), (DUMP_MAX_ELEMS,), generator=torch.Generator().manual_seed(0)).sort().values
+    return t.reshape(-1)[idx.to(t.device)]
+
+
+def dump_outputs(out_dir, loss, output, model):
+    """Write what one training step computed as float32 ``out_dir/<name>.npy``: ``loss``; the model output (``output``, or
+    ``output_0``, ``output_1``, ... for nested tuples, in order: (student (cls, dist), teacher) logits with a distillation
+    teacher); ``params``, every parameter of ``model`` after the optimizer step, flattened in ``model.parameters()`` order."""
+    import numpy as np
+
+    outs = []
+
+    def flatten(o):
+        if isinstance(o, (tuple, list)):
+            for v in o:
+                flatten(v)
+        else:
+            outs.append(o)
+
+    flatten(output)
+    arrays = {"loss": loss}
+    arrays.update({"output": outs[0]} if len(outs) == 1 else {f"output_{i}": t for i, t in enumerate(outs)})
+    arrays["params"] = torch.cat([p.detach().reshape(-1).float() for p in model.parameters()])
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), _dump_array(t).cpu().numpy())
+
+
 def run_reference(args):
     """CPU arm: the restated reference eager path (oracle) on the host cores, bounded sample per step."""
     rank = int(os.environ.get("RANK", "0"))
@@ -201,8 +240,10 @@ def run_reference(args):
         O.train_step(model, crit, opt, x, y)
     t0 = time.perf_counter()
     for _ in range(args.steps):
-        O.train_step(model, crit, opt, x, y)
+        loss, out = O.train_step(model, crit, opt, x, y)
     dt = (time.perf_counter() - t0) / max(args.steps, 1)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, loss, out, model)
     v = sample_b / dt
     cores = torch.get_num_threads()
     sample = f"{args.model} fwd+bwd+AdamW fp32 eager CPU, batch {sample_b} per step (bounded sample of batch {args.batch})"
@@ -291,7 +332,13 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--breakdown", action="store_true", help="print a per-kernel-family time table to stderr")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the last one's loss, model outputs and updated parameters as float32 "
+                         "DIR/<name>.npy (a seeded sample of an array above 2M elements); the inputs are seeded, so two "
+                         "builds run with the same arguments can be compared array for array")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     cfg_model, cfg_batch, cfg_teacher = CONFIGS[args.config if args.config is not None else 3]
     if args.config is None and args.model is not None:
@@ -330,11 +377,12 @@ def main():
 
     def step(i):
         x, y = dev_batches[i % 2]
-        loss = crit(train_model(x), y)
+        out = train_model(x)
+        loss = crit(out, y)
         loss.backward()
         opt.step()
         opt.zero_grad()
-        return loss
+        return loss, out
 
     def barrier():
         if distributed:
@@ -356,7 +404,7 @@ def main():
     barrier()
     e0.record()
     for i in range(args.steps):
-        loss = step(i)
+        loss, out = step(i)
     e1.record()
     barrier()
     ms = e0.elapsed_time(e1)
@@ -370,6 +418,9 @@ def main():
     ms_per_step = ms / args.steps
     value = world * args.batch * args.steps / (ms / 1e3)
     final_loss = float(loss.item())
+    # before the teacher timing and the end-to-end region run the model again
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, loss, out, model)
 
     # the frozen teacher's forward alone (library convolutions), so that the student's share of the step is visible
     teacher_ms = None
