@@ -131,8 +131,8 @@ int vitk_layernorm_bwd(const void* dy_bf16, int64_t ld_dy, const float* x, int64
 /* ------------------------------------------------------------------------------------------------
  * Attention (timm Attention fused path = F.scaled_dot_product_attention, dropout 0, no mask)
  * qkv: bf16 [B, N, 3, H, hd] (exactly the qkv Linear output), out: bf16 [B, N, H*hd],
- * lse: fp32 [B, H, N] (natural-log sum-exp of scaled scores).  hd: a multiple of 8 in [16, 80]; N <= 640
- * (N <= 256 when hd > 64).
+ * lse: fp32 [B, H, N] (natural-log sum-exp of scaled scores).  hd: a multiple of 8 in [16, 80]; N <= 4224
+ * (N <= 256 when hd > 64); a longer sequence returns VITK_ERR_UNSUPPORTED.
  * ---------------------------------------------------------------------------------------------- */
 int vitk_attn_fwd(const void* qkv, void* out, float* lse, int32_t B, int32_t N, int32_t H,
                   int32_t head_dim, float scale, void* stream);

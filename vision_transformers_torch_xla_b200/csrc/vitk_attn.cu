@@ -24,7 +24,8 @@ using namespace vitk;
 constexpr int HD = 64;
 constexpr int TILE = 128;
 constexpr uint32_t TILE_BYTES = TILE * HD * 2;  // 16 KB: [128 rows][128 B]
-constexpr int FWD_MAX_T = 5;                    // N <= 640
+constexpr int FWD_MAX_T = 5;                    // the tiled forward keeps every K / V tile in smem: N <= 640
+constexpr int ATTN_MAX_N = 33 * TILE;           // N <= 4224: 1024 px at patch 16 (N = 4097) with room for prefix tokens
 constexpr int BWD_MAX_T = 2;                    // N <= 256 (dQ accumulators live in TMEM)
 constexpr float LOG2E = 1.4426950408889634f;
 
@@ -2143,6 +2144,256 @@ __global__ void dq_cast_kernel(const float* __restrict__ dq32, __nv_bfloat16* __
   *reinterpret_cast<uint4*>(dqkv + row * 3 * H * hd + h * hd + c) = u;
 }
 
+// ================================================================================================
+// Forward, kv-streaming (any N up to ATTN_MAX_N, head_dim <= 64): the attention-dropout forward above 640 tokens.
+// One CTA per (b, h, 128-row q tile) as in attn_fwd_kernel, thread t owns row t, but K_j / V_j stream through a
+// FWDS_STAGES-deep TMA ring (a stage is refilled as soon as P V_j has retired) and O accumulates in TMEM across kv tiles:
+// before P V_j accumulates into it, a warp rescales its 32 rows of O in place if some row raised its maximum.
+// Per kv tile: S_j (issued behind P V_{j-1}) -> row max -> wait P V_{j-1} -> refill its stage, rescale O -> exps (+ keep
+// mask) -> P -> smem -> P V_j.  Dropout exactly as attn_fwd_kernel (§4.7): the row sum is taken before the mask, m / keep
+// multiplies the P tile that feeds P V, lse is that of the undropped scores.
+// 112 KB of smem and 256 TMEM columns: two CTAs share an SM, so one's exps overlap the other's MMAs.
+// ================================================================================================
+constexpr int FWDS_STAGES = 2;
+
+struct FwdStreamSmem {
+  static constexpr uint32_t Q_OFF = 0;
+  static constexpr uint32_t KV_OFF = TILE_BYTES;                               // [stage][K, V]
+  static constexpr uint32_t P_OFF = KV_OFF + FWDS_STAGES * 2 * TILE_BYTES;
+  static constexpr uint32_t BAR_OFF = P_OFF + 2 * TILE_BYTES;
+  static constexpr uint32_t BYTES = BAR_OFF + 128;
+};
+
+__global__ void __launch_bounds__(128)
+attn_fwd_stream_kernel(const __grid_constant__ CUtensorMap tm_qkv, __nv_bfloat16* __restrict__ out, float* __restrict__ lse,
+                       int N, int H, int hd, float scale, const uint8_t* __restrict__ drop_mask, float drop_scale) {
+  using L = FwdStreamSmem;
+  extern __shared__ __align__(1024) uint8_t smem[];
+  uint64_t* bar_q = reinterpret_cast<uint64_t*>(smem + L::BAR_OFF);
+  uint64_t* kv_full = bar_q + 1;   // [FWDS_STAGES]
+  uint64_t* bar_s = kv_full + FWDS_STAGES;
+  uint64_t* bar_o = bar_s + 1;     // completes once per kv tile: P V_j retired
+  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bar_o + 1);
+
+  const int warp = threadIdx.x >> 5;
+  const int q0 = blockIdx.x * TILE, h = blockIdx.y, b = blockIdx.z;
+  const int nkv = (N + TILE - 1) / TILE;
+
+  if ((smem_u32(smem) & 1023u) != 0) __trap();
+  if (threadIdx.x == 32) {
+    mbar_init(bar_q, 1);
+    for (int s = 0; s < FWDS_STAGES; ++s) mbar_init(&kv_full[s], 1);
+    mbar_init(bar_s, 1);
+    mbar_init(bar_o, 1);
+    fence_mbar_init();
+  }
+  if (warp == 0) {
+    tmem_alloc(tmem_slot, 256);
+    tmem_relinquish();
+  }
+  tc_fence_before();
+  __syncthreads();
+  tc_fence_after();
+  const uint32_t tmem_base = *tmem_slot;
+  const uint32_t tmem_s = tmem_base;         // S_j: 128 columns
+  const uint32_t tmem_o = tmem_base + 128;   // O: 64 columns, accumulated over every kv tile
+
+  auto load_kv = [&](int j) {   // thread 0 only
+    const int st = j % FWDS_STAGES;
+    uint8_t* dst = smem + L::KV_OFF + st * 2 * TILE_BYTES;
+    mbar_arrive_expect_tx(&kv_full[st], 2 * TILE_BYTES);
+    tma_load_head(dst, &tm_qkv, &kv_full[st], H + h, j * TILE, b);
+    tma_load_head(dst + TILE_BYTES, &tm_qkv, &kv_full[st], 2 * H + h, j * TILE, b);
+  };
+  const uint32_t sQ_u = smem_u32(smem + L::Q_OFF);
+  // S_j = Q K_j^T (warp 0: uniform control flow, one elected lane)
+  auto issue_s = [&](int j) {
+    const uint32_t sK_u = smem_u32(smem + L::KV_OFF + (j % FWDS_STAGES) * 2 * TILE_BYTES);
+    mbar_wait(&kv_full[j % FWDS_STAGES], (j / FWDS_STAGES) & 1);
+    tc_fence_after();
+    const uint32_t idesc = umma_idesc(TILE, roundup16(min(TILE, N - j * TILE)), 1, false, false);
+    const uint64_t qd = umma_desc_kmajor(sQ_u), kd = umma_desc_kmajor(sK_u);
+    if (elect_one()) {
+#pragma unroll
+      for (int k = 0; k < HD / 16; ++k) umma_bf16_ss(tmem_s, qd + (uint64_t)(k * 2), kd + (uint64_t)(k * 2), idesc, k > 0);
+      umma_commit(bar_s);
+    }
+    __syncwarp();
+  };
+
+  if (threadIdx.x == 0) {
+    tma_prefetch_desc(&tm_qkv);
+    mbar_arrive_expect_tx(bar_q, TILE_BYTES);
+    tma_load_head(smem + L::Q_OFF, &tm_qkv, bar_q, h, q0, b);
+    for (int j = 0; j < FWDS_STAGES && j < nkv; ++j) load_kv(j);
+  }
+  if (warp == 0) {
+    mbar_wait(bar_q, 0);
+    issue_s(0);
+  }
+
+  const uint32_t lane_addr = static_cast<uint32_t>(warp * 32) << 16;
+  const int r = threadIdx.x;  // row inside the q tile
+  const int qrow = q0 + r;
+  const float c2 = scale * LOG2E;
+  float m_run = -INFINITY, l_run = 0.f;
+  uint8_t* sP = smem + L::P_OFF;
+  const uint32_t sP_u = smem_u32(sP);
+  const uint8_t* mrow_base = drop_mask != nullptr ? drop_mask + (((long long)b * H + h) * N + qrow) * N : nullptr;
+
+  for (int j = 0; j < nkv; ++j) {
+    const int kvn = min(TILE, N - j * TILE);
+    const uint32_t n_eff = roundup16(kvn);
+    const int nchunks = (int)(n_eff + 31) / 32;
+    mbar_wait(bar_s, j & 1);
+    tc_fence_after();
+
+    // the row (<= 128 scores) is read from TMEM once, two chunks per round trip
+    uint32_t sv[4][32];
+    float mx = m_run;
+#pragma unroll
+    for (int cb = 0; cb < 4; cb += 2) {
+      if (cb < nchunks) {
+        tmem_ld_32x32(tmem_s + lane_addr + cb * 32, sv[cb]);
+        if (cb + 1 < nchunks) tmem_ld_32x32(tmem_s + lane_addr + (cb + 1) * 32, sv[cb + 1]);
+        tmem_ld_wait();
+#pragma unroll
+        for (int cc = 0; cc < 2; ++cc) {
+          const int c = cb + cc;
+          if (c < nchunks) {
+#pragma unroll
+            for (int i = 0; i < 32; ++i)
+              if (c * 32 + i < kvn) mx = fmaxf(mx, __uint_as_float(sv[c][i]));
+          }
+        }
+      }
+    }
+    const float alpha = ex2_approx((m_run - mx) * c2);  // 0 on the first tile (m_run = -inf)
+    if (j > 0) {
+      // P V_{j-1} has retired: its K / V stage takes tile j - 1 + FWDS_STAGES, P and O may be touched again
+      mbar_wait(bar_o, (j - 1) & 1);
+      tc_fence_after();
+      if (threadIdx.x == 0 && j - 1 + FWDS_STAGES < nkv) load_kv(j - 1 + FWDS_STAGES);
+      // O <- alpha * O before P V_j accumulates into it (only if some row of the warp raised its maximum)
+      if (__any_sync(0xffffffffu, mx > m_run)) {
+#pragma unroll
+        for (int hh = 0; hh < 2; ++hh) {
+          uint32_t o0[32];
+          tmem_ld_32x32(tmem_o + lane_addr + hh * 32, o0);
+          tmem_ld_wait();
+#pragma unroll
+          for (int u = 0; u < 2; ++u) {
+            uint32_t t16[16];
+#pragma unroll
+            for (int i = 0; i < 16; ++i) t16[i] = __float_as_uint(__uint_as_float(o0[u * 16 + i]) * alpha);
+            tmem_st_32x16(tmem_o + lane_addr + hh * 32 + u * 16, t16);
+          }
+        }
+        tmem_st_wait();
+      }
+    }
+    const float mc = mx * c2;
+    float rowsum = 0.f;
+#pragma unroll
+    for (int c = 0; c < 4; ++c) {
+      if (c < nchunks) {
+#pragma unroll
+        for (int g = 0; g < 4; ++g) {
+          if ((uint32_t)(c * 32 + g * 8) < n_eff) {
+            float p[8];
+#pragma unroll
+            for (int i = 0; i < 8; ++i) {
+              const float e = ex2_approx(fmaf(__uint_as_float(sv[c][g * 8 + i]), c2, -mc));
+              p[i] = (c * 32 + g * 8 + i < kvn) ? e : 0.f;
+            }
+            uint4 u;
+            u.x = pack_bf16x2(p[0], p[1]);
+            u.y = pack_bf16x2(p[2], p[3]);
+            u.z = pack_bf16x2(p[4], p[5]);
+            u.w = pack_bf16x2(p[6], p[7]);
+            // the row sum uses the bf16-rounded probabilities so that P*V and l stay consistent
+            const float2 a0 = unpack_bf16x2(u.x), a1 = unpack_bf16x2(u.y), a2 = unpack_bf16x2(u.z), a3 = unpack_bf16x2(u.w);
+            rowsum += ((a0.x + a0.y) + (a1.x + a1.y)) + ((a2.x + a2.y) + (a3.x + a3.y));
+            if (mrow_base != nullptr) {   // the dropped, rescaled probabilities are what multiplies V
+              const int col = j * TILE + c * 32 + g * 8;
+              const uint8_t* mrow = mrow_base + col;
+#pragma unroll
+              for (int i = 0; i < 8; ++i) p[i] = (qrow < N && col + i < N && mrow[i]) ? p[i] * drop_scale : 0.f;
+              u.x = pack_bf16x2(p[0], p[1]);
+              u.y = pack_bf16x2(p[2], p[3]);
+              u.z = pack_bf16x2(p[4], p[5]);
+              u.w = pack_bf16x2(p[6], p[7]);
+            }
+            st_swz(sP, r, c * 4 + g, u);
+          }
+        }
+      }
+    }
+    l_run = l_run * alpha + rowsum;
+    m_run = mx;
+
+    fence_proxy_async_smem();
+    tc_fence_before();
+    __syncthreads();
+    if (warp == 0) {
+      tc_fence_after();
+      const uint32_t idesc = umma_idesc(TILE, HD, 1, false, true);  // A = P K-major, B = V MN-major
+      const int ksteps = (int)n_eff / 16;
+      const uint32_t sV_u = smem_u32(smem + L::KV_OFF + (j % FWDS_STAGES) * 2 * TILE_BYTES + TILE_BYTES);
+      const uint64_t pdesc = umma_desc_kmajor(sP_u), vdesc = umma_desc_mnmajor(sV_u, TILE_BYTES);
+      if (elect_one()) {
+#pragma unroll 4
+        for (int k = 0; k < ksteps; ++k)
+          umma_bf16_ss(tmem_o, pdesc + (uint64_t)((k >> 2) * (TILE_BYTES >> 4) + (k & 3) * 2), vdesc + (uint64_t)(k * 128), idesc,
+                       j > 0 || k > 0);
+        umma_commit(bar_o);
+      }
+      __syncwarp();
+      // every thread has S_j in registers: S_{j+1} runs behind P V_j
+      if (j + 1 < nkv) issue_s(j + 1);
+    }
+  }
+
+  mbar_wait(bar_o, (nkv - 1) & 1);
+  tc_fence_after();
+  {
+    uint32_t a0[32], a1[32];
+    tmem_ld_32x32(tmem_o + lane_addr, a0);
+    tmem_ld_32x32(tmem_o + lane_addr + 32, a1);
+    tmem_ld_wait();
+    if (qrow < N) {
+      const float inv = 1.0f / l_run;
+#pragma unroll
+      for (int i = 0; i < 32; ++i) {
+        a0[i] = __float_as_uint(__uint_as_float(a0[i]) * inv);
+        a1[i] = __float_as_uint(__uint_as_float(a1[i]) * inv);
+      }
+      store_row_bf16_64(out + ((long long)b * N + qrow) * (H * hd) + h * hd, a0, a1, hd);
+      if (lse) lse[((long long)b * H + h) * N + qrow] = m_run * scale + __logf(l_run);
+    }
+  }
+
+  tc_fence_before();
+  __syncthreads();
+  if (warp == 0) {
+    tc_fence_after();
+    tmem_dealloc(tmem_base, 256);
+  }
+}
+
+int launch_fwd_stream(const CUtensorMap& tm, void* out, float* lse, int B, int N, int H, int hd, float scale, cudaStream_t s,
+                      const uint8_t* drop_mask, float drop_scale) {
+  static bool attr_set = false;
+  if (!attr_set) {
+    cudaError_t e = cudaFuncSetAttribute(attn_fwd_stream_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)FwdStreamSmem::BYTES);
+    if (e != cudaSuccess) return vitk_set_error(VITK_ERR_CUDA, "attn_fwd_stream: cudaFuncSetAttribute: %s", cudaGetErrorString(e));
+    attr_set = true;
+  }
+  dim3 grid((N + TILE - 1) / TILE, H, B);
+  attn_fwd_stream_kernel<<<grid, 128, FwdStreamSmem::BYTES, s>>>(tm, (__nv_bfloat16*)out, lse, N, H, hd, scale, drop_mask, drop_scale);
+  return vitk_check_launch("attn_fwd_stream");
+}
+
 template <int T, bool WIDE = false>
 int launch_fwd(const CUtensorMap& tm, void* out, float* lse, int B, int N, int H, int hd, float scale, cudaStream_t s,
                const uint8_t* drop_mask = nullptr, float drop_scale = 1.f) {
@@ -2178,7 +2429,7 @@ static int attn_fwd_impl(const void* qkv, void* out, float* lse, int32_t B, int3
                          const uint8_t* drop_mask, float drop_scale, void* stream) {
   VITK_REQUIRE(B > 0 && N > 0 && H > 0, VITK_ERR_SHAPE, "attn_fwd: bad shape B=%d N=%d H=%d", B, N, H);
   VITK_REQUIRE(head_dim_ok(head_dim), VITK_ERR_UNSUPPORTED, "attn_fwd: head_dim=%d (built for multiples of 8 in [16, 80])", head_dim);
-  VITK_REQUIRE(N <= FWD_MAX_T * TILE, VITK_ERR_UNSUPPORTED, "attn_fwd: N=%d > %d", N, FWD_MAX_T * TILE);
+  VITK_REQUIRE(N <= ATTN_MAX_N, VITK_ERR_UNSUPPORTED, "attn_fwd: N=%d > %d", N, ATTN_MAX_N);
   VITK_REQUIRE(head_dim <= HD || N <= WIDE_MAX_N, VITK_ERR_UNSUPPORTED, "attn_fwd: head_dim=%d > 64 is built for N <= %d (N=%d)",
                head_dim, WIDE_MAX_N, N);
   VITK_REQUIRE(((uintptr_t)qkv & 15) == 0 && ((uintptr_t)out & 15) == 0, VITK_ERR_ALIGN, "attn_fwd: unaligned");
@@ -2191,7 +2442,19 @@ static int attn_fwd_impl(const void* qkv, void* out, float* lse, int32_t B, int3
   if (hd > HD)   // my_vit_xs (head_dim 72): the tiled kernel with [tile][tail] operands
     return T == 1 ? launch_fwd<1, true>(tm, out, lse, B, N, H, hd, scale, s, drop_mask, drop_scale)
                   : launch_fwd<2, true>(tm, out, lse, B, N, H, hd, scale, s, drop_mask, drop_scale);
-  if (drop_mask != nullptr) {   // attention dropout: the tiled kernel for every N (the mask is read per element)
+  // VITK_ATTN_FWD: unset = attn_fwd4 (whole score row in TMEM, one thread per row) for 128 < N <= 256, attn_fwd6 (kv loop,
+  // score MMA off the softmax's critical path) above that, the tiled one-CTA-per-q-tile kernel for N <= 128 and, with a
+  // keep mask, for N <= 640; the kv-streaming kernel for a keep mask above 640 tokens.
+  // "1" = tiled kernel everywhere (the kv-streaming kernel above 640 tokens); "6" = attn_fwd6 for every unmasked N > 128;
+  // "7" = the kv-streaming kernel for every N, with or without a mask
+  static const int variant = [] {
+    const char* e = getenv("VITK_ATTN_FWD");
+    return e ? atoi(e) : 0;
+  }();
+  const bool fwd6_ok = drop_mask == nullptr && (variant == 0 || variant == 6);
+  if (variant == 7 || (T > FWD_MAX_T && !fwd6_ok))
+    return launch_fwd_stream(tm, out, lse, B, N, H, hd, scale, s, drop_mask, drop_scale);
+  if (drop_mask != nullptr) {   // attention dropout: the tiled kernel up to 640 tokens (the mask is read per element)
     switch (T) {
       case 1: return launch_fwd<1>(tm, out, lse, B, N, H, hd, scale, s, drop_mask, drop_scale);
       case 2: return launch_fwd<2>(tm, out, lse, B, N, H, hd, scale, s, drop_mask, drop_scale);
@@ -2200,14 +2463,7 @@ static int attn_fwd_impl(const void* qkv, void* out, float* lse, int32_t B, int3
       default: return launch_fwd<5>(tm, out, lse, B, N, H, hd, scale, s, drop_mask, drop_scale);
     }
   }
-  // VITK_ATTN_FWD: unset = attn_fwd4 (whole score row in TMEM, one thread per row) for 128 < N <= 256, attn_fwd6 (kv loop,
-  // score MMA off the softmax's critical path) above that, the tiled one-CTA-per-q-tile kernel for N <= 128;
-  // "1" = tiled kernel everywhere; "6" = attn_fwd6 for every N > 128
-  static const int variant = [] {
-    const char* e = getenv("VITK_ATTN_FWD");
-    return e ? atoi(e) : 0;
-  }();
-  if ((variant == 0 || variant == 6) && T >= 2) {
+  if (fwd6_ok && T >= 2) {
     rc = make_head_tmap(&tm_out, out, H, hd, N, B, TILE);
     if (rc) return rc;
     if (variant == 0 && T == 2) return launch_fwd4(tm, tm_out, lse, B, N, H, scale, s);
@@ -2258,7 +2514,7 @@ static int attn_bwd_impl(const void* qkv, const void* out, const void* dout, con
                          void* stream) {
   VITK_REQUIRE(B > 0 && N > 0 && H > 0, VITK_ERR_SHAPE, "attn_bwd: bad shape B=%d N=%d H=%d", B, N, H);
   VITK_REQUIRE(head_dim_ok(head_dim), VITK_ERR_UNSUPPORTED, "attn_bwd: head_dim=%d (built for multiples of 8 in [16, 80])", head_dim);
-  VITK_REQUIRE(N <= FWD_MAX_T * TILE, VITK_ERR_UNSUPPORTED, "attn_bwd: N=%d > %d", N, FWD_MAX_T * TILE);
+  VITK_REQUIRE(N <= ATTN_MAX_N, VITK_ERR_UNSUPPORTED, "attn_bwd: N=%d > %d", N, ATTN_MAX_N);
   VITK_REQUIRE(head_dim <= HD || N <= WIDE_MAX_N, VITK_ERR_UNSUPPORTED, "attn_bwd: head_dim=%d > 64 is built for N <= %d (N=%d)",
                head_dim, WIDE_MAX_N, N);
   VITK_REQUIRE(((uintptr_t)qkv & 15) == 0 && ((uintptr_t)out & 15) == 0 && ((uintptr_t)dout & 15) == 0 && ((uintptr_t)dqkv & 15) == 0,

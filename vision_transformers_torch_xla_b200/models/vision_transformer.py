@@ -132,8 +132,9 @@ class Attention(nn.Module):
         self.head_dim = dim // num_heads
         if self.head_dim % 8 != 0 or not 16 <= self.head_dim <= 80:
             raise NotImplementedError(f"Attention: head_dim={self.head_dim}; the sm_100a attention kernels run on 64-wide head "
-                                      "tiles (head_dim a multiple of 8 in [16, 80]: narrower heads are zero-padded by TMA, heads "
-                                      "of 72 / 80 take a second tile and sequences of at most 256 tokens)")
+                                      "tiles (head_dim a multiple of 8 in [16, 80]: narrower heads are zero-padded by TMA and run "
+                                      "sequences of up to 4224 tokens, heads of 72 / 80 take a second tile and sequences of at most "
+                                      "256 tokens)")
         self.scale = self.head_dim ** -0.5
         self.qkv = nn.Linear(dim, dim * 3, bias=qkv_bias)
         self.q_norm = nn.Identity()
