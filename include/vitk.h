@@ -137,15 +137,15 @@ int vitk_layernorm_bwd(const void* dy_bf16, int64_t ld_dy, const float* x, int64
 int vitk_attn_fwd(const void* qkv, void* out, float* lse, int32_t B, int32_t N, int32_t H,
                   int32_t head_dim, float scale, void* stream);
 /* bwd needs a caller-owned fp32 workspace of vitk_attn_bwd_workspace_bytes(): D = rowsum(O * dO) [B, H, N], plus - when
- * N > 256 or hd > 64 - the dQ accumulator the kv tiles red.add their partials into. */
+ * N > 256, or 128 < N <= 256 with hd > 64 - the dQ accumulator the kv tiles red.add their partials into. */
 int64_t vitk_attn_bwd_workspace_bytes(int32_t B, int32_t N, int32_t H, int32_t head_dim);
 int vitk_attn_bwd(const void* qkv, const void* out, const void* dout, const float* lse,
                   void* dqkv, void* workspace, int32_t B, int32_t N, int32_t H, int32_t head_dim,
                   float scale, void* stream);
 /* Attention dropout (timm Attention.attn_drop: softmax -> Dropout -> @ v; dropout_p of the fused SDPA call): keep_mask holds
  * keep bytes [B, H, N, N] (1 = keep; vitk_dropout_mask), keep_scale = 1 / (1 - p).  out = (softmax(S) * m * keep_scale) V, lse is
- * the log-sum-exp of the undropped scores; the backward sees the same mask.  Runs on the one-CTA-per-tile forward and the
- * streaming backward for every N (the mask is read per element); the backward workspace always holds the fp32 dQ accumulator. */
+ * the log-sum-exp of the undropped scores; the backward sees the same mask.  Runs on the streaming forward and backward for
+ * every N (the mask is read per element); the backward workspace holds the fp32 dQ accumulator when N > 128. */
 int vitk_attn_fwd_dropout(const void* qkv, void* out, float* lse, const uint8_t* keep_mask, float keep_scale, int32_t B,
                           int32_t N, int32_t H, int32_t head_dim, float scale, void* stream);
 int64_t vitk_attn_bwd_dropout_workspace_bytes(int32_t B, int32_t N, int32_t H, int32_t head_dim);
@@ -242,8 +242,9 @@ int vitk_adamw_flat(float* p, float* g, const void* g_bf16, const float* grad_sc
                     void* shadow_bf16, float* ema, int64_t n, const uint8_t* chunk_group, int32_t chunk,
                     int32_t num_groups, const float* lr, const float* wd, float beta1, float beta2, float eps,
                     int64_t step, float grad_scale, float ema_decay, int32_t zero_grad, void* stream);
-/* Tuning aid: when non-NULL, the first CTA of the attention kernels stamps clock64() at its phase boundaries into
- * this device buffer of >= 32 int64 (tools/attn_trace.py prints the timeline).  NULL (default) disables it. */
+/* Tuning aid: when non-NULL, the first CTA of the persistent attention kernels (attn_fwd4 / attn_fwd6 / attn_bwd4) stamps
+ * clock64() at its phase boundaries into this device buffer of >= 128 int64 (tools/attn_trace3.py and tools/attn_trace6.py
+ * print the timelines).  NULL (default) disables it. */
 void vitk_debug_set_trace(long long* device_buf);
 
 /* Gradient clipping (engine.py:175-177; torch.nn.utils.clip_grad_norm_) without a host sync or an extra pass:

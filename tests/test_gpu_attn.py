@@ -110,33 +110,3 @@ def test_attn_unsupported_raises(cuda_device):
     lse = torch.zeros(1, 1, 300, device=cuda_device)
     with pytest.raises(L.VitkError):
         L.attn_fwd(qkv, out, lse, 1, 300, 1, 72, 72 ** -0.5)   # wide heads: N <= 256
-
-
-@pytest.mark.parametrize("fwd,bwd,N,extra", [("1", "1", 197, {}), ("6", "0", 197, {}),
-                                               ("6", "0", 577, {"VITK_ATTN_FWD6_LAZY": "8"}),
-                                               ("6", "0", 385, {"VITK_ATTN_FWD6_STAGGER": "0"})])
-def test_attn_selectable_kernels_still_agree(cuda_device, fwd, bwd, N, extra):
-    """The kernels that are not the default for a sequence length stay selectable (VITK_ATTN_FWD / VITK_ATTN_BWD, read once
-    per process, so this runs them in a child process) and must give the same answers: the simple one-CTA-per-tile
-    kernels (1), the kv-loop forward (6) at N <= 256 and with its lazy-reference and unstaggered modes."""
-    import os
-    import subprocess
-    import sys
-    code = (
-        "import torch, sys; sys.path.insert(0, %r)\n"
-        "from vision_transformers_torch_xla_b200 import _lib as L\n"
-        "torch.manual_seed(0); B, N, H = 5, %d, 6\n"
-        "qkv = torch.randn(B, N, 3 * H * 64, device='cuda').bfloat16(); dout = torch.randn(B, N, H * 64, device='cuda').bfloat16()\n"
-        "out = torch.empty(B, N, H * 64, device='cuda', dtype=torch.bfloat16); lse = torch.empty(B, H, N, device='cuda')\n"
-        "dqkv = torch.empty_like(qkv)\n"
-        "L.attn_fwd(qkv, out, lse, B, N, H, 64, 0.125); L.attn_bwd(qkv, out, dout, lse, dqkv, B, N, H, 64, 0.125)\n"
-        "q, k, v = qkv.float().view(B, N, 3, H, 64).permute(2, 0, 3, 1, 4).unbind(0)\n"
-        "q.requires_grad_(True); k.requires_grad_(True); v.requires_grad_(True)\n"
-        "o = torch.softmax((q @ k.transpose(-1, -2)) * 0.125, -1) @ v\n"
-        "ref = o.transpose(1, 2).reshape(B, N, H * 64); ref.backward(dout.float())\n"
-        "g = torch.stack([q.grad, k.grad, v.grad], 0).permute(1, 3, 0, 2, 4).reshape(B, N, 3 * H * 64)\n"
-        "e1 = ((out.float() - ref).abs().max() / ref.abs().max()).item(); e2 = ((dqkv.float() - g).abs().max() / g.abs().max()).item()\n"
-        "assert e1 < 2e-2 and e2 < 3e-2, (e1, e2)\n" % (os.path.dirname(os.path.dirname(os.path.abspath(__file__))), N))
-    env = dict(os.environ, VITK_ATTN_FWD=fwd, VITK_ATTN_BWD=bwd, **extra)
-    r = subprocess.run([sys.executable, "-c", code], env=env, capture_output=True, text=True, timeout=300)
-    assert r.returncode == 0, r.stderr[-2000:]

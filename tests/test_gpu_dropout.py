@@ -107,7 +107,9 @@ def test_gemm_mask_is_rejected_where_it_has_no_epilogue(cuda_device):
         L.gemm(x, w, out, M=128, N=64, K=64, epilogue=L.EPI_BF16, mask=m, mask_scale=2.0)
 
 
-@pytest.mark.parametrize("B,N,H,hd", [(2, 197, 3, 64), (1, 100, 2, 64), (1, 300, 2, 64), (2, 197, 2, 72), (2, 198, 2, 48)])
+@pytest.mark.parametrize("B,N,H,hd", [(2, 197, 3, 64), (1, 100, 2, 64), (1, 300, 2, 64), (2, 197, 2, 72), (2, 198, 2, 48),
+                                      (3, 577, 4, 64), (3, 640, 4, 64),
+                                      (2, 100, 2, 72)])
 def test_attention_dropout_kernels(cuda_device, B, N, H, hd):
     """attn_drop: out = (softmax(S) * m / keep) V with lse of the undropped scores; backward through the same mask.
     Against torch on the same bf16-rounded qkv and the same mask (N <= 128, 128 < N <= 256, N > 256, wide and narrow heads)."""

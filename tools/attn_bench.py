@@ -2,7 +2,9 @@
 shapes: the three sequence lengths of the BASELINE configs by default.
 
 usage: python tools/attn_bench.py                      (B, N, H, hd) = (256,197,12,64) (256,198,12,64) (64,577,16,64) (256,197,3,48)
-       python tools/attn_bench.py B N H [hd]            one shape
+       python tools/attn_bench.py B N H [hd]            one shape (head_dim 64 by default)
+       ... --attn-drop P                                 with attention dropout: a keep mask [B, H, N, N] drawn with
+                                                         drop probability P feeds the forward and the backward (no SDPA row)
 The SDPA rows are F.scaled_dot_product_attention forward and its autograd backward on [B, H, N, hd] views of the same
 qkv buffer (whichever backend torch picks on this GPU) — a reference point, not part of the product."""
 import os
@@ -31,7 +33,7 @@ def timed(fn):
     return e0.elapsed_time(e1) / ITERS * 1e3
 
 
-def run(B, N, H, hd):
+def run(B, N, H, hd, p_drop=0.0):
     torch.manual_seed(0)
     scale = hd ** -0.5
     qkv = torch.randn(B, N, 3 * H * hd, device=dev).bfloat16()
@@ -39,11 +41,13 @@ def run(B, N, H, hd):
     out = torch.empty(B, N, H * hd, device=dev, dtype=torch.bfloat16)
     lse = torch.empty(B, H, N, device=dev)
     dqkv = torch.empty_like(qkv)
+    mask = (torch.rand(B, H, N, N, device=dev) >= p_drop).to(torch.uint8) if p_drop > 0 else None
+    drop = dict(keep_mask=mask, keep_scale=1.0 / (1.0 - p_drop))
     f = 4.0 * B * H * N * N * hd
-    fwd = timed(lambda: L.attn_fwd(qkv, out, lse, B, N, H, hd, scale))
-    bwd = timed(lambda: L.attn_bwd(qkv, out, dout, lse, dqkv, B, N, H, hd, scale))
-    if os.environ.get("GB_NOSDPA", "0") == "1":
-        print(f"B={B:4d} N={N:4d} H={H:3d} hd={hd:3d} | vitk fwd {fwd:7.1f} us ({f / fwd / 1e6:6.1f} TF)  bwd {bwd:7.1f} us ({2.5 * f / bwd / 1e6:6.1f} TF)", flush=True)
+    fwd = timed(lambda: L.attn_fwd(qkv, out, lse, B, N, H, hd, scale, **drop))
+    bwd = timed(lambda: L.attn_bwd(qkv, out, dout, lse, dqkv, B, N, H, hd, scale, **drop))
+    if mask is not None or os.environ.get("GB_NOSDPA", "0") == "1":
+        print(f"B={B:4d} N={N:4d} H={H:3d} hd={hd:3d}{' drop %.2f' % p_drop if mask is not None else ''} | vitk fwd {fwd:7.1f} us ({f / fwd / 1e6:6.1f} TF)  bwd {bwd:7.1f} us ({2.5 * f / bwd / 1e6:6.1f} TF)", flush=True)
         return
     qkv_g = qkv.clone().requires_grad_(True)
     q, k, v = qkv_g.view(B, N, 3, H, hd).permute(2, 0, 3, 1, 4).unbind(0)
@@ -61,8 +65,14 @@ def run(B, N, H, hd):
           flush=True)
 
 
-if len(sys.argv) > 3:
-    run(int(sys.argv[1]), int(sys.argv[2]), int(sys.argv[3]), int(sys.argv[4]) if len(sys.argv) > 4 else 64)
+args = sys.argv[1:]
+p_drop = 0.0
+if "--attn-drop" in args:
+    i = args.index("--attn-drop")
+    p_drop = float(args[i + 1])
+    del args[i:i + 2]
+if len(args) > 2:
+    run(int(args[0]), int(args[1]), int(args[2]), int(args[3]) if len(args) > 3 else 64, p_drop)
 else:
     for shape in ((256, 197, 12, 64), (256, 198, 12, 64), (64, 577, 16, 64), (256, 197, 6, 64), (256, 197, 3, 48)):
-        run(*shape)
+        run(*shape, p_drop)

@@ -1,5 +1,5 @@
 """Where does the attention forward differ from an fp32 reference?  Prints the error of out / lse per 128-row q tile.
-usage: [VITK_ATTN_FWD=6] attn_check.py B N H [hd]"""
+usage: attn_check.py B N H [hd]"""
 import os
 import sys
 

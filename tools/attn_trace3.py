@@ -59,25 +59,12 @@ L.attn_bwd(qkv, out, dout, lse, dqkv, B, N, H, 64, 0.125)
 torch.cuda.synchronize()
 lib.vitk_debug_set_trace(None)
 t = trace.cpu().tolist()
-import os
-if os.environ.get("VITK_ATTN_BWD", "0") == "3":
-    MMA = ["S_00 issued", "S_10 issued"]
-    for j in (0, 1):
-        for w in (0, 1):
-            MMA += [f"P_{w}{j} ready", f"dV+dP_{w}{j} issued"]
-        for w in (0, 1):
-            MMA += [f"dS_{w}{j} ready", f"dK+dQ{'+S' if j == 0 else ''}_{w}{j} issued"]
-    GRP = [[], []]
-    for w in (0, 1):
-        for j in (0, 1):
-            GRP[w] += [f"S_{j} ready", f"P_{j} written", f"dP_{j} ready", f"dS_{j} written", f"drain_{j} may start", f"drain_{j} done"]
-else:
-    MMA = ["E1 dV0=,dP00 issued", "E2a dK1+=,dQ1+= (prev) issued", "E2b S10 issued", "E3 dK0=,dQ0=,S01 issued", "E4 dV0+=,dP10 issued",
-           "E5 dV1=,dP01 issued", "E6 dK0+=,dQ1=,S11 issued", "E7 dK1=,dQ0+= issued", "E8 dV1+=,dP11 issued", "S00' issued"]
-    GRP = [[], []]
-    for j in (0, 1):
-        GRP[0] += [f"S_0{j} ready", f"P_0{j} written (+deferred drain)", f"dP_0{j} ready", f"dS_0{j} written"]
-        GRP[1] += [f"S_1{j} ready", f"P_1{j} written", f"dP_1{j} ready", f"dS_1{j} written", f"dK_{j} drained"]
+MMA = ["E1 dV0=,dP00 issued", "E2a dK1+=,dQ1+= (prev) issued", "E2b S10 issued", "E3 dK0=,dQ0=,S01 issued", "E4 dV0+=,dP10 issued",
+       "E5 dV1=,dP01 issued", "E6 dK0+=,dQ1=,S11 issued", "E7 dK1=,dQ0+= issued", "E8 dV1+=,dP11 issued", "S00' issued"]
+GRP = [[], []]
+for j in (0, 1):
+    GRP[0] += [f"S_0{j} ready", f"P_0{j} written (+deferred drain)", f"dP_0{j} ready", f"dS_0{j} written"]
+    GRP[1] += [f"S_1{j} ready", f"P_1{j} written", f"dP_1{j} ready", f"dS_1{j} written", f"dK_{j} drained"]
 ev = []
 for i, name in enumerate(MMA):
     if t[i]:

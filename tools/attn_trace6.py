@@ -1,6 +1,6 @@
-"""Timeline (SM cycles) of the second work item of CTA 0 of attn_fwd6 (run with VITK_ATTN_FWD=6): per group and kv step,
+"""Timeline (SM cycles) of the second work item of CTA 0 of attn_fwd6 (unmasked N > 256): per group and kv step,
 when its exps started, when P was written and when the next S was in registers with its maximum known.
-usage: VITK_ATTN_FWD=6 attn_trace6.py [B] [N] [H]"""
+usage: attn_trace6.py [B] [N] [H]"""
 import os
 import sys
 

@@ -13,8 +13,6 @@
 // The same smem bytes serve as a K-major operand ([rows][64 contiguous] = rows x K) and as an
 // MN-major operand (K rows x 64 contiguous MN) — only the UMMA descriptor differs — which is how
 // P / dS feed P*V, P^T*dO, dS^T*Q and dS*K without any transposes.
-#include <cstdlib>
-
 #include "vitk_common.cuh"
 #include "vitk_internal.h"
 
@@ -24,20 +22,13 @@ using namespace vitk;
 constexpr int HD = 64;
 constexpr int TILE = 128;
 constexpr uint32_t TILE_BYTES = TILE * HD * 2;  // 16 KB: [128 rows][128 B]
-constexpr int FWD_MAX_T = 5;                    // the tiled forward keeps every K / V tile in smem: N <= 640
 constexpr int ATTN_MAX_N = 33 * TILE;           // N <= 4224: 1024 px at patch 16 (N = 4097) with room for prefix tokens
-constexpr int BWD_MAX_T = 2;                    // N <= 256 (dQ accumulators live in TMEM)
 constexpr float LOG2E = 1.4426950408889634f;
 
 __device__ __forceinline__ uint32_t roundup16(int v) { return (uint32_t)((v + 15) & ~15); }
 
-// Phase timeline for tuning (vitk_debug_set_trace): the first CTA's thread 0 stamps clock64() into a device buffer.
+// Phase timeline for tuning (vitk_debug_set_trace): attn_fwd4 / attn_fwd6 / attn_bwd4 stamp clock64() into a device buffer.
 long long* g_trace_buf = nullptr;
-#define VITK_STAMP(slot)                                                                    \
-  do {                                                                                      \
-    if (trace != nullptr && threadIdx.x == 0 && blockIdx.x == 0 && blockIdx.y == 0 && blockIdx.z == 0) \
-      trace[(slot)] = clock64();                                                            \
-  } while (0)
 
 // Store 8 consecutive bf16 (one 16-byte unit `u8` of row `r`) into a [chunk][128 rows][128 B] swizzled tile.
 __device__ __forceinline__ void st_swz(uint8_t* tile, int r, int col8, uint4 val) {
@@ -56,25 +47,11 @@ __device__ __forceinline__ void pin32(uint32_t (&r)[32]) {
                "+r"(r[25]), "+r"(r[26]), "+r"(r[27]), "+r"(r[28]), "+r"(r[29]), "+r"(r[30]), "+r"(r[31]));
 }
 
-// ================================================================================================
-// Forward
-// ================================================================================================
-// smem: Q | K_j, V_j for all kv tiles | P [32K] | barriers
-// WIDE (64 < head_dim <= 80, my_vit_xs: 72): every operand is [64-column tile][tail tile] (2 x 16 KB, the tail holding
-// columns 64 .. 127 of the head with everything >= head_dim zero-filled by TMA).  As a K-major operand the tail adds one
-// k-step (columns 64 .. 79) to Q K^T; as an MN-major operand it is the second 64-wide chunk of V, of which P V with
-// N = 80 reads the first 16 columns.  O has 80 accumulator columns.
+// Wide heads (64 < head_dim <= 80, my_vit_xs: 72): every operand is [64-column tile][tail tile] (2 x 16 KB, the tail
+// holding columns 64 .. 127 of the head with everything >= head_dim zero-filled by TMA).  As a K-major operand the tail
+// adds one k-step (columns 64 .. 79) to Q K^T; as an MN-major operand it is the second 64-wide chunk of V (dO, Q, K), of
+// which an MMA with N = 80 reads the first 16 columns.  Accumulators over the head dimension have 80 columns.
 constexpr int HDW_MAX = 80;
-
-template <int T, bool WIDE>
-struct FwdSmem {
-  static constexpr uint32_t OPB = WIDE ? 2 * TILE_BYTES : TILE_BYTES;   // bytes of one operand tile (+ tail)
-  static constexpr uint32_t Q_OFF = 0;
-  static constexpr uint32_t KV_OFF = OPB;
-  static constexpr uint32_t P_OFF = KV_OFF + T * 2 * OPB;
-  static constexpr uint32_t BAR_OFF = P_OFF + 2 * TILE_BYTES;
-  static constexpr uint32_t BYTES = BAR_OFF + 128;
-};
 
 // one operand box (+ its tail for wide heads) of head slot `slot`, rows row0 .., image b
 template <bool WIDE>
@@ -82,235 +59,6 @@ __device__ __forceinline__ void load_head_tiles(uint8_t* dst, const CUtensorMap*
   tma_load_head(dst, tm, bar, slot, row0, b);
   if (WIDE) tma_load_head_col(dst + TILE_BYTES, tm, bar, HD, slot, row0, b);
 }
-
-template <int T, bool WIDE>
-__global__ void __launch_bounds__(128)
-attn_fwd_kernel(const __grid_constant__ CUtensorMap tm_qkv, __nv_bfloat16* __restrict__ out,
-                float* __restrict__ lse, int N, int H, int hd, float scale, const uint8_t* __restrict__ drop_mask,
-                float drop_scale, long long* trace) {
-  // drop_mask (attn_drop, timm Attention: softmax -> Dropout -> @ v): keep bytes [B, H, N, N] or null.  The row sum (the
-  // softmax normaliser) is taken BEFORE the mask, the mask / keep_prob goes onto the P tile that feeds P V.
-  VITK_STAMP(0);
-  using L = FwdSmem<T, WIDE>;
-  constexpr int HDW = WIDE ? HDW_MAX : HD;   // accumulator columns of O
-  extern __shared__ __align__(1024) uint8_t smem[];
-  uint64_t* bar_q = reinterpret_cast<uint64_t*>(smem + L::BAR_OFF);
-  uint64_t* bar_kv = bar_q + 1;       // [T]
-  uint64_t* bar_s = bar_kv + T;
-  uint64_t* bar_o = bar_s + 1;
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bar_o + 1);
-
-  const int warp = threadIdx.x >> 5;
-  const int q0 = blockIdx.x * TILE, h = blockIdx.y, b = blockIdx.z;
-  const int nkv = (N + TILE - 1) / TILE;
-
-  if ((smem_u32(smem) & 1023u) != 0) __trap();
-  if (threadIdx.x == 32) {
-    mbar_init(bar_q, 1);
-    for (int j = 0; j < T; ++j) mbar_init(&bar_kv[j], 1);
-    mbar_init(bar_s, 1);
-    mbar_init(bar_o, 1);
-    fence_mbar_init();
-  }
-  if (warp == 0) {
-    tmem_alloc(tmem_slot, 256);
-    tmem_relinquish();
-  }
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem_base = *tmem_slot;
-  const uint32_t tmem_s = tmem_base;         // S: 128 columns
-  const uint32_t tmem_o = tmem_base + 128;   // O_j: 64 (80) columns
-  VITK_STAMP(1);
-
-  if (threadIdx.x == 0) {
-    tma_prefetch_desc(&tm_qkv);
-    mbar_arrive_expect_tx(bar_q, L::OPB);
-    load_head_tiles<WIDE>(smem + L::Q_OFF, &tm_qkv, bar_q, h, q0, b);
-    for (int j = 0; j < nkv; ++j) {
-      mbar_arrive_expect_tx(&bar_kv[j], 2 * L::OPB);
-      load_head_tiles<WIDE>(smem + L::KV_OFF + j * 2 * L::OPB, &tm_qkv, &bar_kv[j], H + h, j * TILE, b);
-      load_head_tiles<WIDE>(smem + L::KV_OFF + j * 2 * L::OPB + L::OPB, &tm_qkv, &bar_kv[j], 2 * H + h, j * TILE, b);
-    }
-  }
-
-  const uint32_t lane_addr = static_cast<uint32_t>(warp * 32) << 16;
-  const int r = threadIdx.x;  // row inside the q tile
-  const float c2 = scale * LOG2E;
-  float m_run = -INFINITY, l_run = 0.f;
-  float o_acc[HDW];
-#pragma unroll
-  for (int d = 0; d < HDW; ++d) o_acc[d] = 0.f;
-
-  uint8_t* sP = smem + L::P_OFF;
-  const uint32_t sQ_u = smem_u32(smem + L::Q_OFF);
-  const uint32_t sP_u = smem_u32(sP);
-
-  for (int j = 0; j < nkv; ++j) {
-    const int kvn = min(TILE, N - j * TILE);
-    const uint32_t n_eff = roundup16(kvn);
-    const uint32_t sK_u = smem_u32(smem + L::KV_OFF + j * 2 * L::OPB);
-    const uint32_t sV_u = sK_u + L::OPB;
-    if (warp == 0) {   // uniform control flow + one elected lane: the descriptors stay in uniform registers
-      if (j == 0) mbar_wait(bar_q, 0);
-      mbar_wait(&bar_kv[j], 0);
-      tc_fence_after();
-      const uint32_t idesc = umma_idesc(TILE, n_eff, 1, false, false);
-      const uint64_t qd = umma_desc_kmajor(sQ_u), kd = umma_desc_kmajor(sK_u);
-      const uint64_t qd_t = umma_desc_kmajor(sQ_u + TILE_BYTES), kd_t = umma_desc_kmajor(sK_u + TILE_BYTES);
-      if (elect_one()) {
-#pragma unroll
-        for (int k = 0; k < HD / 16; ++k) umma_bf16_ss(tmem_s, qd + (uint64_t)(k * 2), kd + (uint64_t)(k * 2), idesc, k > 0);
-        if (WIDE) umma_bf16_ss(tmem_s, qd_t, kd_t, idesc, true);   // head columns 64 .. 79
-        umma_commit(bar_s);
-      }
-      __syncwarp();
-    }
-    mbar_wait(bar_s, j & 1);
-    tc_fence_after();
-    VITK_STAMP(2 + j * 4);
-
-    // ---- online softmax over this kv tile: the row (<= 128 scores) is read from TMEM once, two chunks per round trip ----
-    const int nchunks = (int)(n_eff + 31) / 32;
-    uint32_t sv[4][32];
-    float mx = m_run;
-#pragma unroll
-    for (int cb = 0; cb < 4; cb += 2) {
-      if (cb < nchunks) {
-        tmem_ld_32x32(tmem_s + lane_addr + cb * 32, sv[cb]);
-        if (cb + 1 < nchunks) tmem_ld_32x32(tmem_s + lane_addr + (cb + 1) * 32, sv[cb + 1]);
-        tmem_ld_wait();
-#pragma unroll
-        for (int cc = 0; cc < 2; ++cc) {
-          const int c = cb + cc;
-          if (c < nchunks) {
-#pragma unroll
-            for (int i = 0; i < 32; ++i)
-              if (c * 32 + i < kvn) mx = fmaxf(mx, __uint_as_float(sv[c][i]));
-          }
-        }
-      }
-    }
-    const float alpha = ex2_approx((m_run - mx) * c2);  // 0 on the first tile (m_run = -inf)
-    const float mc = mx * c2;
-    float rowsum = 0.f;
-#pragma unroll
-    for (int c = 0; c < 4; ++c) {
-      if (c < nchunks) {
-#pragma unroll
-        for (int g = 0; g < 4; ++g) {
-          if ((uint32_t)(c * 32 + g * 8) < n_eff) {
-            float p[8];
-#pragma unroll
-            for (int i = 0; i < 8; ++i) {
-              const float e = ex2_approx(fmaf(__uint_as_float(sv[c][g * 8 + i]), c2, -mc));
-              p[i] = (c * 32 + g * 8 + i < kvn) ? e : 0.f;
-            }
-            uint4 u;
-            u.x = pack_bf16x2(p[0], p[1]);
-            u.y = pack_bf16x2(p[2], p[3]);
-            u.z = pack_bf16x2(p[4], p[5]);
-            u.w = pack_bf16x2(p[6], p[7]);
-            // the row sum uses the bf16-rounded probabilities so that P*V and l stay consistent
-            const float2 a0 = unpack_bf16x2(u.x), a1 = unpack_bf16x2(u.y), a2 = unpack_bf16x2(u.z), a3 = unpack_bf16x2(u.w);
-            rowsum += ((a0.x + a0.y) + (a1.x + a1.y)) + ((a2.x + a2.y) + (a3.x + a3.y));
-            if (drop_mask != nullptr) {   // the dropped, rescaled probabilities are what multiplies V
-              const int qrow = q0 + r, col = j * TILE + c * 32 + g * 8;
-              const uint8_t* mrow = drop_mask + (((long long)b * H + h) * N + qrow) * N + col;
-#pragma unroll
-              for (int i = 0; i < 8; ++i) p[i] = (qrow < N && col + i < N && mrow[i]) ? p[i] * drop_scale : 0.f;
-              u.x = pack_bf16x2(p[0], p[1]);
-              u.y = pack_bf16x2(p[2], p[3]);
-              u.z = pack_bf16x2(p[4], p[5]);
-              u.w = pack_bf16x2(p[6], p[7]);
-            }
-            st_swz(sP, r, c * 4 + g, u);
-          }
-        }
-      }
-    }
-    l_run = l_run * alpha + rowsum;
-    m_run = mx;
-    VITK_STAMP(3 + j * 4);
-
-    fence_proxy_async_smem();
-    tc_fence_before();
-    __syncthreads();
-    VITK_STAMP(4 + j * 4);
-    if (warp == 0) {
-      tc_fence_after();
-      const uint32_t idesc = umma_idesc(TILE, HDW, 1, false, true);  // A = P K-major, B = V MN-major (tail = second 64-wide chunk)
-      const int ksteps = (int)n_eff / 16;
-      const uint64_t pdesc = umma_desc_kmajor(sP_u), vdesc = umma_desc_mnmajor(sV_u, TILE_BYTES);
-      if (elect_one()) {
-#pragma unroll 4
-        for (int k = 0; k < ksteps; ++k)
-          umma_bf16_ss(tmem_o, pdesc + (uint64_t)((k >> 2) * (TILE_BYTES >> 4) + (k & 3) * 2), vdesc + (uint64_t)(k * 128), idesc, k > 0);
-        umma_commit(bar_o);
-      }
-      __syncwarp();
-    }
-    mbar_wait(bar_o, j & 1);
-    tc_fence_after();
-    VITK_STAMP(5 + j * 4);
-#pragma unroll
-    for (int c = 0; c < 2; ++c) {
-      uint32_t ov[32];
-      tmem_ld_32x32(tmem_o + lane_addr + c * 32, ov);
-      tmem_ld_wait();
-#pragma unroll
-      for (int i = 0; i < 32; ++i) o_acc[c * 32 + i] = fmaf(o_acc[c * 32 + i], alpha, __uint_as_float(ov[i]));
-    }
-    if (WIDE) {
-      uint32_t ov[16];
-      tmem_ld_32x16(tmem_o + lane_addr + 64, ov);
-      tmem_ld_wait();
-#pragma unroll
-      for (int i = 0; i < 16; ++i) o_acc[(HDW - 16) + i] = fmaf(o_acc[(HDW - 16) + i], alpha, __uint_as_float(ov[i]));
-    }
-    tc_fence_before();
-  }
-
-  const int q = q0 + r;
-  if (q < N) {
-    const float inv = 1.0f / l_run;
-    __nv_bfloat16* orow = out + ((long long)b * N + q) * (H * hd) + h * hd;
-#pragma unroll
-    for (int g = 0; g < HDW / 8; ++g) {
-      if (g * 8 >= hd) break;   // columns >= head_dim are the zero padding of the tiles
-      uint4 u;
-      u.x = pack_bf16x2(o_acc[g * 8 + 0] * inv, o_acc[g * 8 + 1] * inv);
-      u.y = pack_bf16x2(o_acc[g * 8 + 2] * inv, o_acc[g * 8 + 3] * inv);
-      u.z = pack_bf16x2(o_acc[g * 8 + 4] * inv, o_acc[g * 8 + 5] * inv);
-      u.w = pack_bf16x2(o_acc[g * 8 + 6] * inv, o_acc[g * 8 + 7] * inv);
-      *reinterpret_cast<uint4*>(orow + g * 8) = u;
-    }
-    if (lse) lse[((long long)b * H + h) * N + q] = m_run * scale + __logf(l_run);
-  }
-  VITK_STAMP(30);
-
-  __syncthreads();
-  if (warp == 0) {
-    tc_fence_after();
-    tmem_dealloc(tmem_base, 256);
-  }
-  VITK_STAMP(31);
-}
-
-// ================================================================================================
-// Backward (N <= 256): one CTA per (b, h); kv tile j outer, q tile i inner.
-// TMEM: S [0,128) | dP [128,256) | dV_j [256,320) | dK_j [320,384) | dQ_0 [384,448) | dQ_1 [448,512)
-// smem: Q_i, dO_i (T * 32K) | K_j, V_j (T * 32K) | P (32K) | dS (32K) | barriers
-// ================================================================================================
-struct BwdSmem {
-  static constexpr uint32_t QDO_OFF = 0;
-  static constexpr uint32_t KV_OFF = BWD_MAX_T * 2 * TILE_BYTES;
-  static constexpr uint32_t P_OFF = KV_OFF + BWD_MAX_T * 2 * TILE_BYTES;
-  static constexpr uint32_t DS_OFF = P_OFF + 2 * TILE_BYTES;
-  static constexpr uint32_t BAR_OFF = DS_OFF + 2 * TILE_BYTES;
-  static constexpr uint32_t BYTES = BAR_OFF + 128;
-};
 
 // one accumulator row (columns 0..31 in a, 32..63 in b) -> bf16; only the first `hd` (multiple of 8) columns exist
 __device__ __forceinline__ void store_row_bf16_64(__nv_bfloat16* dst, const uint32_t (&a)[32], const uint32_t (&b)[32], int hd) {
@@ -334,240 +82,6 @@ __device__ __forceinline__ void store_row_bf16_64(__nv_bfloat16* dst, const uint
     u.w = pack_bf16x2(__uint_as_float(b[g * 8 + 6]), __uint_as_float(b[g * 8 + 7]));
     *reinterpret_cast<uint4*>(dst + 32 + g * 8) = u;
   }
-}
-
-__global__ void __launch_bounds__(128)
-attn_bwd_kernel(const __grid_constant__ CUtensorMap tm_qkv, const __grid_constant__ CUtensorMap tm_do,
-                const float* __restrict__ dsum_g, const float* __restrict__ lse, __nv_bfloat16* __restrict__ dqkv, int N, int H, int hd,
-                float scale, long long* trace) {
-  using L = BwdSmem;
-  VITK_STAMP(0);
-  extern __shared__ __align__(1024) uint8_t smem[];
-  uint64_t* bar_ld = reinterpret_cast<uint64_t*>(smem + L::BAR_OFF);
-  uint64_t* bar_sp = bar_ld + 1;
-  uint64_t* bar_drain = bar_sp + 1;  // completes once per kv tile j
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bar_drain + 1);
-
-  const int warp = threadIdx.x >> 5;
-  const int h = blockIdx.x, b = blockIdx.y;
-  const int nt = (N + TILE - 1) / TILE;  // q tiles == kv tiles
-
-  if ((smem_u32(smem) & 1023u) != 0) __trap();
-  if (threadIdx.x == 32) {
-    mbar_init(bar_ld, 1);
-    mbar_init(bar_sp, 1);
-    mbar_init(bar_drain, 1);
-    fence_mbar_init();
-  }
-  if (warp == 0) {
-    tmem_alloc(tmem_slot, 512);
-    tmem_relinquish();
-  }
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem_base = *tmem_slot;
-  const uint32_t tm_s = tmem_base, tm_dp = tmem_base + 128, tm_dv = tmem_base + 256, tm_dk = tmem_base + 320;
-  const uint32_t tm_dq = tmem_base + 384;
-
-  if (threadIdx.x == 0) {
-    tma_prefetch_desc(&tm_qkv);
-    tma_prefetch_desc(&tm_do);
-    mbar_arrive_expect_tx(bar_ld, nt * 4 * TILE_BYTES);
-    for (int t = 0; t < nt; ++t) {
-      tma_load_head(smem + L::QDO_OFF + t * 2 * TILE_BYTES, &tm_qkv, bar_ld, h, t * TILE, b);
-      tma_load_head(smem + L::QDO_OFF + t * 2 * TILE_BYTES + TILE_BYTES, &tm_do, bar_ld, h, t * TILE, b);
-      tma_load_head(smem + L::KV_OFF + t * 2 * TILE_BYTES, &tm_qkv, bar_ld, H + h, t * TILE, b);
-      tma_load_head(smem + L::KV_OFF + t * 2 * TILE_BYTES + TILE_BYTES, &tm_qkv, bar_ld, 2 * H + h, t * TILE, b);
-    }
-  }
-
-  // per-row statistics for the (up to) two q tiles this thread owns a row of (D comes from attn_dsum_kernel)
-  const int r = threadIdx.x;
-  float lse2[BWD_MAX_T], dsum[BWD_MAX_T];
-#pragma unroll
-  for (int i = 0; i < BWD_MAX_T; ++i) {
-    lse2[i] = 0.f;
-    dsum[i] = 0.f;
-    const int q = i * TILE + r;
-    if (i < nt && q < N) {
-      lse2[i] = lse[((long long)b * H + h) * N + q] * LOG2E;
-      dsum[i] = dsum_g[((long long)b * H + h) * N + q];
-    }
-  }
-
-  const uint32_t lane_addr = static_cast<uint32_t>(warp * 32) << 16;
-  const float c2 = scale * LOG2E;
-  uint8_t* sP = smem + L::P_OFF;
-  uint8_t* sDS = smem + L::DS_OFF;
-  const uint32_t sP_u = smem_u32(sP), sDS_u = smem_u32(sDS);
-  uint32_t sp_phase = 0;
-
-  // issue S = Q_i K_j^T and dP = dO_i V_j^T
-  VITK_STAMP(1);
-  auto issue_s_dp = [&](int j, int i) {
-    const uint32_t n_eff = roundup16(min(TILE, N - j * TILE));
-    const uint32_t sQ = smem_u32(smem + L::QDO_OFF + i * 2 * TILE_BYTES), sDO = sQ + TILE_BYTES;
-    const uint32_t sK = smem_u32(smem + L::KV_OFF + j * 2 * TILE_BYTES), sV = sK + TILE_BYTES;
-    const uint32_t idesc = umma_idesc(TILE, n_eff, 1, false, false);
-#pragma unroll
-    for (int k = 0; k < HD / 16; ++k)
-      umma_bf16_ss(tm_s, umma_desc_kmajor(sQ + k * 32), umma_desc_kmajor(sK + k * 32), idesc, k > 0);
-#pragma unroll
-    for (int k = 0; k < HD / 16; ++k)
-      umma_bf16_ss(tm_dp, umma_desc_kmajor(sDO + k * 32), umma_desc_kmajor(sV + k * 32), idesc, k > 0);
-    umma_commit(bar_sp);
-  };
-
-  if (threadIdx.x == 0) {
-    mbar_wait(bar_ld, 0);
-    tc_fence_after();
-    VITK_STAMP(2);
-    issue_s_dp(0, 0);
-  }
-
-  for (int j = 0; j < nt; ++j) {
-    const int kvn = min(TILE, N - j * TILE);
-    const uint32_t n_eff = roundup16(kvn);
-    const int nchunks = (int)(n_eff + 31) / 32;
-    for (int i = 0; i < nt; ++i) {
-      const int qn = min(TILE, N - i * TILE);
-      const uint32_t q_eff = roundup16(qn);
-      const bool row_ok = r < qn;
-      const float my_lse2 = (i == 0) ? lse2[0] : lse2[1];
-      const float my_d = (i == 0) ? dsum[0] : dsum[1];
-
-      // S, dP ready; this also implies the previous iteration's dV/dK/dQ MMAs (which read P/dS) retired.
-      mbar_wait(bar_sp, sp_phase);
-      sp_phase ^= 1;
-      tc_fence_after();
-      VITK_STAMP(3 + (j * 2 + i) * 4);
-
-      // every thread executes the (.sync.aligned) TMEM loads; only rows < q_eff compute and store.
-      // Two chunks of S and of dP per TMEM round trip (the round trip, not the math, dominated this loop).
-      for (int cb = 0; cb < nchunks; cb += 2) {
-        uint32_t sv[2][32], dv[2][32];
-        tmem_ld_32x32(tm_s + lane_addr + cb * 32, sv[0]);
-        tmem_ld_32x32(tm_dp + lane_addr + cb * 32, dv[0]);
-        if (cb + 1 < nchunks) {
-          tmem_ld_32x32(tm_s + lane_addr + (cb + 1) * 32, sv[1]);
-          tmem_ld_32x32(tm_dp + lane_addr + (cb + 1) * 32, dv[1]);
-        }
-        tmem_ld_wait();
-        if ((uint32_t)r < q_eff) {
-#pragma unroll
-          for (int cc = 0; cc < 2; ++cc) {
-            const int c = cb + cc;
-            if (c < nchunks) {
-#pragma unroll
-              for (int g = 0; g < 4; ++g) {
-                if ((uint32_t)(c * 32 + g * 8) < n_eff) {
-                  float p[8], ds[8];
-#pragma unroll
-                  for (int k = 0; k < 8; ++k) {
-                    const bool ok = row_ok && (c * 32 + g * 8 + k < kvn);
-                    const float e = ex2_approx(fmaf(__uint_as_float(sv[cc][g * 8 + k]), c2, -my_lse2));
-                    p[k] = ok ? e : 0.f;
-                    ds[k] = ok ? e * (__uint_as_float(dv[cc][g * 8 + k]) - my_d) * scale : 0.f;
-                  }
-                  uint4 u, w;
-                  u.x = pack_bf16x2(p[0], p[1]);
-                  u.y = pack_bf16x2(p[2], p[3]);
-                  u.z = pack_bf16x2(p[4], p[5]);
-                  u.w = pack_bf16x2(p[6], p[7]);
-                  w.x = pack_bf16x2(ds[0], ds[1]);
-                  w.y = pack_bf16x2(ds[2], ds[3]);
-                  w.z = pack_bf16x2(ds[4], ds[5]);
-                  w.w = pack_bf16x2(ds[6], ds[7]);
-                  st_swz(sP, r, c * 4 + g, u);
-                  st_swz(sDS, r, c * 4 + g, w);
-                }
-              }
-            }
-          }
-        }
-      }
-
-      VITK_STAMP(4 + (j * 2 + i) * 4);
-      fence_proxy_async_smem();
-      tc_fence_before();
-      __syncthreads();
-      VITK_STAMP(5 + (j * 2 + i) * 4);
-      if (threadIdx.x == 0) {
-        tc_fence_after();
-        const uint32_t sQ = smem_u32(smem + L::QDO_OFF + i * 2 * TILE_BYTES), sDO = sQ + TILE_BYTES;
-        const uint32_t sK = smem_u32(smem + L::KV_OFF + j * 2 * TILE_BYTES);
-        // dV_j += P^T dO_i ; dK_j += dS^T Q_i   (A MN-major [kv chunks][q rows][64], B MN-major)
-        const uint32_t idesc_t = umma_idesc(TILE, HD, 1, true, true);
-        const int qsteps = (int)q_eff / 16;
-        // descriptors are built once; a k-step only moves the 16-byte-granular start address
-        const uint64_t dP_mn = umma_desc_mnmajor(sP_u, TILE_BYTES), dDO_mn = umma_desc_mnmajor(sDO, TILE_BYTES);
-        const uint64_t dDS_mn = umma_desc_mnmajor(sDS_u, TILE_BYTES), dQ_mn = umma_desc_mnmajor(sQ, TILE_BYTES);
-        const uint64_t dDS_k = umma_desc_kmajor(sDS_u), dK_mn = umma_desc_mnmajor(sK, TILE_BYTES);
-#pragma unroll 4
-        for (int k = 0; k < qsteps; ++k)
-          umma_bf16_ss(tm_dv, dP_mn + (uint64_t)(k * 128), dDO_mn + (uint64_t)(k * 128), idesc_t, (i > 0 || k > 0));
-#pragma unroll 4
-        for (int k = 0; k < qsteps; ++k)
-          umma_bf16_ss(tm_dk, dDS_mn + (uint64_t)(k * 128), dQ_mn + (uint64_t)(k * 128), idesc_t, (i > 0 || k > 0));
-        // dQ_i += dS K_j   (A K-major, B = K_j MN-major)
-        const uint32_t idesc_q = umma_idesc(TILE, HD, 1, false, true);
-        const int ksteps = (int)n_eff / 16;
-#pragma unroll 4
-        for (int k = 0; k < ksteps; ++k)
-          umma_bf16_ss(tm_dq + i * HD, dDS_k + (uint64_t)((k >> 2) * (TILE_BYTES >> 4) + (k & 3) * 2), dK_mn + (uint64_t)(k * 128),
-                       idesc_q, (j > 0 || k > 0));
-        if (i == nt - 1) umma_commit(bar_drain);
-        // next S/dP pair queues right behind on the tensor pipe
-        int ni = i + 1, nj = j;
-        if (ni == nt) { ni = 0; nj = j + 1; }
-        if (nj < nt) issue_s_dp(nj, ni);
-        VITK_STAMP(6 + (j * 2 + i) * 4);
-      }
-    }
-
-    // ---- drain dV_j, dK_j (row = kv index) ----
-    // tcgen05 ops retire in issue order, so this also covers every earlier MMA of this kv tile.
-    mbar_wait(bar_drain, j & 1);
-    tc_fence_after();
-    VITK_STAMP(20 + j * 2);
-    {
-      uint32_t a0[32], a1[32];
-      tmem_ld_32x32(tm_dv + lane_addr, a0);
-      tmem_ld_32x32(tm_dv + lane_addr + 32, a1);
-      tmem_ld_wait();
-      const int kv = j * TILE + r;
-      if (kv < N) store_row_bf16_64(dqkv + ((long long)b * N + kv) * (3 * H * hd) + (2 * H + h) * hd, a0, a1, hd);
-      tmem_ld_32x32(tm_dk + lane_addr, a0);
-      tmem_ld_32x32(tm_dk + lane_addr + 32, a1);
-      tmem_ld_wait();
-      if (kv < N) store_row_bf16_64(dqkv + ((long long)b * N + kv) * (3 * H * hd) + (H + h) * hd, a0, a1, hd);
-    }
-    // NOTE: the next kv tile's dV/dK MMAs (accumulate = 0) are only issued after the next
-    // iteration's __syncthreads, i.e. after every thread finished these TMEM reads.
-    tc_fence_before();
-    VITK_STAMP(21 + j * 2);
-  }
-
-  // ---- drain dQ_i ----
-  tc_fence_after();
-  for (int i = 0; i < nt; ++i) {
-    uint32_t a0[32], a1[32];
-    tmem_ld_32x32(tm_dq + i * HD + lane_addr, a0);
-    tmem_ld_32x32(tm_dq + i * HD + lane_addr + 32, a1);
-    tmem_ld_wait();
-    const int q = i * TILE + r;
-    if (q < N) store_row_bf16_64(dqkv + ((long long)b * N + q) * (3 * H * hd) + h * hd, a0, a1, hd);
-  }
-
-  VITK_STAMP(30);
-  tc_fence_before();
-  __syncthreads();
-  if (warp == 0) {
-    tc_fence_after();
-    tmem_dealloc(tmem_base, 512);
-  }
-  VITK_STAMP(31);
 }
 
 // ================================================================================================
@@ -920,7 +434,7 @@ struct Fwd6Smem {
 
 __global__ void __launch_bounds__(FWD6_THREADS, 1)
 attn_fwd6_kernel(const __grid_constant__ CUtensorMap tm_qkv, const __grid_constant__ CUtensorMap tm_out, float* __restrict__ lse,
-                 int B, int N, int H, float scale, int stagger, float lazy_thr, long long* trace) {
+                 int B, int N, int H, float scale, long long* trace) {
   using L = Fwd6Smem;
   extern __shared__ __align__(1024) uint8_t smem[];
   uint64_t* q_full = reinterpret_cast<uint64_t*>(smem + L::BAR_OFF);  // [2 g + buf] TMA -> MMA g: Q tile landed
@@ -1039,7 +553,7 @@ attn_fwd6_kernel(const __grid_constant__ CUtensorMap tm_qkv, const __grid_consta
     // together: the hand-over between steps (P stores landing, the last S chunk arriving, the row maximum) issues no exp,
     // and in step the MUFU pipe idles through it twice per step.  Group 1 therefore starts half a step late; after that
     // neither group ever waits for the other, so the offset stays.
-    if (g == 1 && stagger)
+    if (g == 1)
       while (*half_step == 0) __nanosleep(64);
     tc_fence_after();
     issue_s(0, 0, 0, real);
@@ -1296,15 +810,9 @@ attn_fwd6_kernel(const __grid_constant__ CUtensorMap tm_qkv, const __grid_consta
           __syncwarp();
           if (lane == 0) mbar_arrive(&s_read[g]);   // the MMA warp may overwrite S with S_{k+2}
           if (active1) {
-            // lazy_thr = 0: the reference of a row is its running maximum (rescale whenever some row of the warp raised it).
-            // lazy_thr > 0 (VITK_ATTN_FWD6_LAZY, log2 units): the row keeps its old reference unless some row of the warp
-            // outgrew it by more than 2^lazy_thr.  P and l stay relative to the SAME reference, so O = sum(P V) / l and
-            // lse = ref * scale + log(l) are the same numbers in exact arithmetic and the O rescale all but disappears
-            // after the first kv tile — but the dominant key of a peaked row no longer has P = 1 exactly, so its bf16
-            // rounding (2^-9 of the largest term) shows in the output: measured max error 2x, rms error +4 % against the
-            // exact reference, bit-identical to torch's bf16 SDPA on this GPU (tools/attn_check.py).  Default: 0.
+            // the reference of a row is its running maximum (rescale whenever some row of the warp raised it)
             m_new = row_max(kvn1, nch1, m);
-            if (__any_sync(0xffffffffu, (m_new - m) * c2 > lazy_thr)) {
+            if (__any_sync(0xffffffffu, (m_new - m) * c2 > 0.f)) {
               alpha = ex2_approx((m - m_new) * c2);   // 0 on the first kv tile of a q tile (m = -inf)
             } else {
               m_new = m;
@@ -1336,15 +844,7 @@ int launch_fwd6(const CUtensorMap& tm, const CUtensorMap& tm_out, float* lse, in
   const int QT = (N + TILE - 1) / TILE;
   const int items = B * H * ((QT + 1) / 2);
   const int grid = items < vitk_num_sms() ? items : vitk_num_sms();
-  static const int stagger = [] {   // VITK_ATTN_FWD6_STAGGER=0: both groups start together (comparison)
-    const char* e = getenv("VITK_ATTN_FWD6_STAGGER");
-    return e ? atoi(e) : 1;
-  }();
-  static const float lazy_thr = [] {   // see the hand-over in the kernel
-    const char* e = getenv("VITK_ATTN_FWD6_LAZY");
-    return e ? (float)atof(e) : 0.f;
-  }();
-  attn_fwd6_kernel<<<grid, FWD6_THREADS, Fwd6Smem::BYTES, s>>>(tm, tm_out, lse, B, N, H, scale, stagger, lazy_thr, g_trace_buf);
+  attn_fwd6_kernel<<<grid, FWD6_THREADS, Fwd6Smem::BYTES, s>>>(tm, tm_out, lse, B, N, H, scale, g_trace_buf);
   return vitk_check_launch("attn_fwd6");
 }
 
@@ -1829,12 +1329,14 @@ attn_bwd4_kernel(const __grid_constant__ CUtensorMap tm_qkv, const __grid_consta
 }
 
 // ================================================================================================
-// Backward, streaming variant for 256 < N <= 640 (ViT-L/16 at 384 px: N = 577): one CTA per (b, h, kv tile j).
+// Backward, streaming: every call but the unmasked 128 < N <= 256 at head_dim <= 64 (attn_bwd4), e.g. N <= 128, ViT-L/16
+// at 384 px (N = 577), a keep mask, wide heads.  One CTA per (b, h, kv tile j).
 // K_j / V_j stay resident, Q_i / dO_i stream through one smem buffer, dV_j / dK_j accumulate in TMEM over the
-// q tiles, and each dQ_ij partial is read out of a TMEM scratch tile and red.add'ed into an fp32 workspace
-// [B, N, H*64] (the q rows are shared by the T CTAs of a head); a small kernel then casts it into dqkv.
+// q tiles, and each dQ_ij partial is read out of a TMEM scratch tile.  With more than one kv tile it is red.add'ed into
+// an fp32 workspace [B, N, H*64] (the q rows are shared by the T CTAs of a head) that a small kernel then casts into
+// dqkv; with one kv tile (dq32 == null) dQ_i0 is final and is stored as bf16 directly.
 // TMEM: S [0,128) | dP [128,256) | dV_j [256,320) | dK_j [320,384) | dQ_ij [384,448)
-// WIDE (64 < head_dim <= 80, used for every N then): operands are [64-column tile][tail tile] pairs (see FwdSmem), S and dP
+// WIDE (64 < head_dim <= 80, used for every N then): operands are [64-column tile][tail tile] pairs (see HDW_MAX), S and dP
 // take one more k-step, dV / dK / dQ have 80 accumulator columns (TMEM: 256 | 336 | 416 .. 496), Q_i / dO_i are single-
 // buffered (192 KB of smem otherwise) and the fp32 dQ workspace keeps 80-wide heads.
 // ================================================================================================
@@ -1866,7 +1368,7 @@ __device__ __forceinline__ void store_row_bf16_tail(__nv_bfloat16* dst, const ui
 
 // Q_i / dO_i are double-buffered (tile i+1 is loading while tile i is processed), S / dP of tile i+1 are issued right
 // behind the dV / dK / dQ MMAs of tile i (their TMEM buffers are free once the threads have read them), so they execute
-// while the threads read dQ_ij out and red.add it.  D = rowsum(O * dO) comes from the workspace (attn_dsum_kernel).
+// while the threads read dQ_ij out.  D = rowsum(O * dO) comes from the workspace (attn_dsum_kernel).
 // No masks: kv rows >= N are TMA zero fill (they reach only discarded dK / dV rows and add 0 to dQ); q rows >= N have
 // Q = dO = 0 and use lse = D = 0.
 template <bool WIDE>
@@ -1894,6 +1396,7 @@ attn_bwd_stream_kernel(const __grid_constant__ CUtensorMap tm_qkv, const __grid_
   const int nchunks = (int)(n_eff + 31) / 32;
 
   if ((smem_u32(smem) & 1023u) != 0) __trap();
+  if (dq32 == nullptr && gridDim.x > 1) __trap();   // a direct bf16 dQ store is final only with one kv tile
   if (threadIdx.x == 32) {
     mbar_init(bar_kv, 1);
     mbar_init(&bar_q[0], 1);
@@ -2058,8 +1561,11 @@ attn_bwd_stream_kernel(const __grid_constant__ CUtensorMap tm_qkv, const __grid_
       tmem_ld_32x32(tm_dq + lane_addr, a0);
       tmem_ld_32x32(tm_dq + lane_addr + 32, a1);
       tmem_ld_wait();
-      float* dst = dq32 + ((long long)b * N + q) * (H * HDW) + h * HDW;
-      if (row_ok) {
+      __nv_bfloat16* dq_row = dqkv + ((long long)b * N + q) * (3 * H * hd) + h * hd;
+      float* dst = dq32 != nullptr ? dq32 + ((long long)b * N + q) * (H * HDW) + h * HDW : nullptr;
+      if (row_ok && dst == nullptr) {
+        store_row_bf16_64(dq_row, a0, a1, hd);
+      } else if (row_ok) {
 #pragma unroll
         for (int g = 0; g < 8; ++g) {
           asm volatile("red.global.add.v4.f32 [%0], {%1, %2, %3, %4};" ::"l"(dst + g * 4), "f"(__uint_as_float(a0[g * 4])),
@@ -2076,7 +1582,9 @@ attn_bwd_stream_kernel(const __grid_constant__ CUtensorMap tm_qkv, const __grid_
         uint32_t a2[16];
         tmem_ld_32x16(tm_dq + lane_addr + 64, a2);
         tmem_ld_wait();
-        if (row_ok) {
+        if (row_ok && dst == nullptr) {
+          store_row_bf16_tail(dq_row + 64, a2, hd - 64);
+        } else if (row_ok) {
 #pragma unroll
           for (int g = 0; g < 4; ++g)
             asm volatile("red.global.add.v4.f32 [%0], {%1, %2, %3, %4};" ::"l"(dst + 64 + g * 4), "f"(__uint_as_float(a2[g * 4])),
@@ -2145,29 +1653,35 @@ __global__ void dq_cast_kernel(const float* __restrict__ dq32, __nv_bfloat16* __
 }
 
 // ================================================================================================
-// Forward, kv-streaming (any N up to ATTN_MAX_N, head_dim <= 64): the attention-dropout forward above 640 tokens.
-// One CTA per (b, h, 128-row q tile) as in attn_fwd_kernel, thread t owns row t, but K_j / V_j stream through a
-// FWDS_STAGES-deep TMA ring (a stage is refilled as soon as P V_j has retired) and O accumulates in TMEM across kv tiles:
-// before P V_j accumulates into it, a warp rescales its 32 rows of O in place if some row raised its maximum.
+// Forward, kv-streaming: every call but the unmasked 128 < N at head_dim <= 64 (attn_fwd4 / attn_fwd6), i.e. N <= 128, a
+// keep mask at any N up to ATTN_MAX_N, and wide heads (N <= WIDE_MAX_N).
+// One CTA per (b, h, 128-row q tile), thread t owns row t; K_j / V_j stream through a FWDS_STAGES-deep TMA ring (a stage
+// is refilled as soon as P V_j has retired) and O accumulates in TMEM across kv tiles: before P V_j accumulates into it,
+// a warp rescales its rows of O in place if some row raised its maximum.
 // Per kv tile: S_j (issued behind P V_{j-1}) -> row max -> wait P V_{j-1} -> refill its stage, rescale O -> exps (+ keep
-// mask) -> P -> smem -> P V_j.  Dropout exactly as attn_fwd_kernel (§4.7): the row sum is taken before the mask, m / keep
-// multiplies the P tile that feeds P V, lse is that of the undropped scores.
-// 112 KB of smem and 256 TMEM columns: two CTAs share an SM, so one's exps overlap the other's MMAs.
+// mask) -> P -> smem -> P V_j.  Dropout (§4.7): the row sum is taken before the mask, m / keep multiplies the P tile that
+// feeds P V, lse is that of the undropped scores.
+// Narrow: 112 KB of smem and 256 TMEM columns, so two CTAs share an SM and one's exps overlap the other's MMAs.
+// WIDE: operands are [tile][tail] pairs (see HDW_MAX), S takes one more k-step, O has 80 columns; 192 KB of smem.
 // ================================================================================================
 constexpr int FWDS_STAGES = 2;
 
+template <bool WIDE>
 struct FwdStreamSmem {
+  static constexpr uint32_t OPB = WIDE ? 2 * TILE_BYTES : TILE_BYTES;   // bytes of one operand tile (+ tail)
   static constexpr uint32_t Q_OFF = 0;
-  static constexpr uint32_t KV_OFF = TILE_BYTES;                               // [stage][K, V]
-  static constexpr uint32_t P_OFF = KV_OFF + FWDS_STAGES * 2 * TILE_BYTES;
+  static constexpr uint32_t KV_OFF = OPB;                                      // [stage][K, V]
+  static constexpr uint32_t P_OFF = KV_OFF + FWDS_STAGES * 2 * OPB;
   static constexpr uint32_t BAR_OFF = P_OFF + 2 * TILE_BYTES;
   static constexpr uint32_t BYTES = BAR_OFF + 128;
 };
 
+template <bool WIDE>
 __global__ void __launch_bounds__(128)
 attn_fwd_stream_kernel(const __grid_constant__ CUtensorMap tm_qkv, __nv_bfloat16* __restrict__ out, float* __restrict__ lse,
                        int N, int H, int hd, float scale, const uint8_t* __restrict__ drop_mask, float drop_scale) {
-  using L = FwdStreamSmem;
+  using L = FwdStreamSmem<WIDE>;
+  constexpr int HDW = WIDE ? HDW_MAX : HD;   // accumulator columns of O
   extern __shared__ __align__(1024) uint8_t smem[];
   uint64_t* bar_q = reinterpret_cast<uint64_t*>(smem + L::BAR_OFF);
   uint64_t* kv_full = bar_q + 1;   // [FWDS_STAGES]
@@ -2196,19 +1710,19 @@ attn_fwd_stream_kernel(const __grid_constant__ CUtensorMap tm_qkv, __nv_bfloat16
   tc_fence_after();
   const uint32_t tmem_base = *tmem_slot;
   const uint32_t tmem_s = tmem_base;         // S_j: 128 columns
-  const uint32_t tmem_o = tmem_base + 128;   // O: 64 columns, accumulated over every kv tile
+  const uint32_t tmem_o = tmem_base + 128;   // O: 64 (80) columns, accumulated over every kv tile
 
   auto load_kv = [&](int j) {   // thread 0 only
     const int st = j % FWDS_STAGES;
-    uint8_t* dst = smem + L::KV_OFF + st * 2 * TILE_BYTES;
-    mbar_arrive_expect_tx(&kv_full[st], 2 * TILE_BYTES);
-    tma_load_head(dst, &tm_qkv, &kv_full[st], H + h, j * TILE, b);
-    tma_load_head(dst + TILE_BYTES, &tm_qkv, &kv_full[st], 2 * H + h, j * TILE, b);
+    uint8_t* dst = smem + L::KV_OFF + st * 2 * L::OPB;
+    mbar_arrive_expect_tx(&kv_full[st], 2 * L::OPB);
+    load_head_tiles<WIDE>(dst, &tm_qkv, &kv_full[st], H + h, j * TILE, b);
+    load_head_tiles<WIDE>(dst + L::OPB, &tm_qkv, &kv_full[st], 2 * H + h, j * TILE, b);
   };
   const uint32_t sQ_u = smem_u32(smem + L::Q_OFF);
   // S_j = Q K_j^T (warp 0: uniform control flow, one elected lane)
   auto issue_s = [&](int j) {
-    const uint32_t sK_u = smem_u32(smem + L::KV_OFF + (j % FWDS_STAGES) * 2 * TILE_BYTES);
+    const uint32_t sK_u = smem_u32(smem + L::KV_OFF + (j % FWDS_STAGES) * 2 * L::OPB);
     mbar_wait(&kv_full[j % FWDS_STAGES], (j / FWDS_STAGES) & 1);
     tc_fence_after();
     const uint32_t idesc = umma_idesc(TILE, roundup16(min(TILE, N - j * TILE)), 1, false, false);
@@ -2216,6 +1730,7 @@ attn_fwd_stream_kernel(const __grid_constant__ CUtensorMap tm_qkv, __nv_bfloat16
     if (elect_one()) {
 #pragma unroll
       for (int k = 0; k < HD / 16; ++k) umma_bf16_ss(tmem_s, qd + (uint64_t)(k * 2), kd + (uint64_t)(k * 2), idesc, k > 0);
+      if (WIDE) umma_bf16_ss(tmem_s, umma_desc_kmajor(sQ_u + TILE_BYTES), umma_desc_kmajor(sK_u + TILE_BYTES), idesc, true);
       umma_commit(bar_s);
     }
     __syncwarp();
@@ -2223,8 +1738,8 @@ attn_fwd_stream_kernel(const __grid_constant__ CUtensorMap tm_qkv, __nv_bfloat16
 
   if (threadIdx.x == 0) {
     tma_prefetch_desc(&tm_qkv);
-    mbar_arrive_expect_tx(bar_q, TILE_BYTES);
-    tma_load_head(smem + L::Q_OFF, &tm_qkv, bar_q, h, q0, b);
+    mbar_arrive_expect_tx(bar_q, L::OPB);
+    load_head_tiles<WIDE>(smem + L::Q_OFF, &tm_qkv, bar_q, h, q0, b);
     for (int j = 0; j < FWDS_STAGES && j < nkv; ++j) load_kv(j);
   }
   if (warp == 0) {
@@ -2289,6 +1804,14 @@ attn_fwd_stream_kernel(const __grid_constant__ CUtensorMap tm_qkv, __nv_bfloat16
             tmem_st_32x16(tmem_o + lane_addr + hh * 32 + u * 16, t16);
           }
         }
+        if (WIDE) {
+          uint32_t t16[16];
+          tmem_ld_32x16(tmem_o + lane_addr + 64, t16);
+          tmem_ld_wait();
+#pragma unroll
+          for (int i = 0; i < 16; ++i) t16[i] = __float_as_uint(__uint_as_float(t16[i]) * alpha);
+          tmem_st_32x16(tmem_o + lane_addr + 64, t16);
+        }
         tmem_st_wait();
       }
     }
@@ -2337,9 +1860,9 @@ attn_fwd_stream_kernel(const __grid_constant__ CUtensorMap tm_qkv, __nv_bfloat16
     __syncthreads();
     if (warp == 0) {
       tc_fence_after();
-      const uint32_t idesc = umma_idesc(TILE, HD, 1, false, true);  // A = P K-major, B = V MN-major
+      const uint32_t idesc = umma_idesc(TILE, HDW, 1, false, true);  // A = P K-major, B = V MN-major (tail = second 64-wide chunk)
       const int ksteps = (int)n_eff / 16;
-      const uint32_t sV_u = smem_u32(smem + L::KV_OFF + (j % FWDS_STAGES) * 2 * TILE_BYTES + TILE_BYTES);
+      const uint32_t sV_u = smem_u32(smem + L::KV_OFF + (j % FWDS_STAGES) * 2 * L::OPB + L::OPB);
       const uint64_t pdesc = umma_desc_kmajor(sP_u), vdesc = umma_desc_mnmajor(sV_u, TILE_BYTES);
       if (elect_one()) {
 #pragma unroll 4
@@ -2357,9 +1880,10 @@ attn_fwd_stream_kernel(const __grid_constant__ CUtensorMap tm_qkv, __nv_bfloat16
   mbar_wait(bar_o, (nkv - 1) & 1);
   tc_fence_after();
   {
-    uint32_t a0[32], a1[32];
+    uint32_t a0[32], a1[32], t16[16];
     tmem_ld_32x32(tmem_o + lane_addr, a0);
     tmem_ld_32x32(tmem_o + lane_addr + 32, a1);
+    if (WIDE) tmem_ld_32x16(tmem_o + lane_addr + 64, t16);
     tmem_ld_wait();
     if (qrow < N) {
       const float inv = 1.0f / l_run;
@@ -2368,7 +1892,13 @@ attn_fwd_stream_kernel(const __grid_constant__ CUtensorMap tm_qkv, __nv_bfloat16
         a0[i] = __float_as_uint(__uint_as_float(a0[i]) * inv);
         a1[i] = __float_as_uint(__uint_as_float(a1[i]) * inv);
       }
-      store_row_bf16_64(out + ((long long)b * N + qrow) * (H * hd) + h * hd, a0, a1, hd);
+      __nv_bfloat16* orow = out + ((long long)b * N + qrow) * (H * hd) + h * hd;
+      store_row_bf16_64(orow, a0, a1, hd);
+      if (WIDE) {
+#pragma unroll
+        for (int i = 0; i < 16; ++i) t16[i] = __float_as_uint(__uint_as_float(t16[i]) * inv);
+        store_row_bf16_tail(orow + 64, t16, hd - 64);
+      }
       if (lse) lse[((long long)b * H + h) * N + qrow] = m_run * scale + __logf(l_run);
     }
   }
@@ -2381,33 +1911,19 @@ attn_fwd_stream_kernel(const __grid_constant__ CUtensorMap tm_qkv, __nv_bfloat16
   }
 }
 
+template <bool WIDE>
 int launch_fwd_stream(const CUtensorMap& tm, void* out, float* lse, int B, int N, int H, int hd, float scale, cudaStream_t s,
                       const uint8_t* drop_mask, float drop_scale) {
+  using L = FwdStreamSmem<WIDE>;
   static bool attr_set = false;
   if (!attr_set) {
-    cudaError_t e = cudaFuncSetAttribute(attn_fwd_stream_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)FwdStreamSmem::BYTES);
+    cudaError_t e = cudaFuncSetAttribute(attn_fwd_stream_kernel<WIDE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)L::BYTES);
     if (e != cudaSuccess) return vitk_set_error(VITK_ERR_CUDA, "attn_fwd_stream: cudaFuncSetAttribute: %s", cudaGetErrorString(e));
     attr_set = true;
   }
   dim3 grid((N + TILE - 1) / TILE, H, B);
-  attn_fwd_stream_kernel<<<grid, 128, FwdStreamSmem::BYTES, s>>>(tm, (__nv_bfloat16*)out, lse, N, H, hd, scale, drop_mask, drop_scale);
+  attn_fwd_stream_kernel<WIDE><<<grid, 128, L::BYTES, s>>>(tm, (__nv_bfloat16*)out, lse, N, H, hd, scale, drop_mask, drop_scale);
   return vitk_check_launch("attn_fwd_stream");
-}
-
-template <int T, bool WIDE = false>
-int launch_fwd(const CUtensorMap& tm, void* out, float* lse, int B, int N, int H, int hd, float scale, cudaStream_t s,
-               const uint8_t* drop_mask = nullptr, float drop_scale = 1.f) {
-  auto kern = attn_fwd_kernel<T, WIDE>;
-  using L = FwdSmem<T, WIDE>;
-  static bool attr_set = false;
-  if (!attr_set) {
-    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)L::BYTES);
-    if (e != cudaSuccess) return vitk_set_error(VITK_ERR_CUDA, "attn_fwd: cudaFuncSetAttribute: %s", cudaGetErrorString(e));
-    attr_set = true;
-  }
-  dim3 grid((N + TILE - 1) / TILE, H, B);
-  kern<<<grid, 128, L::BYTES, s>>>(tm, (__nv_bfloat16*)out, lse, N, H, hd, scale, drop_mask, drop_scale, g_trace_buf);
-  return vitk_check_launch("attn_fwd");
 }
 
 // The attention tensors are mapped for TMA as (head_dim, head slot, token, image): a [rows][64] box of one head slot
@@ -2421,7 +1937,14 @@ int make_head_tmap(CUtensorMap* tm, const void* base, int slots, int hd, int N, 
 }
 
 bool head_dim_ok(int hd) { return hd >= 16 && hd <= HDW_MAX && hd % 8 == 0; }
-constexpr int WIDE_MAX_N = 2 * TILE;   // heads wider than 64: the forward keeps every K / V tile (+ tail) of a head in smem
+constexpr int WIDE_MAX_N = 2 * TILE;   // heads wider than 64 (my_vit_xs: N = 197) are built and tested up to 256 tokens
+
+// The backward runs attn_bwd4 for the unmasked 128 < N <= 256 at head_dim <= 64 and the streaming kernel for every other call.
+bool use_bwd4(int N, int hd, bool masked) { return N > TILE && N <= 2 * TILE && hd <= HD && !masked; }
+
+// Columns per head of the fp32 dQ accumulator in the backward workspace, 0 when the call needs none: the streaming kernel
+// red.adds dQ partials into it when it runs over more than one kv tile.
+int dq32_pitch(int N, int hd, bool masked) { return N <= TILE || use_bwd4(N, hd, masked) ? 0 : (hd > HD ? HDW_MAX : HD); }
 
 }  // namespace
 
@@ -2437,45 +1960,15 @@ static int attn_fwd_impl(const void* qkv, void* out, float* lse, int32_t B, int3
   CUtensorMap tm, tm_out;
   int rc = make_head_tmap(&tm, qkv, 3 * H, hd, N, B, TILE);
   if (rc) return rc;
-  const int T = (N + TILE - 1) / TILE;
   cudaStream_t s = (cudaStream_t)stream;
-  if (hd > HD)   // my_vit_xs (head_dim 72): the tiled kernel with [tile][tail] operands
-    return T == 1 ? launch_fwd<1, true>(tm, out, lse, B, N, H, hd, scale, s, drop_mask, drop_scale)
-                  : launch_fwd<2, true>(tm, out, lse, B, N, H, hd, scale, s, drop_mask, drop_scale);
-  // VITK_ATTN_FWD: unset = attn_fwd4 (whole score row in TMEM, one thread per row) for 128 < N <= 256, attn_fwd6 (kv loop,
-  // score MMA off the softmax's critical path) above that, the tiled one-CTA-per-q-tile kernel for N <= 128 and, with a
-  // keep mask, for N <= 640; the kv-streaming kernel for a keep mask above 640 tokens.
-  // "1" = tiled kernel everywhere (the kv-streaming kernel above 640 tokens); "6" = attn_fwd6 for every unmasked N > 128;
-  // "7" = the kv-streaming kernel for every N, with or without a mask
-  static const int variant = [] {
-    const char* e = getenv("VITK_ATTN_FWD");
-    return e ? atoi(e) : 0;
-  }();
-  const bool fwd6_ok = drop_mask == nullptr && (variant == 0 || variant == 6);
-  if (variant == 7 || (T > FWD_MAX_T && !fwd6_ok))
-    return launch_fwd_stream(tm, out, lse, B, N, H, hd, scale, s, drop_mask, drop_scale);
-  if (drop_mask != nullptr) {   // attention dropout: the tiled kernel up to 640 tokens (the mask is read per element)
-    switch (T) {
-      case 1: return launch_fwd<1>(tm, out, lse, B, N, H, hd, scale, s, drop_mask, drop_scale);
-      case 2: return launch_fwd<2>(tm, out, lse, B, N, H, hd, scale, s, drop_mask, drop_scale);
-      case 3: return launch_fwd<3>(tm, out, lse, B, N, H, hd, scale, s, drop_mask, drop_scale);
-      case 4: return launch_fwd<4>(tm, out, lse, B, N, H, hd, scale, s, drop_mask, drop_scale);
-      default: return launch_fwd<5>(tm, out, lse, B, N, H, hd, scale, s, drop_mask, drop_scale);
-    }
-  }
-  if (fwd6_ok && T >= 2) {
-    rc = make_head_tmap(&tm_out, out, H, hd, N, B, TILE);
-    if (rc) return rc;
-    if (variant == 0 && T == 2) return launch_fwd4(tm, tm_out, lse, B, N, H, scale, s);
-    return launch_fwd6(tm, tm_out, lse, B, N, H, scale, s);
-  }
-  switch (T) {
-    case 1: return launch_fwd<1>(tm, out, lse, B, N, H, hd, scale, s);
-    case 2: return launch_fwd<2>(tm, out, lse, B, N, H, hd, scale, s);
-    case 3: return launch_fwd<3>(tm, out, lse, B, N, H, hd, scale, s);
-    case 4: return launch_fwd<4>(tm, out, lse, B, N, H, hd, scale, s);
-    default: return launch_fwd<5>(tm, out, lse, B, N, H, hd, scale, s);
-  }
+  // the kv-streaming kernel for wide heads, a keep mask and N <= 128; attn_fwd4 (whole score row in TMEM, one thread per
+  // row) for 128 < N <= 256; attn_fwd6 (kv loop, score MMA off the softmax's critical path) above that
+  if (hd > HD) return launch_fwd_stream<true>(tm, out, lse, B, N, H, hd, scale, s, drop_mask, drop_scale);
+  if (drop_mask != nullptr || N <= TILE) return launch_fwd_stream<false>(tm, out, lse, B, N, H, hd, scale, s, drop_mask, drop_scale);
+  rc = make_head_tmap(&tm_out, out, H, hd, N, B, TILE);
+  if (rc) return rc;
+  if (N <= 2 * TILE) return launch_fwd4(tm, tm_out, lse, B, N, H, scale, s);
+  return launch_fwd6(tm, tm_out, lse, B, N, H, scale, s);
 }
 
 extern "C" int vitk_attn_fwd(const void* qkv, void* out, float* lse, int32_t B, int32_t N, int32_t H, int32_t head_dim,
@@ -2495,18 +1988,13 @@ static int64_t dsum_bytes(int32_t B, int32_t N, int32_t H) {
   return (((int64_t)B * H * N * (int64_t)sizeof(float)) + 255) / 256 * 256;
 }
 
+// D = rowsum(O * dO) [B, H, N] fp32, plus the fp32 dQ accumulator [B, N, H, dq32_pitch] (heads padded to the tile width)
 extern "C" int64_t vitk_attn_bwd_workspace_bytes(int32_t B, int32_t N, int32_t H, int32_t head_dim) {
-  // D = rowsum(O * dO) [B, H, N] fp32, plus (N > 256, or head_dim > 64) the fp32 dQ accumulator [B, N, H, 64 | 80] (heads padded
-  // to the tile width)
-  int64_t bytes = dsum_bytes(B, N, H);
-  if (head_dim > HD) bytes += (int64_t)B * N * H * HDW_MAX * (int64_t)sizeof(float);   // wide heads: streaming kernel for every N
-  else if (N > BWD_MAX_T * TILE) bytes += (int64_t)B * N * H * HD * (int64_t)sizeof(float);
-  return bytes;
+  return dsum_bytes(B, N, H) + (int64_t)B * N * H * dq32_pitch(N, head_dim, false) * (int64_t)sizeof(float);
 }
 
 extern "C" int64_t vitk_attn_bwd_dropout_workspace_bytes(int32_t B, int32_t N, int32_t H, int32_t head_dim) {
-  // attention dropout runs the streaming backward for every N: D plus the fp32 dQ accumulator
-  return dsum_bytes(B, N, H) + (int64_t)B * N * H * (head_dim > HD ? HDW_MAX : HD) * (int64_t)sizeof(float);
+  return dsum_bytes(B, N, H) + (int64_t)B * N * H * dq32_pitch(N, head_dim, true) * (int64_t)sizeof(float);
 }
 
 static int attn_bwd_impl(const void* qkv, const void* out, const void* dout, const float* lse, void* dqkv, void* workspace, int32_t B,
@@ -2527,9 +2015,7 @@ static int attn_bwd_impl(const void* qkv, const void* out, const void* dout, con
   if (rc) return rc;
   static bool attr_set = false;
   if (!attr_set) {
-    cudaError_t e = cudaFuncSetAttribute(attn_bwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)BwdSmem::BYTES);
-    if (e == cudaSuccess)
-      e = cudaFuncSetAttribute(attn_bwd4_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Bwd3Smem::BYTES);
+    cudaError_t e = cudaFuncSetAttribute(attn_bwd4_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Bwd3Smem::BYTES);
     if (e == cudaSuccess)
       e = cudaFuncSetAttribute(attn_bwd_stream_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)BwdStreamSmem<false>::BYTES);
     if (e == cudaSuccess)
@@ -2541,41 +2027,12 @@ static int attn_bwd_impl(const void* qkv, const void* out, const void* dout, con
   VITK_REQUIRE(workspace != nullptr && ((uintptr_t)workspace & 15) == 0, VITK_ERR_ALIGN,
                "attn_bwd: needs a 16-byte aligned workspace of vitk_attn_bwd_workspace_bytes()");
   float* dsum = reinterpret_cast<float*>(workspace);
-  float* dq32 = reinterpret_cast<float*>(reinterpret_cast<uint8_t*>(workspace) + dsum_bytes(B, N, H));
-  {
-    const long long rows = (long long)B * N;
-    attn_dsum_kernel<<<(unsigned)((rows + 7) / 8), 256, 0, st>>>((const __nv_bfloat16*)out, (const __nv_bfloat16*)dout, dsum,
-                                                                 rows, N, H, hd);
-    rc = vitk_check_launch("attn_dsum");
-    if (rc) return rc;
-  }
-  if (N > BWD_MAX_T * TILE || hd > HD || drop_mask != nullptr) {
-    // one CTA per (b, h, kv tile): dQ partials are red.add'ed into the fp32 workspace (156 of the ~820 us per layer at
-    // ViT-L/384, B = 64, H = 16, N = 577; ~90 us are the memset / cast / D kernels around it)
-    const long long rows = (long long)B * N;
-    const int pitch = hd > HD ? HDW_MAX : HD;
-    cudaError_t e = cudaMemsetAsync(dq32, 0, (size_t)rows * H * pitch * sizeof(float), st);
-    if (e != cudaSuccess) return vitk_set_error(VITK_ERR_CUDA, "attn_bwd: memset: %s", cudaGetErrorString(e));
-    dim3 grid((N + TILE - 1) / TILE, H, B);
-    if (hd > HD)
-      attn_bwd_stream_kernel<true><<<grid, 128, BwdStreamSmem<true>::BYTES, st>>>(tm_qkv, tm_do, dsum, lse, (__nv_bfloat16*)dqkv, dq32,
-                                                                                  N, H, hd, scale, drop_mask, drop_scale);
-    else
-      attn_bwd_stream_kernel<false><<<grid, 128, BwdStreamSmem<false>::BYTES, st>>>(tm_qkv, tm_do, dsum, lse, (__nv_bfloat16*)dqkv,
-                                                                                    dq32, N, H, hd, scale, drop_mask, drop_scale);
-    rc = vitk_check_launch("attn_bwd_stream");
-    if (rc) return rc;
-    const long long n8 = rows * H * (hd / 8);
-    dq_cast_kernel<<<(unsigned)((n8 + 255) / 256), 256, 0, st>>>(dq32, (__nv_bfloat16*)dqkv, rows, H, hd, pitch);
-    return vitk_check_launch("attn_bwd_dq_cast");
-  }
-  // VITK_ATTN_BWD: unset = warp-specialised persistent kernel for 128 < N <= 256, single-warpgroup kernel for N <= 128;
-  // "1" = single-warpgroup kernel everywhere
-  static const int variant = [] {
-    const char* e = getenv("VITK_ATTN_BWD");
-    return e ? atoi(e) : 0;
-  }();
-  if (variant == 0 && N > TILE) {
+  const long long rows = (long long)B * N;
+  attn_dsum_kernel<<<(unsigned)((rows + 7) / 8), 256, 0, st>>>((const __nv_bfloat16*)out, (const __nv_bfloat16*)dout, dsum, rows,
+                                                               N, H, hd);
+  rc = vitk_check_launch("attn_dsum");
+  if (rc) return rc;
+  if (use_bwd4(N, hd, drop_mask != nullptr)) {
     const int items = B * H;
     const int g3 = items < vitk_num_sms() ? items : vitk_num_sms();
     CUtensorMap tm_dqkv;   // 32-row boxes: one per warp-level read-out of dQ / dK / dV
@@ -2584,9 +2041,27 @@ static int attn_bwd_impl(const void* qkv, const void* out, const void* dout, con
     attn_bwd4_kernel<<<g3, BWD3_THREADS, Bwd3Smem::BYTES, st>>>(tm_qkv, tm_do, tm_dqkv, dsum, lse, B, N, H, scale, g_trace_buf);
     return vitk_check_launch("attn_bwd4");
   }
-  dim3 grid(H, B);
-  attn_bwd_kernel<<<grid, 128, BwdSmem::BYTES, st>>>(tm_qkv, tm_do, dsum, lse, (__nv_bfloat16*)dqkv, N, H, hd, scale, g_trace_buf);
-  return vitk_check_launch("attn_bwd");
+  // one CTA per (b, h, kv tile); over more than one kv tile the dQ partials are red.add'ed into the fp32 workspace (156 of
+  // the ~820 us per layer at ViT-L/384, B = 64, H = 16, N = 577; ~90 us are the memset / cast / D kernels around it)
+  const int pitch = dq32_pitch(N, hd, drop_mask != nullptr);
+  float* dq32 = nullptr;
+  if (pitch > 0) {
+    dq32 = reinterpret_cast<float*>(reinterpret_cast<uint8_t*>(workspace) + dsum_bytes(B, N, H));
+    cudaError_t e = cudaMemsetAsync(dq32, 0, (size_t)rows * H * pitch * sizeof(float), st);
+    if (e != cudaSuccess) return vitk_set_error(VITK_ERR_CUDA, "attn_bwd: memset: %s", cudaGetErrorString(e));
+  }
+  dim3 grid((N + TILE - 1) / TILE, H, B);
+  if (hd > HD)
+    attn_bwd_stream_kernel<true><<<grid, 128, BwdStreamSmem<true>::BYTES, st>>>(tm_qkv, tm_do, dsum, lse, (__nv_bfloat16*)dqkv, dq32,
+                                                                                N, H, hd, scale, drop_mask, drop_scale);
+  else
+    attn_bwd_stream_kernel<false><<<grid, 128, BwdStreamSmem<false>::BYTES, st>>>(tm_qkv, tm_do, dsum, lse, (__nv_bfloat16*)dqkv,
+                                                                                  dq32, N, H, hd, scale, drop_mask, drop_scale);
+  rc = vitk_check_launch("attn_bwd_stream");
+  if (rc || pitch == 0) return rc;
+  const long long n8 = rows * H * (hd / 8);
+  dq_cast_kernel<<<(unsigned)((n8 + 255) / 256), 256, 0, st>>>(dq32, (__nv_bfloat16*)dqkv, rows, H, hd, pitch);
+  return vitk_check_launch("attn_bwd_dq_cast");
 }
 
 extern "C" int vitk_attn_bwd(const void* qkv, const void* out, const void* dout, const float* lse, void* dqkv,
