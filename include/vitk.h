@@ -23,7 +23,7 @@
 extern "C" {
 #endif
 
-#define VITK_ABI_VERSION 4
+#define VITK_ABI_VERSION 5
 
 enum vitk_status {
   VITK_STATUS_OK = 0,
@@ -56,14 +56,8 @@ enum vitk_epilogue {
   VITK_EPI_F32 = 3,    /* out_f32 = acc + bias                                        (head)       */
   VITK_EPI_DGELU = 4,  /* out_bf16 = rowscale[m/g] * acc * aux_bf16[m,n], aux = gelu'(h) (fc2 dgrad)  */
   VITK_EPI_ATOMIC = 5, /* out_f32 += acc   via red.global.add (split-K)               (wgrad)      */
-  VITK_EPI_PATCH = 6,  /* out_f32[b*(P+prefix)+prefix+t, n] = acc + bias[n] + pos[prefix+t, n]; rows are patches (b, t), or
+  VITK_EPI_PATCH = 6   /* out_f32[b*(P+prefix)+prefix+t, n] = acc + bias[n] + pos[prefix+t, n]; rows are patches (b, t), or
                           the padded rows (b, gy, gx') of an a_image operand                         */
-  /* GELU / x GELU' with the derivative kept in ONE byte per element: aux_u8 = round(200 * gelu'(h)) + 27, i.e. a fixed
-   * grid of step 0.005 over [-0.135, 1.14] that represents gelu'(h) = 0 and 1 exactly (|error| <= 0.0025: what a bf16
-   * rounding costs at gelu' ~ 1); fc1 writes 3 instead of 4 bytes per hidden element, fc2's dgrad reads 1 instead of 2.
-   * N must be a multiple of 256; aux is uint8 [M, N] with ld_aux in elements (= bytes, multiple of 16). */
-  VITK_EPI_GELU_Q8 = 7,
-  VITK_EPI_DGELU_Q8 = 8
 };
 
 typedef struct vitk_gemm_args {
@@ -75,7 +69,7 @@ typedef struct vitk_gemm_args {
   int32_t epilogue;    /* enum vitk_epilogue                                                       */
   void* out;           /* bf16 or f32 depending on the epilogue                                    */
   int64_t ld_out;
-  void* aux;           /* GELU: activation-derivative output (bf16; uint8 for the _Q8 codes); DGELU: the same buffer as input */
+  void* aux;           /* GELU: activation-derivative output (bf16); DGELU: the same buffer as input                    */
   int64_t ld_aux;
   const float* bias;   /* [N] or NULL                                                              */
   const float* resid;  /* RESID: fp32 [M, N] residual stream input                                 */

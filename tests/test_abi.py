@@ -99,6 +99,14 @@ def test_argument_validation_reports_through_error_slot(lib):
     rc = lib.vitk_gemm_bf16(ctypes.byref(args), None)
     assert rc < 0 and b"empty problem" in lib.vitk_last_error()
     assert lib.vitk_gemm_bf16(None, None) < 0
+    # an epilogue code outside enum vitk_epilogue is refused by the dispatcher; the pointers are fake but 16-byte
+    # aligned, so the call gets past the entry checks and still makes no CUDA call
+    args = GemmArgs()
+    args.A = args.B = args.out = 256
+    args.lda = args.ldb = args.ld_out = 64
+    args.M, args.N, args.K, args.epilogue = 128, 64, 64, 7
+    rc = lib.vitk_gemm_bf16(ctypes.byref(args), None)
+    assert rc == -6 and b"epi=7" in lib.vitk_last_error()   # VITK_STATUS_UNSUPPORTED
     rc = lib.vitk_attn_fwd(None, None, None, 1, 16, 1, 96, ctypes.c_float(1.0), None)
     assert rc == -6 and b"head_dim" in lib.vitk_last_error()  # VITK_STATUS_UNSUPPORTED (wider than a head tile + its tail)
     rc = lib.vitk_attn_fwd(None, None, None, 1, 300, 1, 72, ctypes.c_float(1.0), None)

@@ -48,6 +48,23 @@ def test_forward_logits(cuda_device, name, kw):
     assert elem_err(got, want) < 3e-2 and rms_err(got, want) < 1e-2
 
 
+@pytest.mark.parametrize("name,kw", [
+    ("vit_tiny_patch16_224", dict(num_classes=1000)),                 # the image is the patch GEMM's operand
+    ("vit_small_patch16_224", dict(num_classes=100, patch_size=8)),   # im2col PatchEmbed, N = 785
+])
+def test_bf16_image_matches_its_fp32_copy(cuda_device, name, kw):
+    """A bf16 image batch gives the same logits, bit for bit, as the fp32 batch that holds the same values."""
+    from vision_transformers_torch_xla_b200.models import create_model
+
+    torch.manual_seed(0)
+    model = create_model(name, **kw).to(cuda_device).eval()
+    x = torch.randn(4, 3, 224, 224, device=cuda_device).bfloat16()
+    with torch.no_grad():
+        got = model(x)
+        want = model(x.float())
+    assert torch.equal(got, want)
+
+
 def test_per_layer_activations_and_grads(cuda_device):
     ref, mine = _pair("vit_tiny_patch16_224", cuda_device, num_classes=1000, global_pool="avg")
     ref.train()

@@ -53,7 +53,7 @@ def row(name, flops, fn, lib):
 for D in DIMS:
     M = int(os.environ.get("GB_M", ROWS.get(D, 50432)))
     F = 4 * D
-    print(f"---- D = {D}, F = {F}, M = B*N = {M}  (GB_BN={BN}, GB_SPLITS={SPLITS}, VITK_GEMM_192_2CTA={os.environ.get('VITK_GEMM_192_2CTA', '1')}) ----")
+    print(f"---- D = {D}, F = {F}, M = B*N = {M}  (GB_BN={BN}, GB_SPLITS={SPLITS}) ----")
     xD = [torch.randn(M, D, device=dev).bfloat16() for _ in range(R)]
     xF = [torch.randn(M, F, device=dev).bfloat16() for _ in range(R)]
     x3 = [torch.randn(M, 3 * D, device=dev).bfloat16() for _ in range(R)]

@@ -10,10 +10,9 @@ timeout 900 python bench.py --steps 50 --warmup 5 --breakdown > gpurun_out/r02_b
 for c in 2 4 5; do
   timeout 900 python bench.py --config $c --steps 50 --warmup 5 --breakdown > gpurun_out/r02_bench_c$c.json 2> gpurun_out/r02_bench_c$c.err; echo "c$c rc=$?" >> gpurun_out/rc.txt
 done
-VITK_PATCH_EMBED=patchify timeout 900 python bench.py --steps 50 --warmup 5 --no-cpu-baseline --no-e2e > gpurun_out/c3_patchify.json 2>/dev/null
 python - <<'PY'
 import json
-for f in ('r02_bench_c3','c3_patchify','r02_bench_c2','r02_bench_c4','r02_bench_c5'):
+for f in ('r02_bench_c3','r02_bench_c2','r02_bench_c4','r02_bench_c5'):
     try:
         d=json.load(open('gpurun_out/%s.json'%f)); r=d['roofline']
         print(f, round(d['value'],1), 'img/s', round(d['ms_per_step'],2), 'ms  e2e', d['e2e'] and round(d['e2e']['value'],1), ' clk', d['clocks']['sm_mhz'], ' frac_sust %.3f'%d['model_flops']['frac_of_measured_sustained'], ' roof %.3f %s %.1fus'%(r['frac'], r['kernel'][-30:], r['us_per_launch']), 'teacher', d['config']['teacher_fwd_ms_per_step'], 'cpu', d.get('cpu_baseline',{}).get('value'))

@@ -16,11 +16,11 @@ from typing import Optional
 import torch
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
-#: VITK_LIB: another build of the same sources (A/B experiments, e.g. tools/gpu_gelu_fast.sh); the ABI and build-id checks
+#: VITK_LIB: another build of the same sources (A/B experiments); the ABI and build-id checks
 #: below still apply (VITK_ALLOW_STALE_LIB=1 for a build with different compile-time flags)
 LIB_PATH = os.environ.get("VITK_LIB") or os.path.join(_HERE, "libvitk.so")
 
-EPI_BF16, EPI_GELU, EPI_RESID, EPI_F32, EPI_DGELU, EPI_ATOMIC, EPI_PATCH, EPI_GELU_Q8, EPI_DGELU_Q8 = range(9)
+EPI_BF16, EPI_GELU, EPI_RESID, EPI_F32, EPI_DGELU, EPI_ATOMIC, EPI_PATCH = range(7)
 
 #: every symbol include/vitk.h declares (tests check the library exports exactly these)
 EXPORTED_SYMBOLS = (
@@ -34,7 +34,7 @@ EXPORTED_SYMBOLS = (
     "vitk_attn_fwd_dropout", "vitk_attn_bwd_dropout", "vitk_attn_bwd_dropout_workspace_bytes",
 )
 
-ABI_VERSION = 4
+ABI_VERSION = 5
 #: the files whose sha256 csrc/Makefile bakes into the library (same list, same order)
 _BUILD_SOURCES = ("csrc/vitk_host.cu", "csrc/vitk_gemm.cu", "csrc/vitk_attn.cu", "csrc/vitk_norm.cu",
                   "csrc/vitk_elementwise.cu", "csrc/vitk_common.cuh", "csrc/vitk_internal.h", "../include/vitk.h")
@@ -328,10 +328,10 @@ def gemm(a: torch.Tensor, b: torch.Tensor, out: torch.Tensor, *, M: int, N: int,
     for t, nm in ((bias, "bias"), (resid, "resid"), (rowscale, "rowscale"), (colscale, "colscale"), (pos, "pos")):
         if t is not None:
             _req(t, torch.float32, f"gemm {nm}")
-    if epilogue in (EPI_GELU, EPI_DGELU, EPI_GELU_Q8, EPI_DGELU_Q8):
+    if epilogue in (EPI_GELU, EPI_DGELU):
         if aux is None:
             raise VitkError("gemm: the GELU epilogues need the aux (derivative) buffer")
-        _req(aux, torch.uint8 if epilogue in (EPI_GELU_Q8, EPI_DGELU_Q8) else torch.bfloat16, "gemm aux")
+        _req(aux, torch.bfloat16, "gemm aux")
     role = "wgrad" if epilogue == EPI_ATOMIC else ("dgrad" if b_mn else "fprop")
     with _Timed(f"gemm.{role}.epi{epilogue} {M}x{N}x{K}", 2.0 * M * N * K):
         _check(load().vitk_gemm_bf16(ctypes.byref(args), _stream()), "vitk_gemm_bf16")

@@ -42,8 +42,6 @@ int vitk_make_tmap_3d(CUtensorMap* out, const void* base, int elem_bytes, uint64
 int vitk_make_tmap_4d(CUtensorMap* out, const void* base, int elem_bytes, uint64_t d0, uint64_t d1, uint64_t d2, uint64_t d3,
                       uint64_t ld1_elems, uint64_t ld2_elems, uint64_t ld3_elems, uint32_t b0, uint32_t b1, uint32_t b2,
                       uint32_t b3, int swizzle_bytes = 128);
-int vitk_make_tmap_2d_u8(CUtensorMap* out, const void* base, uint64_t inner, uint64_t outer, uint64_t ld_bytes,
-                         uint32_t box_inner, uint32_t box_outer);
 int vitk_make_tmap_2d_sw64(CUtensorMap* out, const void* base, int elem_bytes, uint64_t inner, uint64_t outer,
                            uint64_t ld_elems, uint32_t box_inner, uint32_t box_outer);
 int vitk_num_sms();
@@ -457,32 +455,11 @@ __device__ __forceinline__ float ex2_approx(float x) {
   asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x));
   return y;
 }
-__device__ __forceinline__ float tanh_approx(float x) {
-  float y;
-  asm("tanh.approx.f32 %0, %1;" : "=f"(y) : "f"(x));
-  return y;
-}
-// Exact-erf GELU and its derivative from ONE MUFU op per element (the fc1 epilogue is instruction-bound, not
-// tensor-bound: the tile's MMAs take 6144 cycles, the Abramowitz-Stegun form needed 2 MUFU + ~17 FP32 ops per element):
-//   Phi(h) = 0.5 (1 + erf(h / sqrt2))  ~=  0.5 + 0.5 tanh(h P(h^2)),   P(s) = c0 + c1 s + c2 s^2   (s clamped to 49),
-// coefficients fitted (minimax over |h| <= 7, tools/fit_gelu.py) so that
-//   |h Phi(h) - gelu(h)| <= 3.4e-5   and   |d/dh [h Phi(h)] - gelu'(h)| <= 9.3e-5   (before the 2^-11 relative error of
-// tanh.approx), i.e. two orders of magnitude below the bf16 rounding of the outputs.  The derivative is the analytic
-// derivative of the approximant:  gelu'(h) ~= Phi + 0.5 h (1 - T^2) (c0 + 3 c1 s + 5 c2 s^2).
-__device__ __forceinline__ void gelu_fwd_bwd_fast(float h, float& act, float& deriv) {
-  constexpr float c0 = 0.79745014f, c1 = 0.0369949746f, c2 = -0.00034728153f;
-  const float s = fminf(h * h, 49.0f);
-  const float P = fmaf(fmaf(c2, s, c1), s, c0);
-  const float T = tanh_approx(h * P);
-  const float cdf = fmaf(0.5f, T, 0.5f);
-  const float gp = fmaf(fmaf(2.5f * c2, s, 1.5f * c1), s, 0.5f * c0);   // 0.5 * d/dh [h P(h^2)]
-  act = h * cdf;
-  deriv = fmaf(h * fmaf(-T, T, 1.0f), gp, cdf);
-}
+// Exact-erf GELU and its derivative: gelu(h) = h Phi(h), gelu'(h) = Phi(h) + h phi(h).
 // Phi(h) = 0.5*(1+erf(h/sqrt2)) via Abramowitz-Stegun 7.1.26 (|erf err| < 1.5e-7) evaluated as
 //   Phi(-|h|) = 0.5*erfc(|h|/sqrt2) = t*(a1+t*(a2+t*(a3+t*(a4+t*a5))))*exp(-h^2/2),  t = 1/(1 + p*|h|/sqrt2)
 // with the 0.5 folded into the coefficients, one MUFU.RCP + one MUFU.EX2; exp(-h^2/2) is shared with the density.
-__device__ __forceinline__ void gelu_fwd_bwd_exact(float h, float& act, float& deriv) {
+__device__ __forceinline__ void gelu_fwd_bwd(float h, float& act, float& deriv) {
   const float t = rcp_approx(fmaf(fabsf(h), 0.3275911f * 0.70710678118654752f, 1.0f));
   const float e = ex2_approx(h * h * (-0.5f * 1.4426950408889634f));
   float poly = fmaf(t, 0.5f * 1.061405429f, 0.5f * -1.453152027f);
@@ -493,26 +470,6 @@ __device__ __forceinline__ void gelu_fwd_bwd_exact(float h, float& act, float& d
   const float cdf = h > 0.f ? 1.0f - q : q;
   act = h * cdf;
   deriv = fmaf(h, e * 0.3989422804014327f, cdf);
-}
-__device__ __forceinline__ void gelu_fwd_bwd(float h, float& act, float& deriv) {
-#ifdef VITK_GELU_FAST
-  gelu_fwd_bwd_fast(h, act, deriv);
-#else
-  gelu_fwd_bwd_exact(h, act, deriv);
-#endif
-}
-
-// gelu'(h) on a fixed one-byte grid: q = round(200 g) + 27, g ~= (q - 27) / 200.  The range [-0.135, 1.14] covers
-// gelu' (min -0.1290, max 1.1290) and 0 and 1 land exactly on grid points, so saturated units keep exactly gelu' = 0 / 1.
-// Rounding without F2I: adding 2^23 puts the rounded integer (round-to-nearest-even) into the low mantissa bits.
-__device__ __forceinline__ uint32_t gelu_q8_bits(float g) { return __float_as_uint(fmaf(g, 200.0f, 8388608.0f + 27.0f)); }
-__device__ __forceinline__ uint32_t gelu_q8_pack4(float g0, float g1, float g2, float g3) {
-  const uint32_t lo = __byte_perm(gelu_q8_bits(g0), gelu_q8_bits(g1), 0x0040);   // bytes: g0.b0, g1.b0
-  const uint32_t hi = __byte_perm(gelu_q8_bits(g2), gelu_q8_bits(g3), 0x0040);
-  return __byte_perm(lo, hi, 0x5410);
-}
-__device__ __forceinline__ float gelu_q8_decode(uint32_t word, int byte) {
-  return fmaf((float)((word >> (8 * byte)) & 0xffu), 0.005f, -0.135f);
 }
 
 __device__ __forceinline__ float warp_sum(float v) {

@@ -20,8 +20,6 @@
 //   fprop  Y  = X  W^T   : A K-major,  B K-major   (W is [N,K] like nn.Linear.weight)
 //   dgrad  dX = dY W     : A K-major,  B MN-major  (W itself, no transposed copy)
 //   wgrad  dW = dY^T X   : A MN-major, B MN-major  (split-K, fp32 red.add into the grad buffer)
-#include <cstdlib>
-
 #include <cstring>
 
 #include "vitk_common.cuh"
@@ -117,12 +115,8 @@ template <int EPI>
 constexpr uint32_t kStgBytes = (EPI == EPI_BF16) ? 2048u : 4096u;
 // GELU / x GELU' epilogues with 64 columns per epilogue warp leave (and, for the aux operand, enter) through TMA:
 // two [32 rows][64 B] panels per warp in the 64-byte-swizzle layout (see the epilogue branch of gemm_kernel).
-template <int EPI>
-constexpr bool kGeluFwd = (EPI == EPI_GELU || EPI == EPI_GELU_Q8);
-template <int EPI>
-constexpr bool kGeluBwd = (EPI == EPI_DGELU || EPI == EPI_DGELU_Q8);
 template <int EPI, int PART_N>
-constexpr bool kTmaEpi = (kGeluFwd<EPI> || kGeluBwd<EPI>) && PART_N == 64;
+constexpr bool kTmaEpi = (EPI == EPI_GELU || EPI == EPI_DGELU) && PART_N == 64;
 // Residual epilogue through TMA: every epilogue warp owns a ring of three [32 rows][128 B] fp32 panels (128-byte
 // swizzle).  The residual panels of the warp's tile sequence are loaded up to two panels ahead (across tile
 // boundaries: the tile schedule is static), the sum is formed in place and leaves by a TMA store, so the epilogue
@@ -133,8 +127,8 @@ constexpr bool kTmaEpi = (kGeluFwd<EPI> || kGeluBwd<EPI>) && PART_N == 64;
 // (K = 3072: 183 -> 197 us), so the dispatcher picks this variant (internal epilogue code EPI_RESID_TMA) for K <= 1536.
 constexpr int EPI_RESID_TMA = 100;
 // bf16 epilogue through TMA (internal code): pairs of 32-column chunks leave as ONE [32 rows][128 B] box, so that every
-// row segment reaching L2 is a whole line and the epilogue issues no global stores; taken when the output rows are
-// 16-byte aligned and the warp's share of the tile is a multiple of 64 columns
+// row segment reaching L2 is a whole line and the epilogue issues no global stores; taken whenever the warp's share of
+// the tile is a multiple of 64 columns (BLOCK_N 128 and 256; the entry checks make every bf16 output TMA-compatible)
 constexpr int EPI_BF16_TMA = 101;
 constexpr int kResidTmaMaxK = 1536;
 template <int EPI, int BLOCK_N, bool CTA2>
@@ -177,106 +171,28 @@ __device__ __forceinline__ uint4 pack8(const float* v) {
   return u;
 }
 
-// One W-column chunk (W = 16 or 32) of one accumulator row.  `acc` holds the raw fp32 bits.
-template <int EPI, int W>
-__device__ __forceinline__ void epilogue_chunk(const GemmParams& p, uint32_t (&acc)[W], int row,
-                                               int col0, float rs) {
-  constexpr int G = W / 8;
+// One 32-column chunk of one accumulator row, for the two epilogues that do not go through a staging panel: the
+// ragged fp32 epilogue (scalar stores) and the split-K red.add.  `acc` holds the raw fp32 bits.
+template <int EPI>
+__device__ __forceinline__ void epilogue_chunk(const GemmParams& p, uint32_t (&acc)[32], int row, int col0) {
   if constexpr (EPI == EPI_F32) {
-    if (p.ragged) {  // e.g. a 10- or 100-class head: rows are not 16-byte aligned, store scalars
-      if (row >= p.M) return;
-      float* o = reinterpret_cast<float*>(p.out) + (long long)row * p.ld_out + col0;
+    // e.g. a 10- or 100-class head: rows are not 16-byte aligned, store scalars
+    if (row >= p.M) return;
+    float* o = reinterpret_cast<float*>(p.out) + (long long)row * p.ld_out + col0;
 #pragma unroll
-      for (int j = 0; j < W; ++j)
-        if (col0 + j < p.N) o[j] = __uint_as_float(acc[j]) + (p.bias ? __ldg(p.bias + col0 + j) : 0.f);
-      return;
-    }
-  }
-  // number of valid 8-column groups in this chunk (N % 8 == 0 is a host-side requirement otherwise)
-  const int ngroups = min(G, (p.N - col0) >> 3);
-  if (row >= p.M || ngroups <= 0) return;
-
+    for (int j = 0; j < 32; ++j)
+      if (col0 + j < p.N) o[j] = __uint_as_float(acc[j]) + (p.bias ? __ldg(p.bias + col0 + j) : 0.f);
+  } else if constexpr (EPI == EPI_ATOMIC) {
+    // number of valid 8-column groups in this chunk (N % 8 == 0 is a host-side requirement)
+    const int ngroups = min(4, (p.N - col0) >> 3);
+    if (row >= p.M || ngroups <= 0) return;
 #pragma unroll
-  for (int g = 0; g < G; ++g) {
-    if (g >= ngroups) break;
-    const int c = col0 + g * 8;
-    float v[8];
+    for (int g = 0; g < 4; ++g) {
+      if (g >= ngroups) break;
+      float v[8];
 #pragma unroll
-    for (int j = 0; j < 8; ++j) v[j] = __uint_as_float(acc[g * 8 + j]);
-
-    if constexpr (EPI != EPI_ATOMIC && EPI != EPI_DGELU) {
-      if (p.bias != nullptr) {
-        const float4 b0 = __ldg(reinterpret_cast<const float4*>(p.bias + c));
-        const float4 b1 = __ldg(reinterpret_cast<const float4*>(p.bias + c + 4));
-        v[0] += b0.x; v[1] += b0.y; v[2] += b0.z; v[3] += b0.w;
-        v[4] += b1.x; v[5] += b1.y; v[6] += b1.z; v[7] += b1.w;
-      }
-    }
-
-    if constexpr (EPI == EPI_BF16) {
-      __nv_bfloat16* o = reinterpret_cast<__nv_bfloat16*>(p.out) + (long long)row * p.ld_out + c;
-#pragma unroll
-      for (int j = 0; j < 8; ++j) v[j] *= rs;
-      *reinterpret_cast<uint4*>(o) = pack8(v);
-    } else if constexpr (EPI == EPI_GELU) {
-      // out = gelu(h), aux = gelu'(h): the backward epilogue (EPI_DGELU) is then a plain multiply
-      __nv_bfloat16* o = reinterpret_cast<__nv_bfloat16*>(p.out) + (long long)row * p.ld_out + c;
-      __nv_bfloat16* a = reinterpret_cast<__nv_bfloat16*>(p.aux) + (long long)row * p.ld_aux + c;
-      float gl[8], gd[8];
-#pragma unroll
-      for (int j = 0; j < 8; ++j) gelu_fwd_bwd(v[j], gl[j], gd[j]);
-      *reinterpret_cast<uint4*>(a) = pack8(gd);
-      *reinterpret_cast<uint4*>(o) = pack8(gl);
-    } else if constexpr (EPI == EPI_RESID || EPI == EPI_F32 || EPI == EPI_PATCH) {
-      long long orow = row;
-      const float* addp = nullptr;
-      if constexpr (EPI == EPI_RESID) addp = p.resid + (long long)row * p.ld_resid + c;
-      if constexpr (EPI == EPI_PATCH) {
-        // row = b * P + patch  ->  output token row b * (P + prefix) + prefix + patch
-        int b = row / p.tokens_per_img;
-        int t = row - b * p.tokens_per_img;
-        if (p.a_image) {   // padded rows (b, gy, gx'): gx' >= gw are zero padding, not tokens
-          const int grp = row / p.img_gwp, gx = row - grp * p.img_gwp;
-          if (gx >= p.img_gw) return;
-          b = grp / p.img_gh;
-          t = (grp - b * p.img_gh) * p.img_gw + gx;
-        }
-        orow = (long long)b * (p.tokens_per_img + p.prefix) + p.prefix + t;
-        addp = p.pos + (long long)(p.prefix + t) * p.N + c;
-      }
-      float* o = reinterpret_cast<float*>(p.out) + orow * p.ld_out + c;
-#pragma unroll
-      for (int h = 0; h < 2; ++h) {
-        const int j = h * 4;
-        float4 r = make_float4(v[j], v[j + 1], v[j + 2], v[j + 3]);
-        if constexpr (EPI == EPI_RESID) {
-          float4 cs = make_float4(rs, rs, rs, rs);
-          if (p.colscale != nullptr) {
-            const float4 cc = __ldg(reinterpret_cast<const float4*>(p.colscale + c + j));
-            cs.x *= cc.x; cs.y *= cc.y; cs.z *= cc.z; cs.w *= cc.w;
-          }
-          const float4 a = *reinterpret_cast<const float4*>(addp + j);
-          r.x = fmaf(r.x, cs.x, a.x); r.y = fmaf(r.y, cs.y, a.y);
-          r.z = fmaf(r.z, cs.z, a.z); r.w = fmaf(r.w, cs.w, a.w);
-        }
-        if constexpr (EPI == EPI_PATCH) {
-          const float4 a = __ldg(reinterpret_cast<const float4*>(addp + j));
-          r.x += a.x; r.y += a.y; r.z += a.z; r.w += a.w;
-        }
-        *reinterpret_cast<float4*>(o + j) = r;
-      }
-    } else if constexpr (EPI == EPI_DGELU) {
-      // out = acc * aux, aux = gelu'(h) written by the forward EPI_GELU epilogue
-      __nv_bfloat16* o = reinterpret_cast<__nv_bfloat16*>(p.out) + (long long)row * p.ld_out + c;
-      const __nv_bfloat16* dp = reinterpret_cast<const __nv_bfloat16*>(p.aux) + (long long)row * p.ld_aux + c;
-      const uint4 du = *reinterpret_cast<const uint4*>(dp);
-      const float2 d0 = unpack_bf16x2(du.x), d1 = unpack_bf16x2(du.y);
-      const float2 d2 = unpack_bf16x2(du.z), d3 = unpack_bf16x2(du.w);
-      v[0] *= d0.x * rs; v[1] *= d0.y * rs; v[2] *= d1.x * rs; v[3] *= d1.y * rs;
-      v[4] *= d2.x * rs; v[5] *= d2.y * rs; v[6] *= d3.x * rs; v[7] *= d3.y * rs;
-      *reinterpret_cast<uint4*>(o) = pack8(v);
-    } else if constexpr (EPI == EPI_ATOMIC) {
-      float* o = reinterpret_cast<float*>(p.out) + (long long)row * p.ld_out + c;
+      for (int j = 0; j < 8; ++j) v[j] = __uint_as_float(acc[g * 8 + j]);
+      float* o = reinterpret_cast<float*>(p.out) + (long long)row * p.ld_out + col0 + g * 8;
       red_add_v4(o, v[0], v[1], v[2], v[3]);
       red_add_v4(o + 4, v[4], v[5], v[6], v[7]);
     }
@@ -527,8 +443,7 @@ gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUt
   static_assert(!CTA2 || (BLOCK_N % 128 == 0) || (BLOCK_N == 192 && !B_MN), "CTA pairs need BLOCK_N in {128, 256} (192: K-major B only)");
   constexpr int PARTS = EW / 4;             // column partitions of the tile among epilogue warps
   constexpr int PART_N = BLOCK_N / PARTS;   // columns per epilogue warp
-  constexpr int W = (PART_N % 32 == 0) ? 32 : 16;
-  static_assert(BLOCK_N % PARTS == 0 && PART_N % W == 0, "tile does not split evenly among epilogue warps");
+  static_assert(BLOCK_N % PARTS == 0 && PART_N % 32 == 0, "tile does not split into 32-column chunks per epilogue warp");
 
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) &
@@ -820,7 +735,7 @@ gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUt
         }
       }
       float rs = 1.0f;
-      if constexpr (EPI == EPI_BF16 || EPI == EPI_BF16_TMA || EPI == EPI_RESID || EPI == EPI_RESID_TMA || kGeluBwd<EPI>) {
+      if constexpr (EPI == EPI_BF16 || EPI == EPI_BF16_TMA || EPI == EPI_RESID || EPI == EPI_RESID_TMA || EPI == EPI_DGELU) {
         if (p.rowscale != nullptr && row < p.M) rs = __ldg(p.rowscale + row / p.rows_per_group);
       }
       if constexpr (kTmaEpi<EPI, PART_N>) {
@@ -832,50 +747,7 @@ gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUt
         const int row0 = m_blk * TILE_M + (int)rank * BLOCK_M + quad * 32;
         const int colp = n_blk * BLOCK_N + part * PART_N;
         const uint32_t tacc = tmem_base + (static_cast<uint32_t>(quad * 32) << 16) + as * BLOCK_N + part * PART_N;
-        if constexpr (EPI == EPI_DGELU_Q8) {
-          // aux = gelu'(h) as one byte per element: this warp's [32 rows][64 B] box (64-byte swizzle) lands in the UPPER
-          // half of the warp's 4 KB panel while the tile's MMAs still run; every lane copies its 64-byte row into
-          // registers, and only after the whole warp has done so is the panel overwritten by the [32 rows][128 B] bf16
-          // output rows (128-byte swizzle) that leave as one TMA box
-          if (elect_one()) {
-            tma_store_wait_read();   // the previous tile's output panel has left the buffer
-            mbar_arrive_expect_tx(&aux_bar[ew], 2048);
-            tma_load_2d(buf1, &tmAux, &aux_bar[ew], colp, row0);
-          }
-          __syncwarp();
-          mbar_wait(&tmem_full[as], aphase);
-          tc_fence_after();
-          uint32_t acc0[32], acc1[32];
-          tmem_ld_32x32(tacc, acc0);
-          tmem_ld_32x32(tacc + 32, acc1);
-          mbar_wait(&aux_bar[ew], tphase);
-          uint4 dq[4];
-#pragma unroll
-          for (int u = 0; u < 4; ++u) dq[u] = *reinterpret_cast<const uint4*>(buf1 + stg_b16(lane, u));
-          tmem_ld_wait();
-          release_acc();
-          __syncwarp();   // every lane holds its derivative row: the panel may be overwritten
-#pragma unroll
-          for (int u = 0; u < 8; ++u) {
-            const uint32_t* a = (u < 4 ? acc0 : acc1) + (u & 3) * 8;
-            const uint4 dw = dq[u >> 1];
-            const uint32_t w0 = (u & 1) ? dw.z : dw.x, w1 = (u & 1) ? dw.w : dw.y;   // 8 derivative bytes of this chunk
-            uint4 o;
-            o.x = pack_bf16x2(__uint_as_float(a[0]) * (gelu_q8_decode(w0, 0) * rs), __uint_as_float(a[1]) * (gelu_q8_decode(w0, 1) * rs));
-            o.y = pack_bf16x2(__uint_as_float(a[2]) * (gelu_q8_decode(w0, 2) * rs), __uint_as_float(a[3]) * (gelu_q8_decode(w0, 3) * rs));
-            o.z = pack_bf16x2(__uint_as_float(a[4]) * (gelu_q8_decode(w1, 0) * rs), __uint_as_float(a[5]) * (gelu_q8_decode(w1, 1) * rs));
-            o.w = pack_bf16x2(__uint_as_float(a[6]) * (gelu_q8_decode(w1, 2) * rs), __uint_as_float(a[7]) * (gelu_q8_decode(w1, 3) * rs));
-            *reinterpret_cast<uint4*>(buf0 + lane * 128 + ((u ^ (lane & 7)) << 4)) = o;
-          }
-          fence_proxy_async_smem();
-          __syncwarp();
-          if (elect_one()) {
-            tma_store_2d(&tmOut, buf0, colp, row0);
-            tma_store_commit();
-          }
-          __syncwarp();
-          tphase ^= 1;
-        } else if constexpr (EPI == EPI_DGELU) {
+        if constexpr (EPI == EPI_DGELU) {
           // aux = gelu'(h) of this warp's [32 rows][64 columns] is fetched while the tile's MMAs still run: ONE box of
           // 128-byte rows (128-byte swizzle: chunk u of row r at u ^ (r & 7)), multiplied in place and stored as one box,
           // so every row segment that reaches L2 is a whole line (with two 64-byte boxes per row the L2 write hit
@@ -932,8 +804,7 @@ gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUt
                                                                : make_float4(0.f, 0.f, 0.f, 0.f);
             tmem_ld_wait();
             if (hf == 1) release_acc();
-            constexpr bool Q8 = (EPI == EPI_GELU_Q8);
-            uint32_t act[16], der[Q8 ? 8 : 16];
+            uint32_t act[16], der[16];
 #pragma unroll
             for (int j = 0; j < 8; ++j) {
               float a0, a1, a2, a3, g0, g1, g2, g3;
@@ -943,12 +814,8 @@ gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUt
               gelu_fwd_bwd(__uint_as_float(acc[j * 4 + 3]) + bb[j].w, a3, g3);
               act[j * 2] = pack_bf16x2(a0, a1);
               act[j * 2 + 1] = pack_bf16x2(a2, a3);
-              if constexpr (Q8) {
-                der[j] = gelu_q8_pack4(g0, g1, g2, g3);
-              } else {
-                der[j * 2] = pack_bf16x2(g0, g1);
-                der[j * 2 + 1] = pack_bf16x2(g2, g3);
-              }
+              der[j * 2] = pack_bf16x2(g0, g1);
+              der[j * 2 + 1] = pack_bf16x2(g2, g3);
             }
             // the panels of the previous half (or tile) must have been read by the TMA unit before they are overwritten
             if (elect_one()) tma_store_wait_read();
@@ -956,16 +823,9 @@ gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUt
 #pragma unroll
             for (int u = 0; u < 4; ++u)
               *reinterpret_cast<uint4*>(buf0 + stg_b16(lane, u)) = make_uint4(act[u * 4], act[u * 4 + 1], act[u * 4 + 2], act[u * 4 + 3]);
-            if constexpr (Q8) {   // [32 rows][32 B], 32-byte swizzle: 16-byte chunk u of row r at u ^ ((r >> 2) & 1)
 #pragma unroll
-              for (int u = 0; u < 2; ++u)
-                *reinterpret_cast<uint4*>(buf1 + lane * 32 + ((u ^ ((lane >> 2) & 1)) << 4)) =
-                    make_uint4(der[u * 4], der[u * 4 + 1], der[u * 4 + 2], der[u * 4 + 3]);
-            } else {
-#pragma unroll
-              for (int u = 0; u < 4; ++u)
-                *reinterpret_cast<uint4*>(buf1 + stg_b16(lane, u)) = make_uint4(der[u * 4], der[u * 4 + 1], der[u * 4 + 2], der[u * 4 + 3]);
-            }
+            for (int u = 0; u < 4; ++u)
+              *reinterpret_cast<uint4*>(buf1 + stg_b16(lane, u)) = make_uint4(der[u * 4], der[u * 4 + 1], der[u * 4 + 2], der[u * 4 + 3]);
             fence_proxy_async_smem();
             __syncwarp();
             if (elect_one()) {
@@ -1020,7 +880,6 @@ gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUt
           __syncwarp();
         }
       } else if constexpr (TMA_RESID) {
-        static_assert(W == 32, "residual panels are 32 columns wide");
         const int row0 = m_blk * TILE_M + (int)rank * BLOCK_M + quad * 32;
         mbar_wait(&tmem_full[as], aphase);
         tc_fence_after();
@@ -1067,7 +926,7 @@ gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUt
           ++rq;
           if (++rbuf == kResidBufs) { rbuf = 0; rphase ^= 1; }
         }
-      } else if constexpr (kStaged<EPI> && W == 32) {
+      } else if constexpr (kStaged<EPI>) {
         uint8_t* stg = stg_base + ew * STG_BYTES;
         const int row0 = m_blk * TILE_M + (int)rank * BLOCK_M + quad * 32;
         const bool ragged = (EPI == EPI_F32) && p.ragged;
@@ -1096,7 +955,7 @@ gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUt
           tmem_ld_wait();
           if (c + 1 == PART_N / 32) release_acc();
           if (ragged) {
-            epilogue_chunk<EPI, 32>(p, acc, row, col0, rs);
+            epilogue_chunk<EPI>(p, acc, row, col0);
           } else {
             if constexpr (EPI == EPI_RESID || EPI == EPI_DGELU) {
               if constexpr (EPI == EPI_DGELU) {
@@ -1112,16 +971,15 @@ gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUt
         mbar_wait(&tmem_full[as], aphase);
         tc_fence_after();
 #pragma unroll 1
-        for (int c = 0; c < PART_N / W; ++c) {
-          const int col_in_tile = part * PART_N + c * W;
+        for (int c = 0; c < PART_N / 32; ++c) {
+          const int col_in_tile = part * PART_N + c * 32;
           const uint32_t taddr =
               tmem_base + (static_cast<uint32_t>(quad * 32) << 16) + as * BLOCK_N + col_in_tile;
-          uint32_t acc[W];
-          if constexpr (W == 32) tmem_ld_32x32(taddr, acc);
-          else tmem_ld_32x16(taddr, acc);
+          uint32_t acc[32];
+          tmem_ld_32x32(taddr, acc);
           tmem_ld_wait();
-          if (c + 1 == PART_N / W) release_acc();
-          epilogue_chunk<EPI, W>(p, acc, row, n_blk * BLOCK_N + col_in_tile, rs);
+          if (c + 1 == PART_N / 32) release_acc();
+          epilogue_chunk<EPI>(p, acc, row, n_blk * BLOCK_N + col_in_tile);
         }
       }
       if (!released) release_acc();
@@ -1149,14 +1007,6 @@ inline long long image_batch(const vitk_gemm_args* a) {
   return per_img > 0 ? (rows + per_img - 1) / per_img : 0;
 }
 
-bool use_cta_pairs() {
-  static const bool on = [] {
-    const char* e = getenv("VITK_GEMM_2CTA");  // tuning knob: "0" forces the single-CTA kernel
-    return !(e && e[0] == '0');
-  }();
-  return on;
-}
-
 int pick_splits(int tiles, int num_k_blocks, int slots, int block_n) {
   // Split-K factor of a weight gradient.  Cost model fitted to measurements (profiles/r02_wgrad_splits.txt): a CTA pair
   // runs its units one after the other; a unit costs its k-blocks plus the red.add epilogue of its fp32 tile, which is
@@ -1175,30 +1025,15 @@ int pick_splits(int tiles, int num_k_blocks, int slots, int block_n) {
   return best;
 }
 
-// TMA needs 16-byte aligned bases and row pitches; anything else takes the register-prefetch residual epilogue
-inline bool resid_tma_ok(const vitk_gemm_args* a) {
-  static const bool enabled = [] { const char* e = getenv("VITK_GEMM_RESID_TMA"); return !(e != nullptr && e[0] == '0'); }();
-  return enabled && a->resid != nullptr && (((uintptr_t)a->out | (uintptr_t)a->resid) & 15) == 0 && a->ld_out % 4 == 0 &&
-         a->ld_resid % 4 == 0 && a->N % 4 == 0;
-}
+// TMA needs 16-byte aligned bases and row pitches.  The entry checks already require them of out, ld_out, ld_resid
+// and N; a residual that is not 16-byte aligned takes the register-prefetch residual epilogue.
+inline bool resid_tma_ok(const vitk_gemm_args* a) { return ((uintptr_t)a->resid & 15) == 0; }
 
-inline bool bf16_tma_ok(const vitk_gemm_args* a) {
-  static const bool enabled = [] { const char* e = getenv("VITK_GEMM_BF16_TMA"); return !(e != nullptr && e[0] == '0'); }();
-  return enabled && ((uintptr_t)a->out & 15) == 0 && a->ld_out % 8 == 0 && a->N % 8 == 0;
-}
-
-// Short-K launches (K <= VITK_GEMM_EW16_MAXK, e.g. ViT-S: K = 384 is six k-blocks per tile) are bound by the epilogue,
-// not the main loop: the bf16 TMA epilogue then runs with 16 warps (one 64-column box per warp) instead of 8.
-int ew16_max_k() {
-  static const int v = [] { const char* e = getenv("VITK_GEMM_EW16_MAXK"); return e ? atoi(e) : 0; }();
-  return v;
-}
-
-template <int BLOCK_N, bool A_MN, bool B_MN, int EPI, bool CTA2, bool WIDE_EPI = false>
+template <int BLOCK_N, bool A_MN, bool B_MN, int EPI, bool CTA2>
 int launch_gemm(const vitk_gemm_args* a, cudaStream_t stream) {
   // 16 epilogue warps for the GELU epilogues (~20 instructions per element); 8 elsewhere.  With BLOCK_N = 192 and
   // 16 warps a warp's share is 48 columns, which is not a whole number of 32-column panels -> keep 8 there.
-  constexpr int EW = (((kGeluFwd<EPI> || kGeluBwd<EPI>) && BLOCK_N != 192) || WIDE_EPI) ? 16 : 8;
+  constexpr int EW = ((EPI == EPI_GELU || EPI == EPI_DGELU) && BLOCK_N != 192) ? 16 : 8;
   using Cfg = TileCfg<BLOCK_N, EW, kStgBytesFor<EPI, BLOCK_N, CTA2>, CTA2>;
   constexpr int TILE_M = CTA2 ? 2 * BLOCK_M : BLOCK_M;
   CUtensorMap tmA, tmB;
@@ -1232,18 +1067,8 @@ int launch_gemm(const vitk_gemm_args* a, cudaStream_t stream) {
     rc = vitk_make_tmap_2d(&tmAux, a->resid, 4, a->N, a->M, a->ld_resid, 32, 32);
     if (rc) return rc;
   }
-  if ((EPI == EPI_GELU_Q8 || EPI == EPI_DGELU_Q8) && !kTmaEpi<EPI, BLOCK_N / (EW / 4)>)
-    return vitk_set_error(VITK_ERR_UNSUPPORTED, "gemm: the one-byte GELU' epilogues need N %% 256 == 0 (N=%d)", a->N);
   if (kTmaEpi<EPI, BLOCK_N / (EW / 4)>) {
-    if (EPI == EPI_DGELU_Q8) {  // out: [32 rows][128 B] bf16, 128-byte swizzle; aux: [32 rows][64 B] uint8, 64-byte swizzle
-      rc = vitk_make_tmap_2d(&tmOut, a->out, 2, a->N, a->M, a->ld_out, 64, 32);
-      if (rc) return rc;
-      rc = vitk_make_tmap_2d_u8(&tmAux, a->aux, a->N, a->M, a->ld_aux, 64, 32);
-    } else if (EPI == EPI_GELU_Q8) {  // out: [32 rows][64 B] bf16 (64-byte swizzle); aux: [32 rows][32 B] uint8 (32-byte swizzle)
-      rc = vitk_make_tmap_2d_sw64(&tmOut, a->out, 2, a->N, a->M, a->ld_out, 32, 32);
-      if (rc) return rc;
-      rc = vitk_make_tmap_2d_u8(&tmAux, a->aux, a->N, a->M, a->ld_aux, 32, 32);
-    } else if (EPI == EPI_DGELU) {   // [32 rows][128 B] boxes, 128-byte swizzle
+    if (EPI == EPI_DGELU) {   // [32 rows][128 B] boxes, 128-byte swizzle
       rc = vitk_make_tmap_2d(&tmOut, a->out, 2, a->N, a->M, a->ld_out, 64, 32);
       if (rc) return rc;
       rc = vitk_make_tmap_2d(&tmAux, a->aux, 2, a->N, a->M, a->ld_aux, 64, 32);
@@ -1324,17 +1149,9 @@ int dispatch2(const vitk_gemm_args* a, cudaStream_t stream) {
   if (!amn && !bmn) {
     switch (a->epilogue) {
       case EPI_BF16:
-        if constexpr (BLOCK_N == 256) {
-          if (bf16_tma_ok(a) && a->K <= ew16_max_k()) return launch_gemm<BLOCK_N, false, false, EPI_BF16_TMA, CTA2, true>(a, stream);
-        }
-        if constexpr (BLOCK_N % 128 == 0) {
-          if (bf16_tma_ok(a)) return launch_gemm<BLOCK_N, false, false, EPI_BF16_TMA, CTA2>(a, stream);
-        }
-        return launch_gemm<BLOCK_N, false, false, EPI_BF16, CTA2>(a, stream);
+        if constexpr (BLOCK_N % 128 == 0) return launch_gemm<BLOCK_N, false, false, EPI_BF16_TMA, CTA2>(a, stream);
+        else return launch_gemm<BLOCK_N, false, false, EPI_BF16, CTA2>(a, stream);
       case EPI_GELU:  return launch_gemm<BLOCK_N, false, false, EPI_GELU, CTA2>(a, stream);
-      case EPI_GELU_Q8:
-        if constexpr (BLOCK_N == 256) return launch_gemm<BLOCK_N, false, false, EPI_GELU_Q8, CTA2>(a, stream);
-        break;
       case EPI_RESID:
         if constexpr (CTA2 || BLOCK_N < 256) {
           if (a->K <= kResidTmaMaxK && resid_tma_ok(a) && a->mask == nullptr)   // the dropout mask lives in the staged-panel epilogue
@@ -1348,17 +1165,9 @@ int dispatch2(const vitk_gemm_args* a, cudaStream_t stream) {
     if constexpr (!PAIR192) {
     switch (a->epilogue) {
       case EPI_BF16:
-        if constexpr (BLOCK_N == 256) {
-          if (bf16_tma_ok(a) && a->K <= ew16_max_k()) return launch_gemm<BLOCK_N, false, true, EPI_BF16_TMA, CTA2, true>(a, stream);
-        }
-        if constexpr (BLOCK_N % 128 == 0) {
-          if (bf16_tma_ok(a)) return launch_gemm<BLOCK_N, false, true, EPI_BF16_TMA, CTA2>(a, stream);
-        }
-        return launch_gemm<BLOCK_N, false, true, EPI_BF16, CTA2>(a, stream);
+        if constexpr (BLOCK_N % 128 == 0) return launch_gemm<BLOCK_N, false, true, EPI_BF16_TMA, CTA2>(a, stream);
+        else return launch_gemm<BLOCK_N, false, true, EPI_BF16, CTA2>(a, stream);
       case EPI_DGELU: return launch_gemm<BLOCK_N, false, true, EPI_DGELU, CTA2>(a, stream);
-      case EPI_DGELU_Q8:
-        if constexpr (BLOCK_N == 256) return launch_gemm<BLOCK_N, false, true, EPI_DGELU_Q8, CTA2>(a, stream);
-        break;
       case EPI_F32:   return launch_gemm<BLOCK_N, false, true, EPI_F32, CTA2>(a, stream);
     }
     }
@@ -1367,19 +1176,14 @@ int dispatch2(const vitk_gemm_args* a, cudaStream_t stream) {
                         (int)amn, (int)bmn, a->epilogue);
 }
 
-bool pair192_enabled() {
-  static const bool on = [] { const char* e = getenv("VITK_GEMM_192_2CTA"); return !(e && e[0] == '0'); }();
-  return on;
-}
-
 template <int BLOCK_N>
 int dispatch(const vitk_gemm_args* a, cudaStream_t stream) {
   // CTA pairs pay off once there are enough 256-row tiles to go round; tiny problems keep 128-row tiles
   if constexpr (BLOCK_N != 192) {
-    if (use_cta_pairs() && a->M >= 256) return dispatch2<BLOCK_N, true>(a, stream);
+    if (a->M >= 256) return dispatch2<BLOCK_N, true>(a, stream);
   } else {
     // 256 x 192 pair tiles exist for the forward layouts (both operands K-major, not split-K)
-    if (use_cta_pairs() && pair192_enabled() && a->M >= 256 && !a->a_mn_major && !a->b_mn_major && a->epilogue != EPI_ATOMIC)
+    if (a->M >= 256 && !a->a_mn_major && !a->b_mn_major && a->epilogue != EPI_ATOMIC)
       return dispatch2<BLOCK_N, true>(a, stream);
   }
   return dispatch2<BLOCK_N, false>(a, stream);
@@ -1400,9 +1204,6 @@ extern "C" int vitk_gemm_bf16(const vitk_gemm_args* a, void* stream_) {
   VITK_REQUIRE(a->ld_out % 8 == 0 || a->epilogue == EPI_F32, VITK_ERR_ALIGN, "gemm: ld_out must be a multiple of 8");
   if (a->epilogue == EPI_GELU || a->epilogue == EPI_DGELU)
     VITK_REQUIRE(a->aux != nullptr && a->ld_aux % 8 == 0, VITK_ERR_ALIGN, "gemm: aux pointer/ld required for GELU epilogues");
-  if (a->epilogue == EPI_GELU_Q8 || a->epilogue == EPI_DGELU_Q8)
-    VITK_REQUIRE(a->aux != nullptr && a->ld_aux % 16 == 0 && (reinterpret_cast<uintptr_t>(a->aux) & 15) == 0 && a->N % 256 == 0,
-                 VITK_ERR_ALIGN, "gemm: one-byte GELU' epilogues need a 16-byte aligned aux, ld_aux %% 16 == 0 and N %% 256 == 0");
   if (a->epilogue == EPI_RESID)
     VITK_REQUIRE(a->resid != nullptr && a->ld_resid % 4 == 0, VITK_ERR_ALIGN, "gemm: resid pointer/ld required");
   if (a->epilogue == EPI_PATCH)

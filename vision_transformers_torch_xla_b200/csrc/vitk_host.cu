@@ -62,8 +62,7 @@ static int encode(CUtensorMap* out, const void* base, int elem_bytes, int rank, 
   EncodeTiledFn fn = get_encode();
   if (!fn) return vitk_set_error(VITK_ERR_DRIVER, "cuTensorMapEncodeTiled not available from the driver");
   cuuint32_t estr[5] = {1, 1, 1, 1, 1};
-  CUtensorMapDataType dt = elem_bytes == 2 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16
-                         : elem_bytes == 1 ? CU_TENSOR_MAP_DATA_TYPE_UINT8 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32;
+  CUtensorMapDataType dt = elem_bytes == 2 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32;
   CUresult r = fn(out, dt, (cuuint32_t)rank, const_cast<void*>(base), dims, strides_bytes, box, estr,
                   CU_TENSOR_MAP_INTERLEAVE_NONE, swz,
                   CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
@@ -91,15 +90,6 @@ int vitk_make_tmap_2d_sw64(CUtensorMap* out, const void* base, int elem_bytes, u
   cuuint64_t strides[1] = {ld_elems * (uint64_t)elem_bytes};
   cuuint32_t box[2] = {box_inner, box_outer};
   return encode(out, base, elem_bytes, 2, dims, strides, box, CU_TENSOR_MAP_SWIZZLE_64B);
-}
-
-// uint8 [outer][inner] with 32- or 64-byte box rows in the matching swizzle (the one-byte GELU' panels of the GEMM epilogue)
-int vitk_make_tmap_2d_u8(CUtensorMap* out, const void* base, uint64_t inner, uint64_t outer, uint64_t ld_bytes,
-                         uint32_t box_inner, uint32_t box_outer) {
-  cuuint64_t dims[2] = {inner, outer};
-  cuuint64_t strides[1] = {ld_bytes};
-  cuuint32_t box[2] = {box_inner, box_outer};
-  return encode(out, base, 1, 2, dims, strides, box, box_inner == 32 ? CU_TENSOR_MAP_SWIZZLE_32B : CU_TENSOR_MAP_SWIZZLE_64B);
 }
 
 int vitk_make_tmap_3d(CUtensorMap* out, const void* base, int elem_bytes, uint64_t d0, uint64_t d1, uint64_t d2,

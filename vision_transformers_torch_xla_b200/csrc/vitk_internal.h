@@ -9,5 +9,3 @@ constexpr int EPI_F32 = VITK_EPI_F32;
 constexpr int EPI_DGELU = VITK_EPI_DGELU;
 constexpr int EPI_ATOMIC = VITK_EPI_ATOMIC;
 constexpr int EPI_PATCH = VITK_EPI_PATCH;
-constexpr int EPI_GELU_Q8 = VITK_EPI_GELU_Q8;
-constexpr int EPI_DGELU_Q8 = VITK_EPI_DGELU_Q8;

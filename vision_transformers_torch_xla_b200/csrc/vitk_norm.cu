@@ -12,9 +12,6 @@
 #include "vitk_common.cuh"
 #include "vitk_internal.h"
 
-#include <cstdio>
-#include <cstdlib>
-
 namespace {
 using namespace vitk;
 
@@ -216,7 +213,8 @@ __device__ __forceinline__ void bulk_load_1d(void* smem_dst, const void* gsrc, u
                : "memory");
 }
 
-constexpr int RING_MAX_STAGES = 4;
+constexpr int RING_MAX_STAGES = 4;   // the barrier slots reserved per warp; the host launches RING_STAGES of them
+constexpr int RING_STAGES = 2;
 constexpr int RING_MAX_WARPS = 16;
 
 __host__ __device__ inline uint32_t ring_header_bytes(int dim, int warps) {
@@ -366,25 +364,11 @@ ln_bwd_ring_kernel(const __nv_bfloat16* __restrict__ dy, long long ld_dy, const 
 }
 
 // Largest warp count whose rings fit the 227 KB of one SM (0: does not fit, use the register-resident kernel).
-inline int ring_env(int which) {
-  static int v[2] = {-1, -1};
-  if (v[0] < 0) {
-    v[0] = 0;
-    v[1] = 2;
-    const char* e = getenv("VITK_LN_RING");  // "warps,stages" (tuning knob)
-    if (e != nullptr) sscanf(e, "%d,%d", &v[0], &v[1]);
-    if (v[1] < 1 || v[1] > RING_MAX_STAGES) v[1] = 2;
-  }
-  return v[which];
-}
-
 inline int ring_warps(int dim) {
   const long long budget = 227 * 1024 - 1024;
-  const int stages = ring_env(1);
-  int wmax = (dim <= 512 ? RING_MAX_WARPS : dim <= 768 ? 12 : 8);  // the launch bounds of VPL = 6 / 8
-  if (ring_env(0) > 0 && ring_env(0) < wmax) wmax = ring_env(0);
+  const int wmax = (dim <= 512 ? RING_MAX_WARPS : dim <= 768 ? 12 : 8);  // the launch bounds of VPL = 6 / 8
   for (int w = wmax; w >= 1; --w)
-    if ((long long)ring_header_bytes(dim, w) + (long long)w * stages * 10 * dim <= budget) return w;
+    if ((long long)ring_header_bytes(dim, w) + (long long)w * RING_STAGES * 10 * dim <= budget) return w;
   return 0;
 }
 
@@ -393,8 +377,7 @@ int launch_ln_bwd_ring(const void* dy_bf16, int64_t ld_dy, const float* x, int64
                        const float* rstd, const float* gamma, const float* g_in, float* g_out, int64_t ld_g,
                        void* gb_out_bf16, const float* rowscale, int32_t rows_per_group, float* dgamma, float* dbeta,
                        int64_t rows, int32_t dim, int warps, void* stream) {
-  const int stages = ring_env(1);
-  const size_t smem = ring_header_bytes(dim, warps) + (size_t)warps * stages * 10 * dim;
+  const size_t smem = ring_header_bytes(dim, warps) + (size_t)warps * RING_STAGES * 10 * dim;
   static bool configured = false;  // per instantiation
   if (!configured) {
     if (cudaFuncSetAttribute(ln_bwd_ring_kernel<VPL, EXACT>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024) != cudaSuccess)
@@ -406,7 +389,7 @@ int launch_ln_bwd_ring(const void* dy_bf16, int64_t ld_dy, const float* x, int64
   const unsigned grid = (unsigned)(want < cap ? want : cap);
   ln_bwd_ring_kernel<VPL, EXACT><<<grid, warps * 32, smem, (cudaStream_t)stream>>>(
       (const __nv_bfloat16*)dy_bf16, ld_dy, x, ld_x, mean, rstd, gamma, g_in, g_out, ld_g,
-      (__nv_bfloat16*)gb_out_bf16, rowscale, rows_per_group > 0 ? rows_per_group : 1, dgamma, dbeta, rows, dim, stages);
+      (__nv_bfloat16*)gb_out_bf16, rowscale, rows_per_group > 0 ? rows_per_group : 1, dgamma, dbeta, rows, dim, RING_STAGES);
   return vitk_check_launch("layernorm_bwd");
 }
 
@@ -455,28 +438,27 @@ extern "C" int vitk_layernorm_bwd(const void* dy_bf16, int64_t ld_dy, const floa
   if (rows == 0) return VITK_OK;
   const int vpl = (dim + 127) / 128;
   // bulk-copy path: 16-byte aligned rows of every stream
-  static const int ring_mode = [] { const char* e = getenv("VITK_LN_BWD"); return (e != nullptr && e[0] == 'r' && e[1] == 'e') ? 0 : 1; }();
   const int rw = ring_warps(dim);
-  const bool ring_ok = ring_mode && rw > 0 && rows >= 4096 && dim % 8 == 0 && ld_dy % 8 == 0 && ((uintptr_t)dy_bf16 & 15) == 0 &&
+  const bool ring_ok = rw > 0 && rows >= 4096 && dim % 8 == 0 && ld_dy % 8 == 0 && ((uintptr_t)dy_bf16 & 15) == 0 &&
                        ((uintptr_t)x & 15) == 0 && (g_in == nullptr || ((uintptr_t)g_in & 15) == 0);
   if (ring_ok) {
-#define VITK_LN_RING(V)                                                                                              \
+#define LN_RING_CASE(V)                                                                                              \
   return (dim == (V) * 128 ? launch_ln_bwd_ring<V, true> : launch_ln_bwd_ring<V, false>)(dy_bf16, ld_dy, x, ld_x, mean, rstd, gamma, g_in, g_out, ld_g, gb_out_bf16, rowscale, \
                                rows_per_group, dgamma, dbeta, rows, dim, rw, stream)
-    if (vpl <= 2) VITK_LN_RING(2);
-    if (vpl <= 3) VITK_LN_RING(3);
-    if (vpl <= 4) VITK_LN_RING(4);
-    if (vpl <= 6) VITK_LN_RING(6);
-    VITK_LN_RING(8);
-#undef VITK_LN_RING
+    if (vpl <= 2) LN_RING_CASE(2);
+    if (vpl <= 3) LN_RING_CASE(3);
+    if (vpl <= 4) LN_RING_CASE(4);
+    if (vpl <= 6) LN_RING_CASE(6);
+    LN_RING_CASE(8);
+#undef LN_RING_CASE
   }
-#define VITK_LN_BWD(V)                                                                                          \
+#define LN_BWD_CASE(V)                                                                                          \
   return launch_ln_bwd<V, false>(dy_bf16, ld_dy, x, ld_x, mean, rstd, gamma, g_in, g_out, ld_g, gb_out_bf16, rowscale, \
                           rows_per_group, dgamma, dbeta, rows, dim, stream)
-  if (vpl <= 2) VITK_LN_BWD(2);
-  if (vpl <= 3) VITK_LN_BWD(3);
-  if (vpl <= 4) VITK_LN_BWD(4);
-  if (vpl <= 6) VITK_LN_BWD(6);
-  VITK_LN_BWD(8);
-#undef VITK_LN_BWD
+  if (vpl <= 2) LN_BWD_CASE(2);
+  if (vpl <= 3) LN_BWD_CASE(3);
+  if (vpl <= 4) LN_BWD_CASE(4);
+  if (vpl <= 6) LN_BWD_CASE(6);
+  LN_BWD_CASE(8);
+#undef LN_BWD_CASE
 }

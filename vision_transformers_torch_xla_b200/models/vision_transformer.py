@@ -421,8 +421,6 @@ class VisionTransformer(nn.Module):
         self.patch_embed._check(x)
         if x.dtype not in (torch.float32, torch.bfloat16) or not x.is_cuda:
             raise ops.L.VitkError(f"VisionTransformer expects a float32 (or bfloat16) CUDA image batch, got {x.dtype} on {x.device}")
-        if x.dtype == torch.bfloat16 and ops.PATCH_EMBED != "tma":
-            x = x.float()
         x = x if x.is_contiguous() else x.contiguous()
         x = ops.EmbedFn.apply(x, st.anchor, self, st, torch.is_grad_enabled())
         if self.training and self.pos_drop.p > 0.0:   # _pos_embed ends in pos_drop (vision_transformer.py:780, deit.py:106)

@@ -14,7 +14,6 @@ next stage's backward so that no separate cast pass is needed.
 """
 from __future__ import annotations
 
-import os
 from typing import Optional
 
 import torch
@@ -25,25 +24,6 @@ from .store import ParamStore
 
 def _empty(shape, dtype, dev):
     return torch.empty(shape, dtype=dtype, device=dev)
-
-
-#: storage of gelu'(fc1 out) between forward and backward: "bf16" = two bytes per element (default); "q8" = one byte on a
-#: fixed grid of step 0.005 that holds 0 and 1 exactly (include/vitk.h: VITK_EPI_GELU_Q8; |error| <= 0.0025, what a bf16
-#: rounding costs at gelu' ~ 1; needs a hidden width that is a multiple of 256).  q8 saves 1.9 GB of activations per ViT-B
-#: step and 25 % of fc1's output bytes, but measured on B200 (same box, alternating runs, profiles/r02_ab_gelu_q8.txt) it
-#: buys no time where it was meant to: ViT-B fc1 fprop 234.8 -> 235.4 us, fc2 dgrad 218.7 -> 222.4 us (7 975 / 8 021 vs
-#: 8 001 / 7 974 img/s); ViT-S fc2 dgrad 67.7 -> 80.8 us (the decode costs issue slots the short-K epilogue does not have);
-#: only ViT-L/384's fc1 fprop gains (267 -> 241 us, 666 -> 670 img/s).  The GELU epilogues are not byte-bound.
-GELU_AUX = os.environ.get("VITK_GELU_AUX", "bf16")
-if GELU_AUX not in ("q8", "bf16"):
-    raise ValueError(f"VITK_GELU_AUX={GELU_AUX!r}: expected 'q8' or 'bf16'")
-
-
-def _gelu_codes(F: int):
-    """(forward epilogue, backward epilogue, dtype of the saved derivative) for a hidden width F."""
-    if GELU_AUX == "q8" and F % 256 == 0:
-        return L.EPI_GELU_Q8, L.EPI_DGELU_Q8, torch.uint8
-    return L.EPI_GELU, L.EPI_DGELU, torch.bfloat16
 
 
 def _require_f32_cuda(x: torch.Tensor, what: str) -> torch.Tensor:
@@ -67,14 +47,6 @@ def _bf16_grad(store: ParamStore, g: torch.Tensor, rowscale: Optional[torch.Tens
 # ================================================================================================
 # Patch embedding + prefix tokens + positional embedding
 # ================================================================================================
-#: "tma" (default): im2col-free — the image (cast to bf16 NCHW in one coalesced pass, or handed in as bf16 already) is the
-#: GEMM's A operand through a 4-D tensor map that reads it as its patch matrix; the [B*P, C*ps*ps] matrix is never
-#: materialised, neither for the forward nor for the weight gradient.  "patchify": the explicit im2col + cast kernel.
-PATCH_EMBED = os.environ.get("VITK_PATCH_EMBED", "tma")
-if PATCH_EMBED not in ("tma", "patchify"):
-    raise ValueError(f"VITK_PATCH_EMBED={PATCH_EMBED!r}: expected 'tma' or 'patchify'")
-
-
 def _patch_grid_pad(gw: int) -> int:
     """Patch-grid width rounded up to a multiple of 8: the TMA boxes of the image operand cover 8 neighbouring patches."""
     return (gw + 7) // 8 * 8
@@ -98,8 +70,11 @@ class EmbedFn(torch.autograd.Function):
         w = store.shadow_of(pe.proj.weight).view(D, K)
         pos = model.pos_embed.data.view(N, D)
         bias = None if pe.proj.bias is None else pe.proj.bias.data
-        tma = PATCH_EMBED == "tma" and ps == 16 and pe.patch_size[1] == 16
-        if tma:
+        # 16 x 16 patches: im2col-free.  The image (cast to bf16 NCHW in one coalesced pass, or handed in as bf16 already)
+        # is the GEMM's A operand through a 4-D tensor map that reads it as its patch matrix; the [B*P, C*ps*ps] matrix is
+        # never materialised, neither for the forward nor for the weight gradient.  Other patch sizes: the explicit
+        # im2col + cast kernel, which reads an fp32 image.
+        if ps == 16 and pe.patch_size[1] == 16:
             if img.dtype == torch.bfloat16:
                 src = img                         # a loader that already produces bf16 saves the cast (and half the H2D bytes)
             else:
@@ -110,7 +85,7 @@ class EmbedFn(torch.autograd.Function):
                    image=("a",) + geom)
         else:
             src = _empty((B * P, K), torch.bfloat16, dev)
-            L.patchify(img, src, ps)
+            L.patchify(img.float() if img.dtype == torch.bfloat16 else img, src, ps)
             geom = None
             L.gemm(src, w, x, M=B * P, N=D, K=K, epilogue=L.EPI_PATCH, bias=bias, pos=pos, tokens_per_img=P, prefix=prefix)
         xf = x.view(-1)
@@ -240,10 +215,9 @@ class BlockFn(torch.autograd.Function):
         ln2 = _empty((M, D), torch.bfloat16, dev)
         mean2, rstd2 = _empty((M,), torch.float32, dev), _empty((M,), torch.float32, dev)
         L.layernorm_fwd(x_mid, blk.norm2.weight.data, blk.norm2.bias.data, ln2, mean2, rstd2, M, D, eps)
-        epi_gelu, _, aux_dtype = _gelu_codes(F) if md2 is None else (L.EPI_GELU, L.EPI_DGELU, torch.bfloat16)
-        h = _empty((M, F), aux_dtype, dev)  # receives gelu'(fc1 out) (x the drop1 mask): all the backward needs of it
+        h = _empty((M, F), torch.bfloat16, dev)  # receives gelu'(fc1 out) (x the drop1 mask): all the backward needs of it
         act = _empty((M, F), torch.bfloat16, dev)
-        L.gemm(ln2, sh(blk.mlp.fc1.weight), act, M=M, N=F, K=D, epilogue=epi_gelu, bias=bias(blk.mlp.fc1), aux=h,
+        L.gemm(ln2, sh(blk.mlp.fc1.weight), act, M=M, N=F, K=D, epilogue=L.EPI_GELU, bias=bias(blk.mlp.fc1), aux=h,
                mask=md2, mask_scale=dscale)
         x_out = _empty((B, N, D), torch.float32, dev)
         L.gemm(act, sh(blk.mlp.fc2.weight), x_out, M=M, N=D, K=F, epilogue=L.EPI_RESID, bias=bias(blk.mlp.fc2),
@@ -264,8 +238,8 @@ class BlockFn(torch.autograd.Function):
             ctx.blk, ctx.store, ctx.tag = blk, store, tag
             ctx.dims = (B, N, D, blk.attn.num_heads, blk.attn.head_dim, blk.mlp.fc1.out_features)
             ctx.rs = (rs1, rs2, prev_rs)
-            md1, md2, md3, dscale, ma, ascale = drop if drop is not None else (None, None, None, 1.0, None, 1.0)
-            ctx.drop = (md1, md3, dscale, md2 is not None, ma, ascale)
+            md1, _, md3, dscale, ma, ascale = drop if drop is not None else (None, None, None, 1.0, None, 1.0)
+            ctx.drop = (md1, md3, dscale, ma, ascale)
             ctx.recompute = (x, drop) if checkpoint else None
             ctx.saved = None if checkpoint else saved
         return x_out
@@ -303,7 +277,7 @@ class BlockFn(torch.autograd.Function):
                 L.layerscale_grad(lin.weight.data, gr(lin.weight), None if lin.bias is None else lin.bias.data,
                                   None if lin.bias is None else gr(lin.bias), ls.gamma.data, gr(ls.gamma))
 
-        md1, md3, dscale, gelu_masked, ma, ascale = ctx.drop
+        md1, md3, dscale, ma, ascale = ctx.drop
         gb2 = _bf16_grad(store, g, rs2, N * D).view(M, D)
         ls_bwd_scale(gb2, blk.ls2)   # gb2 is exclusively ours (popped from the side channel or freshly made)
         if md3 is not None:          # Mlp.drop2 sits between fc2 and LayerScale / DropPath: its mask goes on the branch gradient
@@ -312,8 +286,7 @@ class BlockFn(torch.autograd.Function):
         ls_bwd_grad(blk.ls2, blk.mlp.fc2)
         dh = act  # reuse: gelu output is dead after the fc2 wgrad above
         # (Mlp.drop1: the saved derivative already carries mask / keep_prob, so this multiply is the same launch)
-        L.gemm(gb2, sh(blk.mlp.fc2.weight), dh, M=M, N=F, K=D, epilogue=L.EPI_DGELU if gelu_masked else _gelu_codes(F)[1],
-               b_mn=True, aux=h)
+        L.gemm(gb2, sh(blk.mlp.fc2.weight), dh, M=M, N=F, K=D, epilogue=L.EPI_DGELU, b_mn=True, aux=h)
         del gb2, h
         wgrad(dh, ln2, blk.mlp.fc1, F, D)
         dln2 = ln2  # reuse: ln2 output is dead after the fc1 wgrad above
@@ -640,13 +613,11 @@ class MlpFn(torch.autograd.Function):
         sh = store.shadow_of
         xb = _to_bf16(x).view(M, D)
         m1 = dropout_keep_mask("mlp.drop1", M, F, drop1, dev)
-        codes = _gelu_codes(F) if m1 is None else (L.EPI_GELU, L.EPI_DGELU, torch.bfloat16)
-        h = _empty((M, F), codes[2], dev)
+        h = _empty((M, F), torch.bfloat16, dev)
         act = _empty((M, F), torch.bfloat16, dev)
-        L.gemm(xb, sh(mlp.fc1.weight), act, M=M, N=F, K=D, epilogue=codes[0],
+        L.gemm(xb, sh(mlp.fc1.weight), act, M=M, N=F, K=D, epilogue=L.EPI_GELU,
                bias=None if mlp.fc1.bias is None else mlp.fc1.bias.data, aux=h, mask=m1,
                mask_scale=1.0 / (1.0 - drop1) if m1 is not None else 1.0)
-        ctx.dgelu = codes[1]
         out = _empty(x.shape[:-1] + (O,), torch.float32, dev)
         L.gemm(act, sh(mlp.fc2.weight), out, M=M, N=O, K=F, epilogue=L.EPI_F32,
                bias=None if mlp.fc2.bias is None else mlp.fc2.bias.data)
@@ -666,7 +637,7 @@ class MlpFn(torch.autograd.Function):
         L.gemm(dyb, act, gr(mlp.fc2.weight), M=O, N=F, K=M, epilogue=L.EPI_ATOMIC, a_mn=True, b_mn=True,
                colsum=None if mlp.fc2.bias is None else gr(mlp.fc2.bias))
         dh = act
-        L.gemm(dyb, sh(mlp.fc2.weight), dh, M=M, N=F, K=O, epilogue=ctx.dgelu, b_mn=True, aux=h)
+        L.gemm(dyb, sh(mlp.fc2.weight), dh, M=M, N=F, K=O, epilogue=L.EPI_DGELU, b_mn=True, aux=h)
         L.gemm(dh, xb, gr(mlp.fc1.weight), M=F, N=D, K=M, epilogue=L.EPI_ATOMIC, a_mn=True, b_mn=True,
                colsum=None if mlp.fc1.bias is None else gr(mlp.fc1.bias))
         dx = _empty(ctx.shape, torch.float32, dy.device)
