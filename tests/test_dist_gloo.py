@@ -1,5 +1,6 @@
-"""world_size-2 data-parallel plumbing on CPU (gloo): replica broadcast, per-stage gradient buckets, asynchronous
-all-reduce fired by the backward hooks, pre-step wait, 1/world folded into the optimizer, no_sync()."""
+"""world_size-2 data-parallel plumbing on CPU (gloo): replica broadcast, the gradient marked pending by the backward's
+hook and reduced by the optimizer's pre-step hook (fp32 in place, since the gradient is not on CUDA), 1/world folded
+into the optimizer, no_sync() and exactly-once reduction under gradient accumulation, meter reduction."""
 import os
 import socket
 
@@ -46,51 +47,36 @@ def _worker(rank, world, port, q):
         flat = [torch.zeros_like(st.flat) for _ in range(world)]
         dist.all_gather(flat, st.flat)
         assert all(torch.equal(flat[0], f) for f in flat)
-        # 2) buckets tile the flat buffer: embed | blocks.0. | blocks.1. | head
-        r = dp._ranges
-        assert r["embed"][0] == 0 and r["embed"][1] == r["blocks.0."][0] and r["blocks.0."][1] == r["blocks.1."][0]
-        assert r["blocks.1."][1] == r["head"][0] and r["head"][1] == st.total
-        # 3) hooks fire in backward order; the optimizer's pre-step hook waits; grads are SUMMED (mean is in grad_scale).
-        #    "block": one asynchronous all-reduce per bucket; "step" (default): one all-reduce of the flat buffer at step().
-        assert dp.sync_mode == "step"
-        #    "tail" (VITK_DP_SYNC=tail:1): blocks.1 .. head in one asynchronous all-reduce fired when blocks.1 is ready,
-        #    the rest (embed, blocks.0) at step().
-        for mode, in_flight in (("block", 4), ("step", 0), ("tail", 1)):
-            dp.sync_mode = mode
-            if mode == "tail":
-                dp._tail_tag, dp._tail_lo = "blocks.1.", r["blocks.1."][0]
-            st.grad.fill_(float(rank + 1))
-            for tag in ("head", "blocks.1.", "blocks.0.", "embed"):
-                st.fire_grad_ready(tag)
-            assert len(dp._works) == in_flight and dp._pending == (mode in ("step", "tail"))
-            opt.step()
-            assert len(dp._works) == 0 and not dp._pending
-            assert torch.equal(st.grad, torch.full_like(st.grad, float(sum(range(1, world + 1)))))
-            assert torch.equal(m.head.weight.grad, torch.full_like(m.head.weight, 3.0))  # p.grad views the flat buffer
-        dp.sync_mode = "block"
-        # 4) no_sync(): gradient accumulation micro-steps do not communicate
+        # 2) the backward's hook marks the gradient pending; the optimizer's pre-step hook reduces it in one all-reduce of
+        #    the flat buffer (fp32 in place: the gradient is not on CUDA).  Grads are SUMMED (the mean is in grad_scale).
+        st.grad.fill_(float(rank + 1))
+        st.fire_grad_ready()
+        assert dp._pending
+        opt.step()
+        assert not dp._pending and not hasattr(opt, "grad_lowp")
+        assert torch.equal(st.grad, torch.full_like(st.grad, float(sum(range(1, world + 1)))))
+        assert torch.equal(m.head.weight.grad, torch.full_like(m.head.weight, 3.0))  # p.grad views the flat buffer
+        # 3) no_sync(): gradient accumulation micro-steps do not communicate
         st.grad.fill_(float(rank + 1))
         with dp.no_sync():
-            st.fire_grad_ready("head")
-        assert len(dp._works) == 0 and float(st.grad[0]) == float(rank + 1)
-        # 4b) update_freq = 2 the way engine.train_one_epoch drives it: micro-batch 1 under no_sync(), micro-batch 2
-        #     synchronised -> every schedule reduces the ACCUMULATED gradient exactly once (a bucket reduced per
-        #     micro-batch would count the first micro-batch world_size times)
-        for mode in ("block", "step", "tail"):
-            dp.sync_mode = mode
-            st.grad.zero_()
-            with dp.no_sync():
-                st.grad.add_(float(rank + 1))
-                for tag in ("head", "blocks.1.", "blocks.0.", "embed"):
-                    st.fire_grad_ready(tag)
-            assert len(dp._works) == 0 and not dp._pending
-            st.grad.add_(10.0 * (rank + 1))
-            for tag in ("head", "blocks.1.", "blocks.0.", "embed"):
-                st.fire_grad_ready(tag)
-            dp.finish_gradient_sync()
-            dp.finish_gradient_sync()   # idempotent: clipping syncs first, step() must not reduce again
-            opt.step()
-            assert torch.equal(st.grad, torch.full_like(st.grad, 11.0 * sum(range(1, world + 1)))), mode
+            st.fire_grad_ready()
+        assert not dp._pending
+        opt.step()
+        assert float(st.grad[0]) == float(rank + 1)
+        # 4) update_freq = 2 the way engine.train_one_epoch drives it: micro-batch 1 under no_sync(), micro-batch 2
+        #    synchronised -> the ACCUMULATED gradient is reduced exactly once (a reduction per micro-batch would count
+        #    the first micro-batch world_size times)
+        st.grad.zero_()
+        with dp.no_sync():
+            st.grad.add_(float(rank + 1))
+            st.fire_grad_ready()
+        assert not dp._pending
+        st.grad.add_(10.0 * (rank + 1))
+        st.fire_grad_ready()
+        dp.finish_gradient_sync()
+        dp.finish_gradient_sync()   # idempotent: clipping syncs first, step() must not reduce again
+        opt.step()
+        assert torch.equal(st.grad, torch.full_like(st.grad, 11.0 * sum(range(1, world + 1))))
         # 5) metric meters reduce across ranks like the reference's SmoothedValue.synchronize_between_processes
         sv = utils.SmoothedValue()
         sv.update(float(rank + 1), n=1)
@@ -103,7 +89,7 @@ def _worker(rank, world, port, q):
         dist.destroy_process_group()
 
 
-def test_data_parallel_world2_gloo():
+def test_data_parallel_world2_gloo_one_allreduce():
     s = socket.socket()
     s.bind(("127.0.0.1", 0))
     port = s.getsockname()[1]

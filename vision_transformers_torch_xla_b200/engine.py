@@ -6,15 +6,13 @@ rewrites the no-decay group — SURVEY Appendix D #1), ``loss / update_freq``, b
 ``update_freq`` micro-batches, ``zero_grad``, optional EMA, meters, returned ``{meter: global_avg}``.
 What changes underneath: model, criterion and optimizer run on the vitk sm_100a kernels, gradient
 averaging across ranks is the NCCL all-reduce of ``parallel.DataParallel`` (one bf16 all-reduce of the flat
-gradient right after backward by default, per-block buckets overlapped with backward as an option; micro-batches
-that do not end in ``optimizer.step()`` run under ``no_sync()``), gradient clipping acts on the reduced
-gradient, and the device is only synchronised when a metric is actually read (every ``log_freq`` steps) instead
-of after every step (engine.py:278-279, 290-299).
+gradient after backward; micro-batches that do not end in ``optimizer.step()`` run under ``no_sync()``), gradient
+clipping acts on the reduced gradient, and the device is only synchronised when a metric is actually read (every
+``log_freq`` steps) instead of after every step (engine.py:278-279, 290-299).
 """
 from __future__ import annotations
 
 import contextlib
-import os
 from typing import Iterable
 
 import torch
@@ -70,7 +68,7 @@ def train_one_epoch(model: torch.nn.Module, criterion: torch.nn.Module, data_loa
             wandb_logger._wandb.log({"train/loss": metric_logger.meters["loss"].value, "train/learning_rate": lr_now,
                                      "train/epoch": epoch})
 
-    if on_gpu and os.environ.get("VITK_NO_PREFETCH", "0") != "1":
+    if on_gpu:
         data_loader = utils.DevicePrefetcher(data_loader, torch.device(device))   # H2D of batch i+1 overlaps step i
     for data_iter_step, (samples, targets) in enumerate(metric_logger.log_every(data_loader, 10, header, quiet=quiet)):
         step = data_iter_step // update_freq

@@ -212,7 +212,6 @@ class Block(nn.Module):
                              drop=proj_drop)
         self.ls2 = LayerScale(dim, init_values=init_values) if init_values else nn.Identity()
         self.drop_path2 = DropPath(drop_path) if drop_path > 0.0 else nn.Identity()
-        self._vitk_tag = "block"
         self._vitk_index = 0
 
     def _drop_probs(self):
@@ -255,7 +254,7 @@ class Block(nn.Module):
                     ops.dropout_keep_mask(site + "attn.attn_drop", B * H * N, N, pa, x.device), 1.0 / (1.0 - pa))
         root = st.__dict__.get("_in_root")
         ckpt = bool(getattr(root, "grad_checkpointing", False)) and torch.is_grad_enabled()
-        out = ops.BlockFn.apply(x, st.anchor, self, st, rs1, rs2, prev_rs, torch.is_grad_enabled(), self._vitk_tag, drop, ckpt)
+        out = ops.BlockFn.apply(x, st.anchor, self, st, rs1, rs2, prev_rs, torch.is_grad_enabled(), drop, ckpt)
         st.__dict__["_last_rs"] = rs2
         return out
 
@@ -357,7 +356,6 @@ class VisionTransformer(nn.Module):
                      act_layer=act_layer, mlp_layer=mlp_layer)
             for i in range(depth)])
         for i, blk in enumerate(self.blocks):
-            blk._vitk_tag = f"blocks.{i}."
             blk._vitk_index = i
         self.feature_info = [dict(module=f"blocks.{i}", num_chs=embed_dim, reduction=patch_size) for i in range(depth)]
         self.norm = norm_layer(embed_dim) if final_norm and not use_fc_norm else nn.Identity()

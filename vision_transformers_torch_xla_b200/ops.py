@@ -126,7 +126,7 @@ class EmbedFn(torch.autograd.Function):
             L.embed_bwd(g, gp, dpos, dpre[0], dpre[1], B, N, D, prefix)
             L.gemm(gp, ctx.src, dW, M=D, N=K, K=B * P, epilogue=L.EPI_ATOMIC, a_mn=True, b_mn=True, colsum=colsum)
         ctx.src = None
-        store.fire_grad_ready("embed")
+        store.fire_grad_ready()   # the last stage of every backward through the model (it takes store.anchor)
         return None, None, None, None, None
 
 
@@ -225,7 +225,7 @@ class BlockFn(torch.autograd.Function):
         return x_out, (x, ln1, mean1, rstd1, qkv, att, lse, x_mid, ln2, mean2, rstd2, h, act)
 
     @staticmethod
-    def forward(ctx, x, anchor, blk, store: ParamStore, rs1, rs2, prev_rs, save: bool, tag: str, drop=None,
+    def forward(ctx, x, anchor, blk, store: ParamStore, rs1, rs2, prev_rs, save: bool, drop=None,
                 checkpoint: bool = False):
         # drop = (keep masks of attn.proj_drop [M, D], mlp.drop1 [M, F], mlp.drop2 [M, D], 1 / (1 - p_proj),
         #         keep mask of attn.attn_drop [B * H * N, N], 1 / (1 - p_attn)) or None; a mask that is None is a site with p = 0
@@ -235,7 +235,7 @@ class BlockFn(torch.autograd.Function):
         B, N, D = x.shape
         x_out, saved = BlockFn._run(x, blk, store, rs1, rs2, drop)
         if save:
-            ctx.blk, ctx.store, ctx.tag = blk, store, tag
+            ctx.blk, ctx.store = blk, store
             ctx.dims = (B, N, D, blk.attn.num_heads, blk.attn.head_dim, blk.mlp.fc1.out_features)
             ctx.rs = (rs1, rs2, prev_rs)
             md1, _, md3, dscale, ma, ascale = drop if drop is not None else (None, None, None, 1.0, None, 1.0)
@@ -318,8 +318,7 @@ class BlockFn(torch.autograd.Function):
         L.layernorm_bwd(dln1, x, mean1, rstd1, blk.norm1.weight.data, g_mid, g_in, gb_prev, prev_rs, N,
                         gr(blk.norm1.weight), gr(blk.norm1.bias), M, D)
         store.chain[g_in.data_ptr()] = gb_prev
-        store.fire_grad_ready(ctx.tag)
-        return g_in, None, None, None, None, None, None, None, None, None, None
+        return g_in, None, None, None, None, None, None, None, None, None
 
 
 # ================================================================================================
@@ -416,7 +415,6 @@ class HeadFn(torch.autograd.Function):
             else:
                 L.layernorm_bwd(df, x.view(-1)[j * D:], mean, rstd, norm.weight.data, None, g.view(-1)[j * D:], None,
                                 None, 1, gr(norm.weight), gr(norm.bias), B, D, ld_x=N * D, ld_g=N * D)
-        store.fire_grad_ready("head")
         gb = _empty((B, N, D), torch.bfloat16, dev)
         L.rowscale_cast_bf16(g, ctx.prev_rs, N * D, gb)
         store.chain[g.data_ptr()] = gb

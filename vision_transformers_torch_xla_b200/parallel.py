@@ -1,41 +1,26 @@
 """Single-box data parallelism: one process per GPU, NCCL over NVLink 5 / NVSwitch.
 
-Replaces the reference's gradient sync — ``xm.optimizer_step(optimizer, barrier=True)``
-(/root/reference/engine.py:185) on TPU and ``DistributedDataParallel`` (/root/reference/main.py:855-857)
-on GPU — with a bucketed all-reduce driven by the fused backward stages:
+Replaces the reference's gradient sync — ``xm.optimizer_step(optimizer, barrier=True)`` (engine.py:185) on TPU and
+``DistributedDataParallel`` (main.py:855-857) on GPU — with one all-reduce (SUM) of the whole flat gradient buffer after
+backward.  The backward signals once, from its last stage; the all-reduce runs when the optimizer's pre-step hook (or
+``engine.clip_grad_norm_``) calls ``finish_gradient_sync()``.  The 1/world_size of the mean is folded into the AdamW
+kernel (``grad_scale``), so averaging costs no extra pass over the gradients.
 
-  * the flat fp32 gradient buffer is laid out in forward order, so the parameters of ``blocks.i`` (one
-    ~28 MB range for ViT-B) are one bucket;
-  * as soon as a stage's backward has enqueued its last wgrad kernel it fires ``grad_ready``; the bucket is
-    all-reduced (SUM) asynchronously on NCCL's stream while the next block's backward runs;
-  * the optimizer's pre-step hook waits for the outstanding buckets; the 1/world_size of the mean is folded
-    into the AdamW kernel (``grad_scale``), so averaging costs no extra pass over the gradients.
+Wire format: when the fused AdamW kernel consumes the result (an optimizer is attached and the gradient is on the GPU),
+the flat fp32 gradient is cast into a persistent bf16 buffer (one vitk cast kernel, 0.09 ms for ViT-B) and THAT is
+all-reduced (173 MB instead of 346 MB for ViT-B); AdamW reads the summed gradient from it.  Otherwise the fp32 buffer
+is all-reduced in place.
 
-Wire format (``VITK_DP_GRAD``): ``bf16`` (default) casts the flat fp32 gradient into a persistent bf16 buffer (one
-vitk cast kernel, 0.09 ms for ViT-B), all-reduces THAT (173 MB instead of 346 MB for ViT-B) and lets the AdamW kernel
-read the summed gradient from it; ``fp32`` all-reduces the fp32 buffer in place.  bf16 applies to the ``step`` and
-``tail:K`` schedules (a slice is cast when its gradient is final; ``block`` reduces fp32 slices in place).
+Nothing overlaps backward (DESIGN.md section 6): on 8 B200 an all-reduce per block during backward measured 36.17 ms/step
+against 34.98 ms for one after it, because NCCL's CTAs displace GEMM and attention kernels that are persistent with one
+CTA per SM; reducing only the last blocks during backward landed inside the run-to-run spread.
 
-Two schedules (``VITK_DP_SYNC``): ``block`` is the bucketed, overlapped one described above; ``step`` (default) reduces
-the whole flat gradient once, right after backward.  Measured at 8 B200, ViT-B/16, batch 256/GPU, same box, back to back:
-``step`` 34.98 ms/step (58 545 img/s, 96 % of 8 x the 1-GPU rate) vs ``block`` 36.17 ms (56 622 img/s, 93 %): over
-NVSwitch the 346 MB all-reduce costs ~1.2 ms when it runs alone, while NCCL's CTAs running *during* backward take SMs away
-from kernels that are persistent with exactly one CTA per SM (GEMM, attention), and a displaced CTA only starts when
-another one has finished its whole tile loop.
-
-A third schedule, ``tail:K``, reduces blocks K .. head in one asynchronous all-reduce fired when ``blocks.K`` is ready
-(overlapping only the backward of blocks K-1 .. 0 and the embedding) and the rest after backward; at 2 GPUs it measures
-the same as ``step`` (33.13 / 33.42 ms vs 33.43 / 33.40), and at 8 GPUs on the bf16 wire too (tail:9 / tail:6 / tail:3:
-34.05 / 34.07 / 34.23 ms vs 33.94 - 34.24 for ``step``; 1 GPU of that box: 33.05 ms; DESIGN.md section 6).
-
-With ``update_freq > 1`` buckets are only reduced on the micro-batch that precedes ``optimizer.step()``
+With ``update_freq > 1`` the gradient is only reduced on the micro-batch that precedes ``optimizer.step()``
 (``no_sync()`` context, like DDP).
 """
 from __future__ import annotations
 
 import contextlib
-import os
-from typing import List
 
 import torch
 import torch.distributed as dist
@@ -45,40 +30,21 @@ from .store import get_store
 
 
 class DataParallel(nn.Module):
-    def __init__(self, module: nn.Module, optimizer=None, broadcast: bool = True, bucket_tags=None):
+    def __init__(self, module: nn.Module, optimizer=None, broadcast: bool = True):
         super().__init__()
         if not (dist.is_available() and dist.is_initialized()):
             raise RuntimeError("DataParallel needs an initialised torch.distributed process group")
         self.module = module
         self.world_size = dist.get_world_size()
         self.require_sync = True
-        self._works: List = []
         self._pending = False
         st = get_store(self._find_root(module))
         self.store = st
         if broadcast:
             dist.broadcast(st.flat, src=0)  # identical replicas (DDP does the same at construction)
             st._sig = None
-        self._ranges = self._make_buckets(st)
-        # "step": one all-reduce after backward; "block": per-block buckets overlapped with backward; "tail:K": everything
-        # from blocks.K to the head in one all-reduce that overlaps the backward of blocks K-1 .. 0 and the embedding,
-        # the rest after backward
-        self.sync_mode = os.environ.get("VITK_DP_SYNC", "step")
-        self.grad_wire = os.environ.get("VITK_DP_GRAD", "bf16")
-        if self.grad_wire not in ("bf16", "fp32"):
-            raise ValueError(f"VITK_DP_GRAD={self.grad_wire!r}: expected 'bf16' or 'fp32'")
         self._grad16 = None     # persistent bf16 wire buffer (allocated on first use)
         self._optimizer = None
-        self._tail_tag = None
-        if self.sync_mode.startswith("tail:"):
-            k = int(self.sync_mode.split(":", 1)[1])
-            if f"blocks.{k}." not in self._ranges or k < 1:
-                raise ValueError(f"VITK_DP_SYNC={self.sync_mode!r}: the model has no blocks.{k} (or K < 1)")
-            self._tail_tag = f"blocks.{k}."
-            self._tail_lo = self._ranges[self._tail_tag][0]
-            self.sync_mode = "tail"
-        if self.sync_mode not in ("block", "step", "tail"):
-            raise ValueError(f"VITK_DP_SYNC={self.sync_mode!r}: expected 'step', 'block' or 'tail:K'")
         st.grad_ready_hooks.append(self._on_grad_ready)
         if optimizer is not None:
             self.attach_optimizer(optimizer)
@@ -94,74 +60,37 @@ class DataParallel(nn.Module):
             raise NotImplementedError("DataParallel: more than one trainable vitk model inside the wrapped module")
         return roots[0] if roots else module
 
-    @staticmethod
-    def _make_buckets(st):
-        """tag -> [start, end) of the flat buffer: one bucket per block, one for the head, one for the embed."""
-        ranges = {}
-        names = st.names
-        blocks = sorted({n.split(".")[1] for n in names if n.startswith("blocks.")}, key=int)
-        first_block = min((st.name_offsets[n][0] for n in names if n.startswith("blocks.")), default=st.total)
-        last_block_end = 0
-        for b in blocks:
-            lo, hi = st.range_of_prefix(f"blocks.{b}.")
-            ranges[f"blocks.{b}."] = (lo, hi)
-            last_block_end = max(last_block_end, hi)
-        ranges["embed"] = (0, first_block)
-        ranges["head"] = (last_block_end, st.total)
-        return ranges
-
     def attach_optimizer(self, optimizer):
         optimizer.grad_scale = 1.0 / self.world_size
         optimizer.pre_step_hooks.append(lambda opt: self.finish_gradient_sync())
         self._optimizer = optimizer
 
-    def _on_grad_ready(self, tag: str):
-        if not self.require_sync or self.world_size == 1:
-            return
-        if self.sync_mode == "step":
+    def _on_grad_ready(self):
+        if self.require_sync and self.world_size > 1:
             self._pending = True
-            return
-        if self.sync_mode == "tail":
-            self._pending = True
-            if tag == self._tail_tag and not self._works:
-                # the gradient of blocks K .. head is final here (forward-order layout, backward runs in reverse)
-                self._works.append(dist.all_reduce(self._wire(self._tail_lo, self.store.total), op=dist.ReduceOp.SUM,
-                                                   async_op=True))
-            return
-        rng = self._ranges.get(tag)
-        if rng is None or rng[1] <= rng[0]:
-            return
-        lo, hi = rng
-        self._works.append(dist.all_reduce(self.store.grad[lo:hi], op=dist.ReduceOp.SUM, async_op=True))
 
     def finish_gradient_sync(self):
         """Complete the gradient SUM over the replicas (idempotent: a second call before the next backward is a no-op)."""
         if self._pending:
             self._pending = False
-            hi = self._tail_lo if (self.sync_mode == "tail" and self._works) else self.store.total
-            dist.all_reduce(self._wire(0, hi), op=dist.ReduceOp.SUM)
+            dist.all_reduce(self._wire(), op=dist.ReduceOp.SUM)
             if self._lowp():
                 self._optimizer.grad_lowp = self._grad16   # AdamW reads the summed gradient from here (this step only)
-        for w in self._works:
-            w.wait()
-        self._works.clear()
 
     def _lowp(self) -> bool:
-        """bf16 wire: needs the optimizer (it reads the summed bf16 gradient) and a schedule whose slices are final when
-        they are cast (``step``, ``tail``; ``block`` reduces fp32 slices in place)."""
-        return (self.grad_wire == "bf16" and self._optimizer is not None and self.store.grad.is_cuda
-                and self.sync_mode in ("step", "tail"))
+        """bf16 wire: the fused AdamW kernel reads the summed bf16 gradient, so it needs the optimizer and a CUDA store."""
+        return self._optimizer is not None and self.store.grad.is_cuda
 
-    def _wire(self, lo: int, hi: int) -> torch.Tensor:
-        """The buffer that goes on the wire for gradient elements [lo, hi): the fp32 gradient itself, or its bf16 cast."""
+    def _wire(self) -> torch.Tensor:
+        """The buffer that goes on the wire: the fp32 gradient itself, or its bf16 cast."""
         if not self._lowp():
-            return self.store.grad[lo:hi]
+            return self.store.grad
         from . import _lib as L
 
         if self._grad16 is None or self._grad16.numel() != self.store.grad.numel():
             self._grad16 = torch.empty_like(self.store.grad, dtype=torch.bfloat16)
-        L.cast_bf16(self.store.grad[lo:hi], self._grad16[lo:hi])
-        return self._grad16[lo:hi]
+        L.cast_bf16(self.store.grad, self._grad16)
+        return self._grad16
 
     @contextlib.contextmanager
     def no_sync(self):

@@ -2,7 +2,7 @@
 
 Data layout in HBM (DESIGN.md §3): every parameter of the root module lives in ONE fp32 buffer
 (``flat``), padded to 64-element boundaries, in ``named_parameters()`` order — so the parameters of
-``blocks.i`` are one contiguous range (= one gradient all-reduce bucket).  ``grad`` mirrors it (the
+``blocks.i`` are one contiguous range.  ``grad`` mirrors it (the
 wgrad kernels ``red.add`` straight into it; ``p.grad`` are views), ``shadow`` is the bf16 copy the
 tcgen05 GEMMs read as their B operand.  ``nn.Parameter`` objects keep their names and shapes (the
 reference's state_dict contract, SURVEY Appendix B) but their ``.data`` is re-pointed into ``flat``.
@@ -23,7 +23,7 @@ ALIGN = 64  # elements; keeps every tensor 256-byte (fp32) / 128-byte (bf16) ali
 
 class ParamStore:
     def __init__(self, root: nn.Module, allow_cpu: bool = False):
-        """``allow_cpu`` exists for the host-logic tests (bucket ranges, gloo all-reduce plumbing); no kernel
+        """``allow_cpu`` exists for the host-logic tests (gloo all-reduce plumbing); no kernel
         can run on such a store — every launch wrapper rejects CPU tensors."""
         named = list(root.named_parameters())
         if not named:
@@ -33,10 +33,8 @@ class ParamStore:
             raise L.VitkError("vitk kernels only run on CUDA (sm_100a); move the model with .cuda() first — "
                               "there is no CPU path")
         self.device = dev
-        self.names: List[str] = []
         self.params: List[nn.Parameter] = []
         self.offsets: Dict[int, Tuple[int, int]] = {}
-        self.name_offsets: Dict[str, Tuple[int, int]] = {}
         off = 0
         for name, p in named:
             if p.dtype != torch.float32:
@@ -44,10 +42,8 @@ class ParamStore:
             if p.device != dev:
                 raise L.VitkError(f"parameter {name} is on {p.device}, expected {dev}")
             n = p.numel()
-            self.names.append(name)
             self.params.append(p)
             self.offsets[id(p)] = (off, n)
-            self.name_offsets[name] = (off, n)
             off += (n + ALIGN - 1) // ALIGN * ALIGN
         self.total = off
         self.flat = torch.zeros(self.total, dtype=torch.float32, device=dev)
@@ -69,7 +65,7 @@ class ParamStore:
         self.anchor = torch.zeros(1, device=dev, requires_grad=True)
         #: side channel between consecutive stage backwards: fp32 grad data_ptr -> bf16 copy (ops.py)
         self.chain: Dict[int, torch.Tensor] = {}
-        #: callbacks(name_prefix) fired when a stage's parameter gradients are complete (parallel.py)
+        #: callbacks() fired when a backward pass has enqueued its last gradient kernel (parallel.py)
         self.grad_ready_hooks: List = []
         self.attach_grads()
 
@@ -91,18 +87,6 @@ class ParamStore:
     def grad_of(self, p: nn.Parameter) -> torch.Tensor:
         o, n = self.offsets[id(p)]
         return self.grad[o:o + n].view(p.shape)
-
-    def range_of_prefix(self, prefix: str) -> Tuple[int, int]:
-        """[start, end) element range of all parameters whose name starts with ``prefix``."""
-        lo, hi = None, None
-        for name in self.names:
-            if name.startswith(prefix):
-                o, n = self.name_offsets[name]
-                lo = o if lo is None else min(lo, o)
-                hi = max(hi or 0, (o + n + ALIGN - 1) // ALIGN * ALIGN)
-        if lo is None:
-            raise KeyError(prefix)
-        return lo, hi
 
     # ------------------------------------------------------------------------------------
     def sync_shadow(self) -> None:
@@ -140,9 +124,9 @@ class ParamStore:
         if missing:
             self.grad.zero_()
 
-    def fire_grad_ready(self, prefix: str) -> None:
+    def fire_grad_ready(self) -> None:
         for hook in self.grad_ready_hooks:
-            hook(prefix)
+            hook()
 
 
 _tls = threading.local()
