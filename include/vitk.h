@@ -69,15 +69,15 @@ typedef struct vitk_gemm_args {
   int32_t epilogue;    /* enum vitk_epilogue                                                       */
   void* out;           /* bf16 or f32 depending on the epilogue                                    */
   int64_t ld_out;
-  void* aux;           /* GELU: activation-derivative output (bf16); DGELU: the same buffer as input                    */
+  void* aux;           /* GELU: activation-derivative output (bf16); DGELU: the same buffer as input; 16-byte aligned   */
   int64_t ld_aux;
-  const float* bias;   /* [N] or NULL                                                              */
-  const float* resid;  /* RESID: fp32 [M, N] residual stream input                                 */
+  const float* bias;   /* [N] or NULL; 16-byte aligned                                             */
+  const float* resid;  /* RESID: fp32 [M, N] residual stream input; 16-byte aligned, ld_resid % 4 == 0 */
   int64_t ld_resid;
   const float* rowscale; /* per-sample DropPath scale (mask/keep_prob), indexed by m/rows_per_group, or NULL */
   int32_t rows_per_group;
-  const float* colscale; /* LayerScale gamma [N] or NULL                                           */
-  const float* pos;    /* PATCH: pos_embed fp32 [(P+prefix), N]                                    */
+  const float* colscale; /* LayerScale gamma [N] or NULL; 16-byte aligned                          */
+  const float* pos;    /* PATCH: pos_embed fp32 [(P+prefix), N]; 16-byte aligned                   */
   int32_t tokens_per_img; /* PATCH: P                                                              */
   int32_t prefix;      /* PATCH: number of prefix (cls/dist) tokens                                */
   int32_t splits;      /* ATOMIC: split-K factor, 0 = choose to fill 148 SMs                       */

@@ -121,6 +121,23 @@ def test_argument_validation_reports_through_error_slot(lib):
     assert rc < 0 and b"drop_probs" in lib.vitk_last_error()
 
 
+@pytest.mark.parametrize("field", ["bias", "colscale", "pos", "resid", "aux"])
+def test_gemm_rejects_misaligned_side_operands(lib, field):
+    """The epilogues read bias / colscale / pos / resid with float4 loads and aux with 16-byte loads or TMA, so each must be
+    16-byte aligned whatever the epilogue.  The call carries epilogue code 7, which the dispatcher refuses ("epi=7") before
+    any CUDA call: a missing entry check fails this test instead of launching a kernel on a fake pointer."""
+    from vision_transformers_torch_xla_b200._lib import GemmArgs
+
+    args = GemmArgs()
+    args.A = args.B = args.out = 256
+    args.lda = args.ldb = args.ld_out = args.ld_aux = args.ld_resid = 64
+    args.M, args.N, args.K, args.epilogue = 128, 64, 64, 7
+    setattr(args, field, 256 + 4)
+    rc = lib.vitk_gemm_bf16(ctypes.byref(args), None)
+    assert rc == -2, lib.vitk_last_error()   # VITK_STATUS_ALIGN
+    assert field.encode() in lib.vitk_last_error()
+
+
 def test_missing_library_fails_loudly(monkeypatch, tmp_path):
     from vision_transformers_torch_xla_b200 import _lib
 

@@ -281,7 +281,7 @@ class _Timed:
 def gemm(a: torch.Tensor, b: torch.Tensor, out: torch.Tensor, *, M: int, N: int, K: int, epilogue: int,
          a_mn: bool = False, b_mn: bool = False, lda: Optional[int] = None, ldb: Optional[int] = None,
          ld_out: Optional[int] = None, aux: Optional[torch.Tensor] = None, ld_aux: Optional[int] = None,
-         bias: Optional[torch.Tensor] = None, resid: Optional[torch.Tensor] = None,
+         bias: Optional[torch.Tensor] = None, resid: Optional[torch.Tensor] = None, ld_resid: Optional[int] = None,
          rowscale: Optional[torch.Tensor] = None, rows_per_group: int = 1,
          colscale: Optional[torch.Tensor] = None, pos: Optional[torch.Tensor] = None,
          tokens_per_img: int = 0, prefix: int = 0, splits: int = 0, block_n: int = 0,
@@ -304,7 +304,7 @@ def gemm(a: torch.Tensor, b: torch.Tensor, out: torch.Tensor, *, M: int, N: int,
     args.out, args.ld_out = out.data_ptr(), (ld_out if ld_out is not None else N)
     args.aux, args.ld_aux = _ptr(aux), (ld_aux if ld_aux is not None else N)
     args.bias = _ptr(bias)
-    args.resid, args.ld_resid = _ptr(resid), N
+    args.resid, args.ld_resid = _ptr(resid), (ld_resid if ld_resid is not None else N)
     args.rowscale, args.rows_per_group = _ptr(rowscale), rows_per_group
     if mask is not None:
         _req(mask, torch.uint8, "gemm mask")

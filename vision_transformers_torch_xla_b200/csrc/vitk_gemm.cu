@@ -1025,10 +1025,6 @@ int pick_splits(int tiles, int num_k_blocks, int slots, int block_n) {
   return best;
 }
 
-// TMA needs 16-byte aligned bases and row pitches.  The entry checks already require them of out, ld_out, ld_resid
-// and N; a residual that is not 16-byte aligned takes the register-prefetch residual epilogue.
-inline bool resid_tma_ok(const vitk_gemm_args* a) { return ((uintptr_t)a->resid & 15) == 0; }
-
 template <int BLOCK_N, bool A_MN, bool B_MN, int EPI, bool CTA2>
 int launch_gemm(const vitk_gemm_args* a, cudaStream_t stream) {
   // 16 epilogue warps for the GELU epilogues (~20 instructions per element); 8 elsewhere.  With BLOCK_N = 192 and
@@ -1153,8 +1149,9 @@ int dispatch2(const vitk_gemm_args* a, cudaStream_t stream) {
         else return launch_gemm<BLOCK_N, false, false, EPI_BF16, CTA2>(a, stream);
       case EPI_GELU:  return launch_gemm<BLOCK_N, false, false, EPI_GELU, CTA2>(a, stream);
       case EPI_RESID:
+        // TMA needs 16-byte aligned bases and row pitches: the entry checks require them of out, resid, ld_out, ld_resid and N
         if constexpr (CTA2 || BLOCK_N < 256) {
-          if (a->K <= kResidTmaMaxK && resid_tma_ok(a) && a->mask == nullptr)   // the dropout mask lives in the staged-panel epilogue
+          if (a->K <= kResidTmaMaxK && a->mask == nullptr)   // the dropout mask lives in the staged-panel epilogue
             return launch_gemm<BLOCK_N, false, false, EPI_RESID_TMA, CTA2>(a, stream);
         }
         return launch_gemm<BLOCK_N, false, false, EPI_RESID, CTA2>(a, stream);
@@ -1202,6 +1199,12 @@ extern "C" int vitk_gemm_bf16(const vitk_gemm_args* a, void* stream_) {
                VITK_ERR_ALIGN, "gemm: A/B must be 16-byte aligned");
   VITK_REQUIRE(a->out != nullptr && (reinterpret_cast<uintptr_t>(a->out) & 15) == 0, VITK_ERR_ALIGN, "gemm: out must be 16-byte aligned");
   VITK_REQUIRE(a->ld_out % 8 == 0 || a->epilogue == EPI_F32, VITK_ERR_ALIGN, "gemm: ld_out must be a multiple of 8");
+  // The epilogues read bias, colscale, pos and resid with float4 loads (or TMA) and aux with 16-byte loads (or TMA).
+  // Checked whatever the epilogue, so that no layout or epilogue choice below depends on a side operand's address.
+  const struct { const void* ptr; const char* name; } side[] = {
+      {a->bias, "bias"}, {a->colscale, "colscale"}, {a->pos, "pos"}, {a->resid, "resid"}, {a->aux, "aux"}};
+  for (const auto& s : side)
+    VITK_REQUIRE((reinterpret_cast<uintptr_t>(s.ptr) & 15) == 0, VITK_ERR_ALIGN, "gemm: %s must be 16-byte aligned", s.name);
   if (a->epilogue == EPI_GELU || a->epilogue == EPI_DGELU)
     VITK_REQUIRE(a->aux != nullptr && a->ld_aux % 8 == 0, VITK_ERR_ALIGN, "gemm: aux pointer/ld required for GELU epilogues");
   if (a->epilogue == EPI_RESID)
