@@ -112,6 +112,8 @@ int vitk_gemm_bf16(const vitk_gemm_args* args, void* stream);
  *      Row r of x starts at x + r*ld_x (lets the 'token' pool normalise only the cls rows).
  * bwd: dx = LN'(dy); g_out = (g_in ? g_in : 0) + dx; gb_out = bf16(rowscale * g_out) (optional);
  *      dgamma/dbeta are ACCUMULATED (atomicAdd) into fp32 [dim] buffers.
+ *      Alignment (checked before anything else, also when rows == 0; NULL passes): x, g_in, g_out, gamma, dgamma and
+ *      dbeta 16-byte, dy and gb_out 8-byte; otherwise VITK_STATUS_ALIGN naming the pointer.
  * ---------------------------------------------------------------------------------------------- */
 int vitk_layernorm_fwd(const float* x, int64_t ld_x, const float* gamma, const float* beta,
                        void* y_bf16, int64_t ld_y, float* mean, float* rstd, int64_t rows,
@@ -154,7 +156,7 @@ int vitk_attn_bwd_dropout(const void* qkv, const void* out, const void* dout, co
  * embed_bwd: from g fp32 [B, N, D]: gp_bf16 [B*P, D] (patch rows; with gw > 0 the padded row order of an image operand:
  *            [B * (P / gw) * gwp, D], row (b, gy, gx'), zeros for gx' >= gw), dpos[N, D] += sum_b g,
  *            dprefix0[D] += sum_b g[b, 0, :] (cls_token), dprefix1[D] += sum_b g[b, 1, :] (dist_token, prefix == 2);
- *            either may be NULL (frozen token)
+ *            either may be NULL (frozen token).  g must be 16-byte and gp 8-byte aligned (checked before the shape).
  * ---------------------------------------------------------------------------------------------- */
 int vitk_patchify(const float* img, void* patches_bf16, int32_t B, int32_t C, int32_t H, int32_t W,
                   int32_t ps, void* stream);
@@ -174,13 +176,14 @@ int vitk_droppath_masks(float* rs, const float* drop_probs, int32_t rows, int32_
 /* ------------------------------------------------------------------------------------------------
  * Pooling (global_pool_nlc: vision_transformer.py:419-441).  mode 0 = 'avg' over non-prefix
  * tokens, mode 1 = 'token' (x[:, 0]).  bwd writes the full g [B, N, D] (zeros elsewhere).
+ * x, pooled, dpooled and g must be 16-byte aligned (checked before the shape).
  * ---------------------------------------------------------------------------------------------- */
 int vitk_pool_fwd(const float* x, float* pooled, int32_t B, int32_t N, int32_t D, int32_t prefix,
                   int32_t mode, void* stream);
 int vitk_pool_bwd(const float* dpooled, float* g, int32_t B, int32_t N, int32_t D, int32_t prefix,
                   int32_t mode, void* stream);
 
-/* out[c] += sum_r x[r, c]   (bias gradients).  x bf16 [rows, cols] pitch ld. */
+/* out[c] += sum_r x[r, c]   (bias gradients).  x bf16 [rows, cols] pitch ld; x 16-byte aligned (also when rows == 0). */
 int vitk_colsum_bf16(const void* x_bf16, int64_t ld, float* out, int64_t rows, int32_t cols,
                      void* stream);
 
@@ -231,6 +234,8 @@ int vitk_cast_bf16(const float* in, void* out_bf16, int64_t n, void* stream);
  * g_bf16 (optional): read the gradient from this bf16 copy instead of g (the copy the data-parallel layer all-reduces
  * at half the bytes); g is then only zeroed (zero_grad).  grad_scale_dev (optional): device scalar multiplied into the
  * gradient, e.g. the clip coefficient vitk_clip_coef left on the device.
+ * Alignment (checked before anything else, also when n == 0; NULL passes): p, m, v and ema 16-byte, g_bf16 and shadow_bf16
+ * 8-byte, and g 16-byte whenever it is read or zeroed (g_bf16 == NULL or zero_grad); otherwise VITK_STATUS_ALIGN.
  * ---------------------------------------------------------------------------------------------- */
 int vitk_adamw_flat(float* p, float* g, const void* g_bf16, const float* grad_scale_dev, float* m, float* v,
                     void* shadow_bf16, float* ema, int64_t n, const uint8_t* chunk_group, int32_t chunk,

@@ -138,6 +138,77 @@ def test_gemm_rejects_misaligned_side_operands(lib, field):
     assert field.encode() in lib.vitk_last_error()
 
 
+_FAKE = 1 << 20   # a 16-byte aligned fake device address; no call below reaches a kernel
+
+
+def _ln_bwd(lib, ptrs):
+    p = dict(dy=_FAKE, x=_FAKE, mean=_FAKE, rstd=_FAKE, gamma=_FAKE, g_in=_FAKE, g_out=_FAKE, gb_out=_FAKE, rowscale=None,
+             dgamma=_FAKE, dbeta=_FAKE)
+    p.update(ptrs)
+    return lib.vitk_layernorm_bwd(p["dy"], 768, p["x"], 768, p["mean"], p["rstd"], p["gamma"], p["g_in"], p["g_out"], 768,
+                                  p["gb_out"], p["rowscale"], 197, p["dgamma"], p["dbeta"], 0, 768, None)   # rows = 0
+
+
+def _adamw(lib, ptrs, g_bf16=None, zero_grad=0):
+    p = dict(p=_FAKE, g=_FAKE, g_bf16=g_bf16, m=_FAKE, v=_FAKE, shadow=_FAKE, ema=_FAKE)
+    p.update(ptrs)
+    lr, wd = (ctypes.c_float * 1)(1e-3), (ctypes.c_float * 1)(0.05)
+    return lib.vitk_adamw_flat(p["p"], p["g"], p["g_bf16"], None, p["m"], p["v"], p["shadow"], p["ema"], 0, None, 0, 1, lr, wd,
+                               ctypes.c_float(0.9), ctypes.c_float(0.999), ctypes.c_float(1e-8), 1, ctypes.c_float(1.0),
+                               ctypes.c_float(0.0), zero_grad, None)   # n = 0
+
+
+def _pool_fwd(lib, ptrs):
+    p = dict(x=_FAKE, pooled=_FAKE)
+    p.update(ptrs)
+    return lib.vitk_pool_fwd(p["x"], p["pooled"], 0, 197, 768, 1, 0, None)   # B = 0
+
+
+def _pool_bwd(lib, ptrs):
+    p = dict(dpooled=_FAKE, g=_FAKE)
+    p.update(ptrs)
+    return lib.vitk_pool_bwd(p["dpooled"], p["g"], 0, 197, 768, 1, 0, None)   # B = 0
+
+
+def _embed_bwd(lib, ptrs):
+    p = dict(g=_FAKE, gp=_FAKE)
+    p.update(ptrs)
+    return lib.vitk_embed_bwd(p["g"], p["gp"], _FAKE, _FAKE, None, 0, 197, 768, 1, 14, 16, None)   # B = 0
+
+
+def _colsum(lib, ptrs):
+    p = dict(x=_FAKE)
+    p.update(ptrs)
+    return lib.vitk_colsum_bf16(p["x"], 768, _FAKE, 0, 768, None)   # rows = 0
+
+
+# (entry point, pointer, status the call returns with every pointer aligned: 0 = VITK_STATUS_OK, -1 = VITK_STATUS_SHAPE)
+_ALIGN_CASES = [(_ln_bwd, nm, 0) for nm in ("x", "g_in", "g_out", "gamma", "dy", "gb_out", "dgamma", "dbeta")] + \
+               [(_adamw, nm, 0) for nm in ("p", "g", "g_bf16", "m", "v", "shadow", "ema")] + \
+               [(_pool_fwd, "x", -1), (_pool_fwd, "pooled", -1), (_pool_bwd, "dpooled", -1), (_pool_bwd, "g", -1),
+                (_embed_bwd, "g", -1), (_embed_bwd, "gp", -1), (_colsum, "x", 0)]
+
+
+@pytest.mark.parametrize("fn,name,aligned_rc", _ALIGN_CASES,
+                         ids=[f"{fn.__name__[1:]}-{nm}" for fn, nm, _ in _ALIGN_CASES])
+def test_misaligned_vector_pointers_are_refused(lib, fn, name, aligned_rc):
+    """Every pointer the LayerNorm backward, AdamW, pooling, embedding-backward and column-sum kernels access as 16- or
+    8-byte vectors is checked before the shape and before the early return of an empty problem.  Each call has rows,
+    n or B = 0, so with the check missing it returns VITK_STATUS_OK or a shape error and no kernel ever runs on the fake
+    pointer, which is off by 4 bytes."""
+    assert fn(lib, {}) == aligned_rc, lib.vitk_last_error()
+    rc = fn(lib, {name: _FAKE + 4})
+    assert rc == -2, lib.vitk_last_error()   # VITK_STATUS_ALIGN
+    assert f": {name} must be".encode() in lib.vitk_last_error()
+
+
+def test_adamw_ignores_the_alignment_of_a_gradient_it_does_not_touch(lib):
+    """With a bf16 gradient and zero_grad off, adamw_flat neither reads nor writes g."""
+    assert _adamw(lib, {"g": _FAKE + 4}, g_bf16=_FAKE) == 0, lib.vitk_last_error()
+    assert _adamw(lib, {"g": _FAKE + 4}, g_bf16=_FAKE, zero_grad=1) == -2
+    assert _adamw(lib, {"g": _FAKE + 4}) == -2
+
+
 def test_missing_library_fails_loudly(monkeypatch, tmp_path):
     from vision_transformers_torch_xla_b200 import _lib
 

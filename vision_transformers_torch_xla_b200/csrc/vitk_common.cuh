@@ -32,6 +32,12 @@ int vitk_check_launch(const char* what);
     if (!(cond)) return vitk_set_error(code, __VA_ARGS__); \
   } while (0)
 
+// A pointer that a kernel loads or stores as BYTES-wide vectors must be BYTES-aligned (NULL passes).  Entry points check
+// these first, ahead of the shape checks and of any early return on an empty problem.
+#define VITK_REQUIRE_ALIGNED(fn, name, ptr, bytes)                                                  \
+  VITK_REQUIRE((reinterpret_cast<uintptr_t>(ptr) & ((bytes) - 1)) == 0, VITK_ERR_ALIGN, \
+               fn ": " name " must be %d-byte aligned", (int)(bytes))
+
 // Encode a 2-D bf16/f32 tiled tensor map with 128-byte swizzle.
 //   inner = contiguous dimension (elements), outer = rows, ld = row pitch in elements.
 int vitk_make_tmap_2d(CUtensorMap* out, const void* base, int elem_bytes, uint64_t inner,

@@ -654,6 +654,8 @@ extern "C" int vitk_prefix_rows(float* x, const float* prefix_tok, const float* 
 
 extern "C" int vitk_embed_bwd(const float* g, void* gp_bf16, float* dpos, float* dprefix0, float* dprefix1, int32_t B,
                               int32_t N, int32_t D, int32_t prefix, int32_t gw, int32_t gwp, void* stream) {
+  VITK_REQUIRE_ALIGNED("embed_bwd", "g", g, 16);
+  VITK_REQUIRE_ALIGNED("embed_bwd", "gp", gp_bf16, 8);
   VITK_REQUIRE(B > 0 && N > 0 && D > 0 && D % 4 == 0 && prefix >= 0 && prefix <= 2 && prefix <= N, VITK_ERR_SHAPE,
                "embed_bwd: bad shape (prefix must be 0, 1 or 2)");
   VITK_REQUIRE(gw == 0 || (gw > 0 && gwp >= gw && (N - prefix) % gw == 0), VITK_ERR_SHAPE,
@@ -673,6 +675,8 @@ extern "C" int vitk_embed_bwd(const float* g, void* gp_bf16, float* dpos, float*
 
 extern "C" int vitk_pool_fwd(const float* x, float* pooled, int32_t B, int32_t N, int32_t D, int32_t prefix,
                              int32_t mode, void* stream) {
+  VITK_REQUIRE_ALIGNED("pool_fwd", "x", x, 16);
+  VITK_REQUIRE_ALIGNED("pool_fwd", "pooled", pooled, 16);
   VITK_REQUIRE(B > 0 && N > prefix && D > 0 && D % 4 == 0, VITK_ERR_SHAPE, "pool_fwd: bad shape");
   VITK_REQUIRE(mode == 0 || mode == 1, VITK_ERR_UNSUPPORTED, "pool_fwd: mode %d (0=avg, 1=token)", mode);
   dim3 grid(blocks_for(D / 4, 64), B), block(64, 4);
@@ -682,6 +686,8 @@ extern "C" int vitk_pool_fwd(const float* x, float* pooled, int32_t B, int32_t N
 
 extern "C" int vitk_pool_bwd(const float* dpooled, float* g, int32_t B, int32_t N, int32_t D, int32_t prefix,
                              int32_t mode, void* stream) {
+  VITK_REQUIRE_ALIGNED("pool_bwd", "dpooled", dpooled, 16);
+  VITK_REQUIRE_ALIGNED("pool_bwd", "g", g, 16);
   VITK_REQUIRE(B > 0 && N > prefix && D > 0 && D % 4 == 0, VITK_ERR_SHAPE, "pool_bwd: bad shape");
   VITK_REQUIRE(mode == 0 || mode == 1, VITK_ERR_UNSUPPORTED, "pool_bwd: mode %d (0=avg, 1=token)", mode);
   VITK_REQUIRE((long long)B * N < (1LL << 31), VITK_ERR_SHAPE, "pool_bwd: B * N must be below 2^31");
@@ -691,6 +697,7 @@ extern "C" int vitk_pool_bwd(const float* dpooled, float* g, int32_t B, int32_t 
 }
 
 extern "C" int vitk_colsum_bf16(const void* x_bf16, int64_t ld, float* out, int64_t rows, int32_t cols, void* stream) {
+  VITK_REQUIRE_ALIGNED("colsum", "x", x_bf16, 16);
   VITK_REQUIRE(rows >= 0 && cols > 0 && cols % 8 == 0 && ld % 8 == 0, VITK_ERR_SHAPE, "colsum: cols/ld must be multiples of 8");
   if (rows == 0) return VITK_OK;
   const unsigned gx = blocks_for(cols, 256);
@@ -748,6 +755,15 @@ extern "C" int vitk_adamw_flat(float* p, float* g, const void* g_bf16, const flo
                                void* shadow_bf16, float* ema, int64_t n, const uint8_t* chunk_group, int32_t chunk,
                                int32_t num_groups, const float* lr, const float* wd, float beta1, float beta2, float eps,
                                int64_t step, float grad_scale, float ema_decay, int32_t zero_grad, void* stream) {
+  // float4 accesses to p, g, m, v, ema; 8-byte ones to g_bf16 and shadow.  g is read only without g_bf16, and written
+  // only by zero_grad.
+  VITK_REQUIRE_ALIGNED("adamw", "p", p, 16);
+  if (g_bf16 == nullptr || zero_grad) VITK_REQUIRE_ALIGNED("adamw", "g", g, 16);
+  VITK_REQUIRE_ALIGNED("adamw", "g_bf16", g_bf16, 8);
+  VITK_REQUIRE_ALIGNED("adamw", "m", m, 16);
+  VITK_REQUIRE_ALIGNED("adamw", "v", v, 16);
+  VITK_REQUIRE_ALIGNED("adamw", "shadow", shadow_bf16, 8);
+  VITK_REQUIRE_ALIGNED("adamw", "ema", ema, 16);
   VITK_REQUIRE(n >= 0 && n % 4 == 0, VITK_ERR_SHAPE, "adamw: n=%lld must be a multiple of 4", (long long)n);
   VITK_REQUIRE(num_groups >= 1 && num_groups <= ADAMW_MAX_GROUPS, VITK_ERR_SHAPE, "adamw: num_groups=%d not in [1,%d]", num_groups, ADAMW_MAX_GROUPS);
   VITK_REQUIRE(chunk_group == nullptr || (chunk > 0 && chunk % 4 == 0), VITK_ERR_SHAPE, "adamw: chunk must be a positive multiple of 4");
@@ -765,7 +781,6 @@ extern "C" int vitk_adamw_flat(float* p, float* g, const void* g_bf16, const flo
   h.inv_bc1 = (float)(1.0 / bc1);
   h.inv_sqrt_bc2 = (float)(1.0 / sqrt(bc2));
   h.grad_scale = grad_scale; h.ema_decay = ema_decay; h.zero_grad = zero_grad;
-  VITK_REQUIRE(g_bf16 == nullptr || ((uintptr_t)g_bf16 & 7) == 0, VITK_ERR_ALIGN, "adamw: g_bf16 must be 8-byte aligned");
   adamw_kernel<<<blocks_for(n / 4, 256), 256, 0, (cudaStream_t)stream>>>(p, g, (const __nv_bfloat16*)g_bf16, grad_scale_dev, m, v,
                                                                           (__nv_bfloat16*)shadow_bf16, ema, n, chunk_group,
                                                                           chunk > 0 ? chunk : 4, h);

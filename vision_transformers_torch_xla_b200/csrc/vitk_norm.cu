@@ -429,18 +429,24 @@ extern "C" int vitk_layernorm_bwd(const void* dy_bf16, int64_t ld_dy, const floa
                                   const float* g_in, float* g_out, int64_t ld_g, void* gb_out_bf16,
                                   const float* rowscale, int32_t rows_per_group, float* dgamma,
                                   float* dbeta, int64_t rows, int32_t dim, void* stream) {
+  // both kernels read x, g_in, gamma and write g_out as float4, read dy and write gb_out as 8-byte vectors
+  VITK_REQUIRE_ALIGNED("layernorm_bwd", "x", x, 16);
+  VITK_REQUIRE_ALIGNED("layernorm_bwd", "g_in", g_in, 16);
+  VITK_REQUIRE_ALIGNED("layernorm_bwd", "g_out", g_out, 16);
+  VITK_REQUIRE_ALIGNED("layernorm_bwd", "gamma", gamma, 16);
+  VITK_REQUIRE_ALIGNED("layernorm_bwd", "dy", dy_bf16, 8);
+  VITK_REQUIRE_ALIGNED("layernorm_bwd", "gb_out", gb_out_bf16, 8);
+  VITK_REQUIRE_ALIGNED("layernorm_bwd", "dgamma", dgamma, 16);   // 16-byte vector reductions
+  VITK_REQUIRE_ALIGNED("layernorm_bwd", "dbeta", dbeta, 16);
   VITK_REQUIRE(rows >= 0 && rows < (1LL << 31) && dim > 0, VITK_ERR_SHAPE, "layernorm_bwd: bad shape");
   VITK_REQUIRE(dim % 4 == 0 && dim <= MAXV * 128, VITK_ERR_SHAPE, "layernorm_bwd: dim=%d must be a multiple of 4 and <= %d", dim, MAXV * 128);
   VITK_REQUIRE(ld_x % 4 == 0 && ld_dy % 4 == 0 && ld_g % 4 == 0, VITK_ERR_ALIGN, "layernorm_bwd: row pitches must be multiples of 4 elements");
   VITK_REQUIRE(mean && rstd && g_out, VITK_ERR_SHAPE, "layernorm_bwd: mean/rstd/g_out required");
-  VITK_REQUIRE(((uintptr_t)dgamma & 15) == 0 && ((uintptr_t)dbeta & 15) == 0, VITK_ERR_ALIGN,
-               "layernorm_bwd: dgamma / dbeta must be 16-byte aligned (vector reductions)");
   if (rows == 0) return VITK_OK;
   const int vpl = (dim + 127) / 128;
-  // bulk-copy path: 16-byte aligned rows of every stream
+  // bulk-copy path: 16-byte aligned rows of every stream (x and g_in are by the checks above)
   const int rw = ring_warps(dim);
-  const bool ring_ok = rw > 0 && rows >= 4096 && dim % 8 == 0 && ld_dy % 8 == 0 && ((uintptr_t)dy_bf16 & 15) == 0 &&
-                       ((uintptr_t)x & 15) == 0 && (g_in == nullptr || ((uintptr_t)g_in & 15) == 0);
+  const bool ring_ok = rw > 0 && rows >= 4096 && dim % 8 == 0 && ld_dy % 8 == 0 && ((uintptr_t)dy_bf16 & 15) == 0;
   if (ring_ok) {
 #define LN_RING_CASE(V)                                                                                              \
   return (dim == (V) * 128 ? launch_ln_bwd_ring<V, true> : launch_ln_bwd_ring<V, false>)(dy_bf16, ld_dy, x, ld_x, mean, rstd, gamma, g_in, g_out, ld_g, gb_out_bf16, rowscale, \
